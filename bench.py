@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]                 # our sm_100a path
   python bench.py --impl reference [--gpus N] [--steps K] [--warmup W]  # CPU oracle port of the reference
+  python bench.py --dump-outputs DIR ...    # also store the last timed step's outputs as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input:
 thermal preprocessing of 2B raw 16-bit frames -> fused thermal-aware loss
@@ -24,6 +25,7 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (no __pycache__)
 sys.path.insert(0, ROOT)
 
 METRIC = "frames/sec of fused loss fwd+bwd+preproc"
@@ -49,7 +51,15 @@ def parse():
                          "(640x512 u16 preprocessing + pointmap->depth + metrics over a dataset shard; extra line)")
     ap.add_argument("--eval-frames", type=int, default=2560, help="frames per rank for --workload eval (8 ranks: 20 480)")
     ap.add_argument("--eval-batch", type=int, default=256, help="frames per evaluation step (the dataset shard is cut into batches of this size)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned to its caller as DIR/<name>.npy "
+                         "(float32 / float64; arrays above %d elements as a fixed seeded sample, see dump_outputs)" % DUMP_SAMPLE)
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and (a.impl != "b200" or a.workload != "train"):
+        ap.error("--dump-outputs applies to the timed step of --impl b200 --workload train")
+    return a
 
 
 def workload_name(a):
@@ -312,6 +322,30 @@ def load_peak():
     return peak, src
 
 
+DUMP_SAMPLE = 1 << 20      # elements kept of each large output: 5 sampled arrays x 4 MB stay well under 64 MB
+
+
+def dump_outputs(step, out_dir):
+    """Write the outputs of the step's latest call as out_dir/<name>.npy: the packed result vector, the per-sample
+    loss rows, the per-image metrics, the percentiles, the four gradients and the preprocessed thermal batch.  An
+    array with more than DUMP_SAMPLE elements is stored as the elements at DUMP_SAMPLE flat indices drawn without
+    replacement (sorted) by a generator seeded with 0, so that two runs with the same arguments store the same
+    positions.  Call after the step's results are ordered on the current stream (finish() / wait_result())."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"result": step.result, "per_sample": step.loss_out["per_sample"], "batch": step.loss_out["batch"],
+              "metrics": step.met_out["metrics_f64"], "percentiles": step.pre_both["percentiles"],
+              "thermal": step.pre_both["thermal"]}
+    arrays.update({k: step.loss_out[k] for k in ("dpred1", "dpred2", "dconf1", "dconf2")})
+    for name, t in arrays.items():
+        if t.numel() > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        a = t.cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64 if a.dtype == np.float64 else np.float32))
+
+
 def time_steps(fn, steps, warmup, finish=None):
     """CUDA-event time of `steps` calls of fn() after `warmup` untimed ones (ms per call)."""
     import torch
@@ -478,6 +512,8 @@ def run_b200(a):
     clocks = sampler.stop() if rank == 0 else None
     result_vec = step.wait_result().clone()
     step_result_size = result_vec.numel()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(step, a.dump_outputs)
     summary = HotPathStep.summarize(result_vec.cpu())
 
     # ---------------- data parallel: the exchanged vector against an independent all-gather of the local vectors

@@ -1,18 +1,33 @@
-"""CPU, build container only: the oracle restatements equal the LIVE, unmodified reference on fresh
-random inputs.  Skipped where /root/reference is not mounted (the GPU box): there the golden
-fixtures (test_oracle_golden.py) carry the pin."""
+"""CPU: the oracle restatements equal the LIVE, unmodified reference on fresh random inputs, and the stock
+libraries the reference calls (cv2, numpy, scipy).  The reference tree is not part of this repository
+(oracle/reference_bridge.py): where it is not mounted, the comparisons with the live reference functions skip and the
+golden vectors it wrote (tests/golden/, test_oracle_golden.py) carry the pin; the comparisons with the stock
+libraries and with those golden vectors run everywhere."""
 import numpy as np
 import pytest
 import torch
 
 from oracle import ref_loss, ref_metrics, ref_preprocess, ref_sobel, reference_bridge
 
-pytestmark = pytest.mark.skipif(not reference_bridge.available(), reason="reference tree not mounted")
-
 
 @pytest.fixture(scope="module")
 def ref():
+    if not reference_bridge.available():
+        pytest.skip("reference tree not mounted")
     return reference_bridge.load()
+
+
+@pytest.fixture(scope="module")
+def live_ref():
+    """The loaded reference, or None where it is not mounted."""
+    return reference_bridge.load() if reference_bridge.available() else None
+
+
+@pytest.fixture(scope="module")
+def cv2():
+    cv2 = pytest.importorskip("cv2")
+    cv2.ipp.setUseIPP(False)        # the deterministic C++ paths, as reference_bridge.load() sets them
+    return cv2
 
 
 @pytest.mark.parametrize("H,W,multi", [(33, 47, True), (64, 64, False), (224, 224, True)])
@@ -38,15 +53,17 @@ def test_loss_equals_live_reference(ref, H, W, multi):
         assert (x - y).abs().max().item() <= 2e-9
 
 
-def test_preprocess_equals_live_reference(ref):
+def test_preprocess_equals_live_reference(live_ref, cv2):
     raw = ref_preprocess.make_raw_frames(2, seed=11)
     for frame in raw:
         for (w, h) in ((224, 224), (512, 384), (301, 199)):
-            assert (ref.cv2.resize(frame, (w, h)) == ref_preprocess.resize_bilinear(frame, (h, w))).all()
+            assert (cv2.resize(frame, (w, h)) == ref_preprocess.resize_bilinear(frame, (h, w))).all()
             x = frame.astype(np.float32) / 65535.0
-            assert (ref.cv2.resize(x, (w, h)) == ref_preprocess.resize_bilinear(x, (h, w))).all()
-            t = torch.from_numpy(np.repeat(ref.cv2.resize(frame, (w, h)).astype(np.float32)[None], 3, 0))
-            assert (ref.preprocessing.enhance_thermal_contrast(t).numpy() == ref_preprocess.train_path(frame, (h, w))[0]).all()
+            assert (cv2.resize(x, (w, h)) == ref_preprocess.resize_bilinear(x, (h, w))).all()
+            if live_ref is not None:
+                t = torch.from_numpy(np.repeat(cv2.resize(frame, (w, h)).astype(np.float32)[None], 3, 0))
+                assert (live_ref.preprocessing.enhance_thermal_contrast(t).numpy() ==
+                        ref_preprocess.train_path(frame, (h, w))[0]).all()
 
 
 def test_metrics_equal_live_reference(ref):
@@ -66,16 +83,16 @@ def test_sobel_equals_live_reference(ref):
     assert torch.equal(m.preprocess_thermal(x), ref_sobel.preprocess_thermal_torch(x, m.edge_weight, m.temp_scale))
 
 
-def test_evaluate_golden_is_the_live_reference(ref):
+def test_evaluate_golden_is_the_live_reference(live_ref):
     """tests/golden/evaluate_kat.npz (what the GPU test of evaluate_thermal_depth compares with) is what the live
     reference function returns for the fake model / loader of oracle/fake_eval.py, and equals the oracle's
     accumulate_dataset over per-sample oracle metrics."""
     import os
     from oracle import fake_eval
     gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "evaluate_kat.npz"))
-    for conv in fake_eval.CONVENTIONS:
+    for conv in (fake_eval.CONVENTIONS if live_ref is not None else ()):
         model = fake_eval.FakeModel(conv)
-        res = ref.metrics.evaluate_thermal_depth(model, fake_eval.make_loader(seed=7), torch.device("cpu"))
+        res = live_ref.metrics.evaluate_thermal_depth(model, fake_eval.make_loader(seed=7), torch.device("cpu"))
         np.testing.assert_array_equal(fake_eval.as_vector(res), gold[conv])
     per = []
     model = fake_eval.FakeModel("tuple_tensor")
@@ -90,14 +107,13 @@ def test_evaluate_golden_is_the_live_reference(ref):
     np.testing.assert_allclose([acc[k] for k in fake_eval.KEYS], gold["tuple_tensor"], rtol=1e-6)
 
 
-def test_fire_restatements_equal_live_libraries(ref):
+def test_fire_restatements_equal_live_libraries(live_ref, cv2):
     """oracle/ref_fire.py: the NumPy restatements of cv2 CLAHE / Canny / np.histogram / scipy find_peaks are identical
     to the live libraries, Sobel / bilateral agree to rounding; the three reference functions restated on the stock
     libraries equal the live reference (np.random seeded); tests/golden/fire_kat.npz is what the live reference gives."""
     import importlib, os, sys
     from scipy.signal import find_peaks
     from oracle import ref_fire
-    cv2 = ref.cv2
     rng = np.random.default_rng(0)
     for (h, w) in ((96, 128), (75, 100), (224, 224)):
         f = ref_fire.make_fire_frame(h, w, seed=h)
@@ -115,19 +131,24 @@ def test_fire_restatements_equal_live_libraries(ref):
     for _ in range(300):
         hh = rng.integers(0, rng.integers(3, 60), 100)
         assert list(find_peaks(hh, height=hh.max() * 0.3, distance=10)[0]) == list(ref_fire.find_peaks_height_distance(hh, hh.max() * 0.3, 10))
-    sys.path.insert(0, ref.root)
-    try:
-        m = importlib.import_module("thermal_dustr_inference_for_experiment")
-    finally:
-        sys.path.remove(ref.root)
+    m = None
+    if live_ref is not None:
+        sys.path.insert(0, live_ref.root)
+        try:
+            m = importlib.import_module("thermal_dustr_inference_for_experiment")
+        finally:
+            sys.path.remove(live_ref.root)
     gold = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "fire_kat.npz"))
     for (h, w) in ((96, 128), (75, 100)):
         tag = f"{h}x{w}"
         f = ref_fire.make_fire_frame(h, w, seed=h)
-        np.random.seed(11); live = m.preprocess_fire_scene_thermal(torch.from_numpy(f)).numpy()
         np.random.seed(11); nz = np.random.rand(h, w)
-        assert np.array_equal(live, gold["pre_" + tag]) and np.array_equal(ref_fire.preprocess_fire_scene_thermal(f, nz), live)
-        np.random.seed(12); live = m.advanced_fire_scene_processing(torch.from_numpy(f)).numpy()
+        assert np.array_equal(ref_fire.preprocess_fire_scene_thermal(f, nz), gold["pre_" + tag])
         np.random.seed(12); nz = np.random.rand(h, w)
-        assert np.array_equal(live, gold["adv_" + tag]) and np.array_equal(ref_fire.advanced_fire_scene_processing(f, nz), live)
+        assert np.array_equal(ref_fire.advanced_fire_scene_processing(f, nz), gold["adv_" + tag])
+        if m is not None:
+            np.random.seed(11); live = m.preprocess_fire_scene_thermal(torch.from_numpy(f)).numpy()
+            assert np.array_equal(live, gold["pre_" + tag])
+            np.random.seed(12); live = m.advanced_fire_scene_processing(torch.from_numpy(f)).numpy()
+            assert np.array_equal(live, gold["adv_" + tag])
         assert np.array_equal(ref_fire.depth_refinement(gold["depth_" + tag]), gold["refined_" + tag])

@@ -262,6 +262,42 @@ def test_pipelined_steps_equal_plain_steps(cuda_device):
     assert torch.equal(r, want[-1][0]) and torch.equal(piped.loss_out["dpred1"], want[-1][1])
 
 
+def test_bench_dump_outputs(cuda_device, tmp_path):
+    """bench.py --dump-outputs: two runs with different step counts store the same outputs of their last timed step,
+    and those are what one HotPathStep call on bench's inputs returns."""
+    import json
+    import os
+    import subprocess
+    import sys
+    from thermal3d_vision_b200.pipeline import HotPathStep
+    import bench
+    B, H, W = 2, 64, 96
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    dumps = []
+    for steps in (2, 5):
+        out = tmp_path / f"steps{steps}"
+        res = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--steps", str(steps), "--warmup", "0",
+                              "--batch", str(B), "--height", str(H), "--width", str(W), "--no-extras", "--no-cpu-baseline",
+                              "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert json.loads(res.stdout.strip().splitlines()[-1])["steps"] == steps
+        dumps.append({f[:-4]: np.load(out / f) for f in sorted(os.listdir(out))})
+    assert set(dumps[0]) == {"result", "per_sample", "batch", "metrics", "percentiles", "thermal",
+                             "dpred1", "dpred2", "dconf1", "dconf2"}
+    for name, a in dumps[0].items():
+        assert a.dtype in (np.float32, np.float64), name
+        np.testing.assert_array_equal(a, dumps[1][name], err_msg=name)
+    d = bench.make_inputs_torch(B, H, W, seed=0, device=cuda_device)
+    step = HotPathStep(B, H, W, device=cuda_device, pipelined=True, **KW)
+    r = step.run_device(*[d[n] for n in bench.KEYS])
+    step.finish()
+    np.testing.assert_array_equal(dumps[0]["result"], r.cpu().numpy())
+    for name in ("dpred1", "dpred2", "dconf1", "dconf2", "per_sample"):
+        np.testing.assert_array_equal(dumps[0][name], step.loss_out[name].cpu().numpy(), err_msg=name)
+    np.testing.assert_array_equal(dumps[0]["thermal"], step.pre_both["thermal"].cpu().numpy())
+    np.testing.assert_array_equal(dumps[0]["metrics"], step.met_out["metrics_f64"].cpu().numpy())
+
+
 def test_bench_configuration_matches_oracle(cuda_device):
     """The exact thing bench.py times -- HotPathStep at batch 64, 512x384 pointmaps, 640x512 raw frames from
     bench.make_inputs_torch, replicated-plane flag, statistics hand-off, internal streams, epilogue -- against the
