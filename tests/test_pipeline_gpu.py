@@ -459,7 +459,7 @@ def test_pipelined_soak_without_host_syncs(cuda_device):
         torch.cuda.synchronize()
         want.append((r, plain.pre_both["thermal"].clone(), plain.loss_out["dpred2"].clone()))
     step = HotPathStep(B, H, W, raw_hw=(120, 320), device=cuda_device, pipelined=True)
-    assert step.sample_ahead
+    assert step.pipelined
     snaps, prev = [], None
     for k in range(60):
         j = (k * 5 // 2) & 1 if k % 3 else k & 1

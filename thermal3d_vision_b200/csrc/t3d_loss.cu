@@ -15,8 +15,6 @@
 #include <type_traits>
 #include <string.h>
 
-#include <stdlib.h>
-
 namespace {
 
 constexpr float kEps = 1e-5f;          // utils/loss.py:240
@@ -158,11 +156,8 @@ __global__ void __launch_bounds__(kSThreads, 4) thermal_stats_kernel(const Stats
 // (the strip's right edge: one 8-byte load); the half-resolution sums ride along on row pairs.  No shared memory.
 // MODE 0: one plane, 1: three planes, 2: three bit-identical planes (plane 0 is read, gray = gray3(v, v, v)).
 constexpr int kSMWarps = 4;
-// rows per work item (even; tuning knob T3D_STATS_ROWS): shorter marches = finer load balance, more halo rows
-static int stats_march_rows() {
-    static const int v = [] { const char* e = getenv("T3D_STATS_ROWS"); const int r = e ? atoi(e) : 32; return r < 4 ? 4 : (r & ~3); }();
-    return v;
-}
+// rows per work item (a multiple of 4): shorter marches = finer load balance, more halo rows
+constexpr int kStatsMarchRows = 32;
 struct SRow { float g[4], e0, e1; };     // gray of the lane's quad and of the two pixels right of it
 
 template <bool MULTI, int MODE>
@@ -956,7 +951,7 @@ WsLayout ws_layout(int B, int H, int W, int multi = 0) {
     L.tiles_x = (W + kTW - 1) / kTW;    L.tiles_y = (H + kTH - 1) / kTH;
     size_t off = 0;
     L.counter = off;        off += 256;
-    L.sm_bands = (H + stats_march_rows() - 1) / stats_march_rows(); L.sm_strips = (W + 127) / 128;
+    L.sm_bands = (H + kStatsMarchRows - 1) / kStatsMarchRows; L.sm_strips = (W + 127) / 128;
     const size_t stats_tiles = (size_t)max(L.stiles_x * L.stiles_y, L.sm_bands * L.sm_strips);
     L.stats_partials = off; off += t3d_align_up((size_t)B * 2 * stats_tiles * 4 * sizeof(float), 256);
     // sized for the tile kernel (16-row tiles) and the marching kernel (>= 8-row bands)
@@ -986,9 +981,9 @@ template <bool MULTI>
 int launch_stats_march(const StatsArgs& sa, int nbands, int nstrips, cudaStream_t st) {
     const int items = sa.B * 2 * nbands * nstrips;
     const int grid = (items + kSMWarps - 1) / kSMWarps;
-    if (sa.replicated) T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 2><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, stats_march_rows())));
-    else if (sa.tch == 3) T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 1><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, stats_march_rows())));
-    else T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 0><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, stats_march_rows())));
+    if (sa.replicated) T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 2><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, kStatsMarchRows)));
+    else if (sa.tch == 3) T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 1><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, kStatsMarchRows)));
+    else T3D_LAUNCH("thermal_stats_march_kernel", st, (thermal_stats_march_kernel<MULTI, 0><<<grid, kSMWarps * 32, 0, st>>>(sa, nbands, nstrips, kStatsMarchRows)));
     return T3D_OK;
 }
 
@@ -1102,14 +1097,9 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
     const bool ms = multi && thermal_on;
     int n_partials = L.tiles_x * L.tiles_y;
     int rc;
-    static const int march_rows = [] {
-        const char* e = getenv("T3D_MARCH_ROWS");           // tuning knob; 0 disables the fast path
-        const int v = e ? atoi(e) : 32;
-        return (v == 0) ? 0 : (v < 8 ? 8 : v);
-    }();
     const float* partials2 = nullptr;
     int tiles2 = 0;
-    if (vec && thermal_on && march_rows > 0 && !conf_min_only && !resampled && (!ms || (H >= 4 && W >= 4))) {
+    if (vec && thermal_on && !conf_min_only && !resampled && (!ms || (H >= 4 && W >= 4))) {
         // fast path: TMA-fed warp-marching kernel (t3d_loss_march.cu); multi-scale: the half-resolution terms run
         // first as their own pass (t3d_loss_scale2.cu) and hand their gradient to the marching kernel
         MarchArgs ma;
@@ -1118,8 +1108,7 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
             ma.dpred[v] = la.dpred[v]; ma.dconf[v] = la.dconf[v]; ma.dzp[v] = nullptr;
         }
         // multi-scale with one staged thermal plane: both scales in one pass over the rows (loss_march_ms_kernel)
-        static const bool ms_one_pass = [] { const char* e = getenv("T3D_MS_ONE_PASS"); return e ? atoi(e) != 0 : true; }();
-        const bool fused_ms = ms && ms_one_pass && (tch == 1 || replicated);
+        const bool fused_ms = ms && (tch == 1 || replicated);
         if (ms && !fused_ms) {
             Scale2Args sa;
             float* dzp = reinterpret_cast<float*>(ws + L.s2_dzp);
@@ -1137,12 +1126,13 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         }
         ma.stats[0] = stats_v[0]; ma.stats[1] = stats_v[1]; ma.partials = loss_partials; ma.queue = counter + 1;
         ma.B = B; ma.H = H; ma.W = W; ma.tch = tch; ma.stiles = la.stiles; ma.replicated = replicated;
-        // bands of march_rows rows (a band re-reads the row above and the row below it: taller = less overfetch), the
-        // last ~1/8 of the image in 8-row bands queued behind all the large ones (shorter tail of the persistent grid)
-        static const int tail_div = [] { const char* e = getenv("T3D_MARCH_TAIL"); const int v = e ? atoi(e) : 8; return v < 0 ? 0 : v; }();
+        // bands of 32 rows (a band re-reads the row above and the row below it: taller = less overfetch), the last ~1/8
+        // of the image in 8-row bands queued behind all the large ones (shorter tail of the persistent grid); other band
+        // heights and tails: DESIGN §4 experiment 12 and §5
+        constexpr int kMarchRows = 32, kMarchTailDiv = 8;
         // (one-pass multi-scale: a band brings 4 halo rows instead of 2 and must start on an even row: 16-row tail bands)
-        const int rows_l = fused_ms ? ((march_rows + 1) & ~1) : march_rows, rows_s = fused_ms ? 16 : 8;
-        const int small_rows = tail_div > 0 ? ((H / tail_div + rows_s - 1) / rows_s) * rows_s : 0;
+        const int rows_l = kMarchRows, rows_s = fused_ms ? 16 : 8;
+        const int small_rows = ((H / kMarchTailDiv + rows_s - 1) / rows_s) * rows_s;
         ma.rows_l = rows_l; ma.rows_s = rows_s;
         ma.nbands_l = (small_rows > 0) ? max(0, H - small_rows) / rows_l : (H + rows_l - 1) / rows_l;
         if (small_rows == 0) { ma.nbands_s = 0; /* the last large band may be ragged: handle it as one small band */

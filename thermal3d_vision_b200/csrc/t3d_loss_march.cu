@@ -19,7 +19,6 @@
 //    (q_y of the row above is carried, q_x of the left neighbour is shuffled),
 //    gradients are gathered (no atomics) and written once with 128-bit stores.
 #include "t3d_loss_internal.cuh"
-#include <stdlib.h>
 #include <type_traits>
 
 namespace {
@@ -757,8 +756,11 @@ __global__ void __maxnreg__((WARPS >= 12) ? 168 : 255) loss_march_ms_kernel(cons
     }
 }
 
-template <bool REP, bool BWD, int NS, int WARPS>
-int launch_ms_w(const MarchArgs& a, cudaStream_t st) {
+// 12 warps x 5 ring stages x 168 registers: registers are allocated to a CTA in units of 4 warps, so 10 or 11 warps with
+// more registers each do not launch, and 8 warps run slower (DESIGN §4, loss_march_ms_kernel)
+template <bool REP, bool BWD>
+int launch_ms(const MarchArgs& a, cudaStream_t st) {
+    constexpr int NS = 5, WARPS = 12;
     constexpr size_t smem = (size_t)WARPS * NS * StageF::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
     static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
     static bool attr_done[kT3dMaxDevices] = {};
@@ -773,19 +775,11 @@ int launch_ms_w(const MarchArgs& a, cudaStream_t st) {
     return T3D_OK;
 }
 
-template <bool REP, bool BWD>
-int launch_ms(const MarchArgs& a, cudaStream_t st) {
-    // warps x ring depth (tuning knob T3D_MS_SHAPE = 125 | 87 | 86); registers are allocated to a CTA in units of
-    // 4 warps, so 10 or 11 warps with more registers each do not launch: 12 x 168 or 8 x 255
-    static const int shape = [] { const char* e = getenv("T3D_MS_SHAPE"); return e ? atoi(e) : 125; }();
-    if (shape == 87) return launch_ms_w<REP, BWD, 7, 8>(a, st);
-    if (shape == 86) return launch_ms_w<REP, BWD, 6, 8>(a, st);
-    return launch_ms_w<REP, BWD, 5, 12>(a, st);
-}
-
-template <int TCH, bool REP, bool BWD, bool S2, int WARPS>
-int launch_w(const MarchArgs& a, cudaStream_t st) {
-    constexpr int NS = 4;
+// One persistent CTA per SM with as many warps as the register file / shared memory hold: 12, or 10 with three staged
+// thermal planes.  Fewer warps (DESIGN §4 experiment 2) or fewer CTAs (experiment 15) slow the step.
+template <int TCH, bool REP, bool BWD, bool S2>
+int launch(const MarchArgs& a, cudaStream_t st) {
+    constexpr int NS = 4, WARPS = (TCH == 3) ? 10 : 12;
     constexpr size_t smem = (size_t)WARPS * NS * Stage<TCH, S2>::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
     static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
     static bool attr_done[kT3dMaxDevices] = {};
@@ -795,26 +789,9 @@ int launch_w(const MarchArgs& a, cudaStream_t st) {
                                       cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         attr_set = true;
     }
-    // T3D_MARCH_CTAS (tuning knob): fewer persistent CTAs than SMs leave whole SMs to other streams' kernels
-    static const int env_ctas = [] { const char* e = getenv("T3D_MARCH_CTAS"); return e ? atoi(e) : 0; }();
-    const int grid = (env_ctas > 0 && env_ctas < t3d_sm_count()) ? env_ctas : t3d_sm_count();
     T3D_LAUNCH("loss_march_kernel", st,
-               loss_march_kernel<TCH, REP, BWD, S2, NS, WARPS><<<grid, WARPS * 32, smem, st>>>(a));
+               loss_march_kernel<TCH, REP, BWD, S2, NS, WARPS><<<t3d_sm_count(), WARPS * 32, smem, st>>>(a));
     return T3D_OK;
-}
-
-// Warps per CTA (one CTA per SM).  Default: as many as the register file / shared memory hold (12; 10 with three
-// staged thermal planes).  T3D_MARCH_WARPS=8 / 10 (tuning knob): fewer warps leave registers and shared memory for
-// other streams' kernels to run UNDER this DRAM-bound one.  Measured (round 2): the kernel alone 212 -> 230 us with 8
-// warps, and with the next step's sampling + resize kernels co-resident 262 us -- what the step gains by hiding them
-// it loses here (they compete for the same issue slots): not used.
-template <int TCH, bool REP, bool BWD, bool S2>
-int launch(const MarchArgs& a, cudaStream_t st) {
-    static const int env_warps = [] { const char* e = getenv("T3D_MARCH_WARPS"); return e ? atoi(e) : 0; }();
-    const int want = env_warps ? env_warps : 12;
-    if (want <= 8) return launch_w<TCH, REP, BWD, S2, 8>(a, st);
-    if (want <= 10 || TCH == 3) return launch_w<TCH, REP, BWD, S2, 10>(a, st);
-    return launch_w<TCH, REP, BWD, S2, (TCH == 3) ? 10 : 12>(a, st);
 }
 
 }  // namespace

@@ -13,8 +13,6 @@
 // (IEEE div/mul, no FMA), summed in fp64 in a fixed order (deterministic).
 #include "t3d_metrics_internal.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 using namespace t3d_metrics;
@@ -60,8 +58,10 @@ MetricsWs metrics_ws(void* base, int B, int n, int chunks) {
 }
 
 int chunks_for(int n) {
-    static const int px = [] { const char* e = getenv("T3D_METRIC_CHUNK_PX"); const int v = e ? atoi(e) : 12288; return v < 1024 ? 1024 : v; }();
-    return max(1, min(96, (n + px - 1) / px));
+    // 16 CTAs per 512x384 image: 1.15 waves instead of 1.73 with 8 192 (DESIGN §4 experiment 7); must stay below
+    // 24 576, which overflows the per-CTA candidate stage (kCtaCand)
+    constexpr int kChunkPx = 12288;
+    return max(1, min(96, (n + kChunkPx - 1) / kChunkPx));
 }
 
 struct PixelSrc {            // how to read (gt, pred, valid) of pixel i of image b

@@ -12,8 +12,6 @@
 #include <atomic>
 #include "t3d_select.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 template <typename SrcT, bool DIV65535>
@@ -530,9 +528,8 @@ thread_local int g_pre_stats_scales = 1;
 // shapes whose bands the half-resolution pass handles: even bands of <= 16 rows, W / 2 columns <= one per thread,
 // the band + two rows below fit the staging area
 static bool norm_s2_supported(int H, int W) {
-    static const bool stage_on = [] { const char* e = getenv("T3D_NORM_STAGE"); return e ? atoi(e) != 0 : true; }();
     const int rows_per = (H + kNormBands - 1) / kNormBands;
-    return stage_on && H >= 2 && W >= 8 && (W % 8) == 0 && (W / 2) <= kNormThreads && (rows_per % 2) == 0 && rows_per / 2 + 1 <= 9 /* kS2MaxPool */ &&
+    return H >= 2 && W >= 8 && (W % 8) == 0 && (W / 2) <= kNormThreads && (rows_per % 2) == 0 && rows_per / 2 + 1 <= 9 /* kS2MaxPool */ &&
            (size_t)(rows_per + 2) * W * sizeof(uint16_t) <= (size_t)kNormStageMax;
 }
 constexpr int kNormWarps = kNormThreads / 32;
@@ -964,16 +961,15 @@ int t3d_preprocess_train_u16_phase(const uint16_t* raw, int B, int src_h, int sr
             T3D_CUDA(cudaFuncSetAttribute(normalize_stats_u16_kernel<3, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutMax * 8 + kStageMax));
             nattr = true;
         }
-        static const int norm_ctas = [] { const char* e = getenv("T3D_NORM_CTAS"); const int v = e ? atoi(e) : 32; return v < 1 ? 1 : v; }();
-        static const bool norm_stage = [] { const char* e = getenv("T3D_NORM_STAGE"); return e ? atoi(e) != 0 : true; }();
+        constexpr int kNormCtasPerSm = 32;
         const int nitems = B * kNormBands;
-        const int grid = min(nitems, t3d_sm_count() * norm_ctas);
+        const int grid = min(nitems, t3d_sm_count() * kNormCtasPerSm);
         // half-resolution sums too (t3d_preprocess_set_stats_scales(2)) where the shape allows: two rows below the band
         const bool s2 = grad_stats && g_pre_stats_scales == 2 && norm_s2_supported(dst_h, dst_w);
         if (s2) T3D_REQUIRE(t3d_aligned16(nsrc), "half-resolution statistics need 16-byte aligned frames");
         const int band_rows = (dst_h + kNormBands - 1) / kNormBands + (s2 ? 2 : 1);  // + the row(s) below (gradient statistics)
         const size_t stage_bytes = (size_t)band_rows * dst_w * sizeof(uint16_t);
-        const bool staged = norm_stage && (dst_w % 8 == 0) && stage_bytes <= (size_t)kStageMax && t3d_aligned16(nsrc);
+        const bool staged = (dst_w % 8 == 0) && stage_bytes <= (size_t)kStageMax && t3d_aligned16(nsrc);
 #define T3D_NORM_LAUNCH(REP_, ST_) do { \
             if (staged) T3D_LAUNCH("normalize_stats_u16_kernel", st, (normalize_stats_u16_kernel<REP_, ST_, true><<<grid, kNormThreads, kLutMax * 8 + stage_bytes, st>>>( \
                 nsrc, percentiles, out, dst_h, dst_w, grad_stats, w.lut, w.lutmeta, nitems))); \

@@ -18,8 +18,6 @@
 #include "t3d_preprocess_internal.cuh"
 #include "t3d_select.cuh"
 
-#include <stdlib.h>
-
 namespace {
 
 constexpr int kSamp = 4096;
@@ -583,8 +581,7 @@ int t3d_launch_bracket_percentiles(const uint16_t* raw, int B, int sh, int sw, i
             int* max_ctas = max_ctas_dev[slot];
             size_t* attr_smem = attr_smem_dev[slot];
             // the dataset's 5:4 horizontal geometry: compile-time x taps (dense only: 5:4 implies scale < 2)
-            static const bool use54 = [] { const char* e = getenv("T3D_RZ_54"); return e ? atoi(e) != 0 : true; }();
-            const bool h54 = use54 && dense && sw * 4 == dw * 5 && (dw & 31) == 0;
+            const bool h54 = dense && sw * 4 == dw * 5 && (dw & 31) == 0;
             const int di = h54 ? 2 : (dense ? 1 : 0);
             const void* fn = h54 ? (const void*)resize_march_kernel<true, true> :
                              dense ? (const void*)resize_march_kernel<true, false> : (const void*)resize_march_kernel<false, false>;
@@ -598,8 +595,7 @@ int t3d_launch_bracket_percentiles(const uint16_t* raw, int B, int sh, int sw, i
             // pipeline.HotPathStep does with the metric pipeline): 2 of the 3 CTAs per SM that fit -- the registers
             // left over let the memory-bound kernels of the other stream co-reside with this issue-bound one
             // (436.6 -> 432.9 us per step); alone, 3 CTAs per SM are faster (56.7 vs 65.8 us).
-            static const int env_ctas = [] { const char* e = getenv("T3D_RZ_CTAS"); return (e && atoi(e) >= 1) ? atoi(e) : 0; }();
-            const int ctas = min(max_ctas[di], env_ctas ? env_ctas : (t3d_preprocess_shared() ? 2 : max_ctas[di]));
+            const int ctas = min(max_ctas[di], t3d_preprocess_shared() ? 2 : max_ctas[di]);
             const long long total = (long long)B * nstrips * dh;
             long long grid = (long long)t3d_sm_count() * ctas;
             if (grid * kRzWarps > total) grid = (total + kRzWarps - 1) / kRzWarps;

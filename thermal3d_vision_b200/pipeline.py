@@ -9,7 +9,6 @@ only owns buffers, streams and the (optional) data-parallel all-reduce.
 """
 from __future__ import annotations
 
-import os
 from typing import Dict, Optional
 
 import torch
@@ -91,18 +90,16 @@ class HotPathStep:
         # also means ONE planar-Z scratch: the extraction pass parks it in the L2 for the sum pass, t3d_metrics.cu.)
         # Pipelined: the metric chains of consecutive steps alternate between two streams (and two workspaces), so that
         # step i+1's extraction pass does not queue behind the tail of step i's sum pass, which the loss kernel held
-        # up (406.2 -> 403.4 us per step); T3D_MET_STREAMS=1 puts them back on one stream with one shared scratch.
-        self.met_two_streams = self.pipelined and os.environ.get("T3D_MET_STREAMS", "2") == "2"
-        if not self.met_two_streams:
+        # up (406.2 -> 403.4 us per step).
+        if not self.pipelined:
             self.met_sets[1]["workspace"] = self.met_sets[0]["workspace"]
         # Sampling ahead (pipelined steps): the two chains' sampling kernels -- one CTA per image, latency-bound, 30 us
         # of nearly idle machine at the head of every step -- are launched for step i+1 as soon as its inputs are
         # known, in their thin form, on streams of their own: they run beside step i's streaming kernels, and at the
         # gate step i+1 starts with its heavy kernels.  What they write exists per set (the preprocessing workspace;
         # for the metric chain a small state block -- its big scratch stays shared).
-        self.sample_ahead = self.pipelined and os.environ.get("T3D_SAMPLE_AHEAD", "1") != "0"
         self._primed = False
-        if self.sample_ahead:
+        if self.pipelined:
             for m in self.met_sets:
                 m["state"] = torch.empty(lib.t3d_depth_metrics_state_bytes(B), dtype=torch.uint8, device=dev)
         else:
@@ -127,7 +124,7 @@ class HotPathStep:
         self.s_loss = torch.cuda.Stream(device=dev, priority=hi_pri)
         self.s_pre = torch.cuda.Stream(device=dev, priority=min(hi_pri + 1, lo_pri))
         self.s_met = torch.cuda.Stream(device=dev, priority=lo_pri)
-        self.s_met_alt = torch.cuda.Stream(device=dev, priority=lo_pri) if self.met_two_streams else self.s_met
+        self.s_met_alt = torch.cuda.Stream(device=dev, priority=lo_pri) if self.pipelined else self.s_met
         self.s_samp_p = torch.cuda.Stream(device=dev, priority=lo_pri)
         self.s_samp_m = torch.cuda.Stream(device=dev, priority=lo_pri)
         self.ev_sp = [torch.cuda.Event() for _ in range(2)]
@@ -162,8 +159,6 @@ class HotPathStep:
         self.reduced = [True, True]     # results[i] holds the global vector of the step that last used set i
         self.step_of = [-1, -1]
         if distributed and _dist.world()[1] > 1:
-            import os
-            exchange = os.environ.get("T3D_EXCHANGE", exchange)      # tuning knob
             if exchange not in ("peer", "nccl"):
                 raise ValueError("exchange must be 'peer' or 'nccl'")
             self.exchange = exchange
@@ -254,7 +249,7 @@ class HotPathStep:
         raw_both = torch.as_strided(raw1, (2 * B,) + tuple(raw1.shape[1:]), raw1.stride(), raw1.storage_offset()) if stacked else None
         # (the first step after finish() has no step in flight to hide its sampling behind: it takes the one-call
         # form with the 1 024-thread sampling kernels, which are faster when they have the machine to themselves)
-        ahead = self.sample_ahead and self.pipelined and stacked and not self.histogram and self._primed
+        ahead = self.pipelined and stacked and not self.histogram and self._primed
         self._primed = True
         if ahead:
             # ungated, on their own streams: ordered only after the inputs and after the last user of this set's

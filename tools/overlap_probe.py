@@ -1,4 +1,4 @@
-"""Developer tool: loss kernel alone, plain step and pipelined step under the current T3D_* tuning knobs."""
+"""Developer tool: loss kernel alone, preprocessing alone, metric chain alone, plain step and pipelined step."""
 import sys, os, json
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -10,7 +10,7 @@ B, H, W = 64, 384, 512
 d = bench.make_inputs_torch(B, H, W, 0, dev)
 args = tuple(d[k] for k in bench.KEYS)
 kw = dict(alpha=0.2, edge_weight=0.5, smoothness_weight=0.3, detail_weight=0.4, multi_scale=False)
-res = {k: os.environ.get(k) for k in ("T3D_MARCH_WARPS", "T3D_METRIC_FUSED", "T3D_RZ_CTAS") if os.environ.get(k)}
+res = {}
 raw2 = torch.cat([d["raw1"], d["raw2"]])
 tb = pp.preprocess_thermal_batch(raw2, (W, H), histogram=False)
 out = {}

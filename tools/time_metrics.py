@@ -21,8 +21,7 @@ for _ in range(20):
     e0.record(); run(); e1.record(); torch.cuda.synchronize()
     ts.append(e0.elapsed_time(e1) * 1e3)
 ts.sort()
-print(f"metric chain, L2 flushed before each call: median {ts[len(ts)//2]:.1f} us  min {ts[0]:.1f} us   "
-      f"(fused={os.environ.get('T3D_METRIC_FUSED', '1')} wave={os.environ.get('T3D_METRIC_WAVE', '8')} ctas={os.environ.get('T3D_METRIC_CTAS', '3')})")
+print(f"metric chain, L2 flushed before each call: median {ts[len(ts)//2]:.1f} us  min {ts[0]:.1f} us")
 _lib.profile_begin("", 64)
 flush.fill_(1.0)
 run(); torch.cuda.synchronize()
