@@ -142,7 +142,14 @@ int t3d_loss_fwd_bwd(const float* pred1, const float* pred2,
  * kernel's loads (same ATen arithmetic), so the resampled pointmaps are never written or re-read.
  * gt1/gt2 [B,gt_h,gt_w,3]; conf1/conf2 [B,conf_h,conf_w] (NULL -> ones; conf_h x conf_w = H x W for a predicted
  * confidence, which may take a gradient, = gt_h x gt_w for a pseudo-GT confidence, which never does).
- * dpred1/dpred2 NULL -> forward only.  Runs on the general tile kernel. */
+ * dpred1/dpred2 NULL -> forward only.
+ * Kernel: a downsampled gt (gt_h >= H, gt_w >= W, gt_w % 4 == 0) with thermal on, single scale, no
+ * T3D_LOSS_CONF_MIN_ONLY, no confidence or one at the prediction's size, W % 4 == 0 and 16-byte aligned arrays runs on
+ * the TMA-fed marching kernel, which resamples the gt rows as it stages them (loss_march_rs_kernel), when a 128-pixel
+ * strip's gt source segment is at most 144 pixels (gt_w = W, e.g. 512x384 <- 512x512) -- bit-identical to
+ * t3d_interp_bilinear_f32 followed by t3d_loss_fwd_bwd.  Everything else (wider segments such as 224x224 <- 512x512,
+ * where the tile kernel measured faster; multi-scale, upsampled gt, a gt-sized confidence, unaligned data) runs on
+ * the general tile kernel. */
 int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2,
                                const float* gt1, const float* gt2, int gt_h, int gt_w,
                                const float* conf1, const float* conf2, int conf_h, int conf_w,
@@ -153,6 +160,21 @@ int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2,
                                float grad_scale,
                                float* out_sample, float* out_batch, double* out_sample_f64,
                                void* workspace, size_t workspace_bytes, void* stream);
+
+/* t3d_loss_fwd_bwd_resampled with the thermal-gradient statistics of the preprocessing (thermal_stats1/2,
+ * stats_tiles and T3D_LOSS_STATS_TWO_SCALES as in t3d_loss_fwd_bwd): when given, the statistics pass is skipped.
+ * t3d_loss_fwd_bwd_resampled is this call with NULL statistics. */
+int t3d_loss_fwd_bwd_resampled_stats(const float* pred1, const float* pred2,
+                                     const float* gt1, const float* gt2, int gt_h, int gt_w,
+                                     const float* conf1, const float* conf2, int conf_h, int conf_w,
+                                     const float* thermal1, const float* thermal2, int thermal_channels,
+                                     const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
+                                     float* dpred1, float* dpred2, float* dconf1, float* dconf2,
+                                     int B, int H, int W, int flags,
+                                     float alpha, float edge_weight, float smoothness_weight, float detail_weight,
+                                     float grad_scale,
+                                     float* out_sample, float* out_batch, double* out_sample_f64,
+                                     void* workspace, size_t workspace_bytes, void* stream);
 
 /* Scheduling hook: `cuda_event` (a cudaEvent_t, or NULL to cancel) is recorded on the stream of the NEXT
  * t3d_loss_fwd_bwd / t3d_loss_fwd call of the calling thread right behind its main kernel, i.e. BEFORE the small

@@ -41,6 +41,9 @@ _SIGNATURES = {
                          + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
     "t3d_loss_fwd_bwd_resampled": (C.c_int, [c_ptr] * 4 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int]
                                    + [c_ptr] * 4 + [C.c_int] * 4 + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
+    "t3d_loss_fwd_bwd_resampled_stats": (C.c_int, [c_ptr] * 4 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int] * 2 + [c_ptr] * 2
+                                         + [C.c_int] + [c_ptr, c_ptr, C.c_int] + [c_ptr] * 4 + [C.c_int] * 4
+                                         + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
     "t3d_loss_fwd": (C.c_int, [c_ptr] * 8 + [C.c_int] + [c_ptr, c_ptr, C.c_int] + [C.c_int] * 4 + [C.c_float] * 4
                      + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
     "t3d_loss_v1_workspace_bytes": (C.c_size_t, [C.c_int] * 3),

@@ -314,21 +314,12 @@ struct LossArgs {
     int conf_h, conf_w;           // size of the conf arrays; 0 = the prediction's size
 };
 
-// F.interpolate(mode='bilinear', align_corners=False) tap of one output coordinate (ATen: scale = in / out in fp32;
-// src = max(scale * (dst + 0.5) - 0.5, 0); i0 = (int)src; i1 = i0 + (i0 < in - 1); l1 = src - i0; l0 = 1 - l1)
-struct BTap { int i0, i1; float l0, l1; };
-__device__ __forceinline__ BTap btap(int dst, int in, float scale) {
-    const float f = fmaxf(scale * ((float)dst + 0.5f) - 0.5f, 0.f);
-    BTap t;
-    t.i0 = (int)f; t.i1 = t.i0 + ((t.i0 < in - 1) ? 1 : 0);
-    t.l1 = f - (float)t.i0; t.l0 = 1.f - t.l1;
-    return t;
-}
-// one channel-last value: l0y (l0x v00 + l1x v01) + l1y (l0x v10 + l1x v11), as interp_bilinear_kernel (t3d_preprocess.cu)
+// one channel-last value of F.interpolate(mode='bilinear', align_corners=False): taps btap, weights blerp
+// (t3d_bilinear.cuh), as interp_bilinear_kernel (t3d_preprocess.cu)
 __device__ __forceinline__ float bsample(const float* __restrict__ img, int sw, int C, int c, const BTap& ty, const BTap& tx) {
     const float v00 = __ldg(img + ((size_t)ty.i0 * sw + tx.i0) * C + c), v01 = __ldg(img + ((size_t)ty.i0 * sw + tx.i1) * C + c);
     const float v10 = __ldg(img + ((size_t)ty.i1 * sw + tx.i0) * C + c), v11 = __ldg(img + ((size_t)ty.i1 * sw + tx.i1) * C + c);
-    return ty.l0 * (tx.l0 * v00 + tx.l1 * v01) + ty.l1 * (tx.l0 * v10 + tx.l1 * v11);
+    return blerp(v00, v01, v10, v11, ty, tx);
 }
 
 template <bool MULTI>
@@ -1099,7 +1090,14 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
     int rc;
     const float* partials2 = nullptr;
     int tiles2 = 0;
-    if (vec && thermal_on && !conf_min_only && !resampled && (!ms || (H >= 4 && W >= 4))) {
+    // gt at another size, downsampled: the marching kernel resamples it as it stages the rows (loss_march_rs_kernel)
+    // when a strip's source segment is one it is faster at (gt_w ~ W); wider segments, upsampled gt, a gt-sized
+    // confidence, multi-scale: tile kernel
+    int rs_span = 0;
+    const bool march_rs = vec && thermal_on && !conf_min_only && !ms && gt_h != 0 && conf_h == 0 &&
+                          gt_h >= H && gt_w >= W && gt_w % 4 == 0 && t3d_aligned16(gt1) && t3d_aligned16(gt2) &&
+                          t3d_loss_march_rs_fits(rs_span = t3d_loss_march_rs_span(W, gt_w));
+    if (vec && thermal_on && !conf_min_only && (!resampled || march_rs) && (!ms || (H >= 4 && W >= 4))) {
         // fast path: TMA-fed warp-marching kernel (t3d_loss_march.cu); multi-scale: the half-resolution terms run
         // first as their own pass (t3d_loss_scale2.cu) and hand their gradient to the marching kernel
         MarchArgs ma;
@@ -1141,8 +1139,10 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         ma.nstrips = (W + 127) / 128;
         ma.alpha = alpha; ma.kb = la.kb; ma.kc = la.kc; ma.kE = la.kE[0]; ma.kS = la.kS[0]; ma.kD = la.kD[0];
         ma.kE2 = la.kE[1]; ma.kS2 = la.kS[1]; ma.kD2 = la.kD[1];
+        ma.gt_h = gt_h; ma.gt_w = gt_w;
         n_partials = (ma.nbands_l + ma.nbands_s) * ma.nstrips;
-        rc = fused_ms ? t3d_launch_loss_march_ms(ma, bwd, st) : t3d_launch_loss_march(ma, bwd, st);
+        rc = march_rs ? t3d_launch_loss_march_rs(ma, rs_span, bwd, st)
+           : fused_ms ? t3d_launch_loss_march_ms(ma, bwd, st) : t3d_launch_loss_march(ma, bwd, st);
     } else if (bwd) {
         if (ms) rc = vec ? launch_loss<true, true, true>(la, st) : launch_loss<true, false, true>(la, st);
         else    rc = vec ? launch_loss<false, true, true>(la, st) : launch_loss<false, false, true>(la, st);
@@ -1211,6 +1211,25 @@ int t3d_loss_fwd_bwd(const float* pred1, const float* pred2, const float* gt1, c
                      workspace, workspace_bytes, stream);
 }
 
+int t3d_loss_fwd_bwd_resampled_stats(const float* pred1, const float* pred2, const float* gt1, const float* gt2,
+                                     int gt_h, int gt_w, const float* conf1, const float* conf2, int conf_h, int conf_w,
+                                     const float* thermal1, const float* thermal2, int thermal_channels,
+                                     const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
+                                     float* dpred1, float* dpred2, float* dconf1, float* dconf2,
+                                     int B, int H, int W, int flags,
+                                     float alpha, float edge_weight, float smoothness_weight, float detail_weight,
+                                     float grad_scale, float* out_sample, float* out_batch, double* out_sample_f64,
+                                     void* workspace, size_t workspace_bytes, void* stream) {
+    T3D_REQUIRE(gt_h >= 1 && gt_w >= 1, "bad gt size");
+    T3D_REQUIRE((conf1 == nullptr && conf2 == nullptr) || (conf_h >= 1 && conf_w >= 1), "bad conf size");
+    T3D_REQUIRE(!(dconf1 || dconf2) || (conf_h == H && conf_w == W), "a confidence that takes a gradient has the prediction's size");
+    const bool bwd = dpred1 != nullptr && dpred2 != nullptr;
+    return loss_impl(bwd, pred1, pred2, gt1, gt2, conf1, conf2, thermal1, thermal2, thermal_channels,
+                     thermal_stats1, thermal_stats2, stats_tiles, dpred1, dpred2, dconf1, dconf2, B, H, W, flags, alpha,
+                     edge_weight, smoothness_weight, detail_weight, grad_scale, out_sample, out_batch, out_sample_f64,
+                     workspace, workspace_bytes, stream, gt_h, gt_w, conf1 ? conf_h : 0, conf1 ? conf_w : 0);
+}
+
 int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2, const float* gt1, const float* gt2, int gt_h, int gt_w,
                                const float* conf1, const float* conf2, int conf_h, int conf_w,
                                const float* thermal1, const float* thermal2, int thermal_channels,
@@ -1219,14 +1238,11 @@ int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2, const flo
                                float alpha, float edge_weight, float smoothness_weight, float detail_weight,
                                float grad_scale, float* out_sample, float* out_batch, double* out_sample_f64,
                                void* workspace, size_t workspace_bytes, void* stream) {
-    T3D_REQUIRE(gt_h >= 1 && gt_w >= 1, "bad gt size");
-    T3D_REQUIRE((conf1 == nullptr && conf2 == nullptr) || (conf_h >= 1 && conf_w >= 1), "bad conf size");
-    T3D_REQUIRE(!(dconf1 || dconf2) || (conf_h == H && conf_w == W), "a confidence that takes a gradient has the prediction's size");
-    const bool bwd = dpred1 != nullptr && dpred2 != nullptr;
-    return loss_impl(bwd, pred1, pred2, gt1, gt2, conf1, conf2, thermal1, thermal2, thermal_channels,
-                     nullptr, nullptr, 0, dpred1, dpred2, dconf1, dconf2, B, H, W, flags, alpha, edge_weight,
-                     smoothness_weight, detail_weight, grad_scale, out_sample, out_batch, out_sample_f64,
-                     workspace, workspace_bytes, stream, gt_h, gt_w, conf1 ? conf_h : 0, conf1 ? conf_w : 0);
+    return t3d_loss_fwd_bwd_resampled_stats(pred1, pred2, gt1, gt2, gt_h, gt_w, conf1, conf2, conf_h, conf_w,
+                                            thermal1, thermal2, thermal_channels, nullptr, nullptr, 0,
+                                            dpred1, dpred2, dconf1, dconf2, B, H, W, flags, alpha, edge_weight,
+                                            smoothness_weight, detail_weight, grad_scale, out_sample, out_batch,
+                                            out_sample_f64, workspace, workspace_bytes, stream);
 }
 
 int t3d_loss_fwd(const float* pred1, const float* pred2, const float* gt1, const float* gt2,

@@ -2,6 +2,7 @@
 // second-stage reduction) and t3d_loss_march.cu (TMA-fed warp-marching fast path).
 #pragma once
 #include "t3d_common.cuh"
+#include "t3d_bilinear.cuh"
 
 struct MarchArgs {
     const float* pred[2]; const float* gt[2]; const float* conf[2]; const float* thermal[2];
@@ -18,6 +19,7 @@ struct MarchArgs {
     float alpha, kb, kc, kE, kS, kD;
     float kE2, kS2, kD2;           // scale-2 constants of the one-pass multi-scale kernel
     const float* dzp[2];           // multi-scale: per view [B][H/2][W/2], added to d/d(pred z) of each cell's 4 pixels (or NULL)
+    int gt_h, gt_w;                // t3d_launch_loss_march_rs: size of the gt arrays (bilinearly resampled to H x W)
 };
 
 // half-resolution (scale 2) terms of the multi-scale loss as their own pass (t3d_loss_scale2.cu)
@@ -36,3 +38,10 @@ int t3d_launch_loss_scale2(const Scale2Args& a, bool bwd, cudaStream_t st);
 int t3d_launch_loss_march(const MarchArgs& a, bool bwd, cudaStream_t st);
 // multi-scale, full and half resolution in one pass (tch == 1 or replicated planes; H >= 4; even band heights)
 int t3d_launch_loss_march_ms(const MarchArgs& a, bool bwd, cudaStream_t st);
+// single scale with the gt at gt_h x gt_w, bilinearly resampled while it is staged: what t3d_launch_loss_march
+// requires, plus gt_h >= H, gt_w >= W, gt_w % 4 == 0, 16-byte aligned gt.  t3d_loss_march_rs_span: the widest gt
+// source segment (pixels) a strip stages; t3d_loss_march_rs_fits: whether the kernel takes that width (the widths
+// it measured faster than the tile kernel at).
+int t3d_loss_march_rs_span(int W, int gt_w);
+bool t3d_loss_march_rs_fits(int span);
+int t3d_launch_loss_march_rs(const MarchArgs& a, int span, bool bwd, cudaStream_t st);

@@ -30,13 +30,16 @@ constexpr float kConfMin = 1e-5f, kConfMax = 10.0f;
 constexpr int kStripPx = 128;            // 32 lanes x 4 pixels
 constexpr int kSegPx = kStripPx + 8;     // + 4-pixel halo each side (keeps 16-byte alignment of AoS rows)
 
-template <int TCH, bool S2 = false> struct Stage {
+// SEG > 0 (loss_march_rs_kernel): the gt is not staged at the prediction's size; instead the two source rows of the
+// row's bilinear y-tap, SEG pixels each (the strip's x-taps, 16-byte aligned segment), from which the lanes resample
+template <int TCH, bool S2 = false, int SEG = 0> struct Stage {
     static constexpr int kPred = 0;
     static constexpr int kGt = kSegPx * 3;
-    static constexpr int kConf = 2 * kSegPx * 3;
+    static constexpr int kConf = (SEG ? 1 : 2) * kSegPx * 3;
     static constexpr int kTh = kConf + kStripPx;
     static constexpr int kDz = kTh + TCH * kSegPx;         // multi-scale: the strip's 64 pooled-cell gradients of this row pair
-    static constexpr int kFloats = kDz + (S2 ? kStripPx / 2 : 0);     // 1352 floats (TCH = 3, single scale)
+    static constexpr int kSrc = kDz + (S2 ? kStripPx / 2 : 0);
+    static constexpr int kFloats = kSrc + 2 * SEG * 3;     // 1352 floats (TCH = 3, single scale, SEG = 0)
 };
 
 // ------------------------------------------------------------------ PTX helpers (sm_100a)
@@ -141,12 +144,44 @@ __device__ __forceinline__ void load_row(const float* __restrict__ st, int idx, 
     gray_quad<TCH, REP>(st + Stage<TCH>::kTh, idx, r.g);       // (offsets up to kTh do not depend on S2)
 }
 
+// Resampled gt (SEG > 0): the source rows staged at `src` (row i0, then row i1 at src + 3 SEG) start at source column
+// s0; output column x of the row whose y-tap is ty.
+struct RsCtx { int s0, gw; float sx; };
+template <int SEG>
+__device__ __forceinline__ float gt_rs(const float* __restrict__ src, int x, int ch, const RsCtx& rs, const BTap& ty) {
+    const BTap tx = btap(x, rs.gw, rs.sx);
+    const float* p0 = src + (tx.i0 - rs.s0) * 3 + ch;
+    const float* p1 = src + (tx.i1 - rs.s0) * 3 + ch;
+    return blerp(p0[0], p1[0], p0[SEG * 3], p1[SEG * 3], ty, tx);
+}
+// load_row with the gt resampled: columns x0 .. x0+3 (clamped to the image: lanes past its right edge compute garbage
+// that is never used, but stay inside the staged segment)
+template <int TCH, bool REP, int SEG>
+__device__ __forceinline__ void load_row_rs(const float* __restrict__ st, int idx, int x0, int xmax, const RsCtx& rs,
+                                            const BTap& ty, RowRegs& r) {
+    using St = Stage<TCH, false, SEG>;
+    const float4* p = reinterpret_cast<const float4*>(st + St::kPred + idx * 3);
+    const float4 a = p[0], b = p[1], c = p[2];
+    r.P[0] = a.x; r.P[1] = a.y; r.P[2] = a.z; r.P[3] = a.w; r.P[4] = b.x; r.P[5] = b.y; r.P[6] = b.z; r.P[7] = b.w;
+    r.P[8] = c.x; r.P[9] = c.y; r.P[10] = c.z; r.P[11] = c.w;
+#pragma unroll
+    for (int e = 0; e < 4; ++e) {
+        const int x = min(x0 + e, xmax);
+#pragma unroll
+        for (int ch = 0; ch < 3; ++ch) r.G[3 * e + ch] = gt_rs<SEG>(st + St::kSrc, x, ch, rs, ty);
+    }
+    gray_quad<TCH, REP>(st + St::kTh, idx, r.g);
+}
+
 // ------------------------------------------------------------------ kernel
 // S2: multi-scale -- the scale-2 pass (t3d_loss_scale2.cu) left 0.25 * d(loss)/d(pooled z) per 2x2 cell in a.dzp
-template <int TCH, bool REP, bool BWD, bool S2, int NS, int WARPS>
-__global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(const MarchArgs a) {
+// SEG > 0: the gt is [B, gt_h, gt_w, 3] and is bilinearly resampled to H x W as its rows are loaded from the ring
+// (loss_march_rs_kernel); everything downstream of the gt values is the same code
+template <int TCH, bool REP, bool BWD, bool S2, int SEG, int NS, int WARPS>
+__device__ __forceinline__ void march_body(const MarchArgs& a) {
     static_assert(!REP || TCH == 1, "replicated planes: one plane is staged");
-    using St = Stage<TCH, S2>;
+    static_assert(!(S2 && SEG), "multi-scale with a resampled gt runs on the tile kernel");
+    using St = Stage<TCH, S2, SEG>;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
     float* ring = reinterpret_cast<float*>(smem_raw) + (size_t)wrp * NS * St::kFloats;
@@ -168,6 +203,8 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
     const float kE = a.kE, kS2 = 2.0f * a.kS, kD = a.kD, kb = a.kb, kc = a.kc, alpha = a.alpha;
     const float alpha_ln2 = alpha * 0.69314718055994531f;
     uint32_t pos = 0;                                  // rows streamed so far by this warp (ring position)
+    const int gh = SEG ? a.gt_h : H, gw = SEG ? a.gt_w : W;
+    const float sy = SEG ? bscale(gh, H) : 1.f, sx = SEG ? bscale(gw, W) : 1.f;
 
     for (;;) {
         int task = 0;
@@ -198,9 +235,16 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
         const int idx = 4 * lane + off;                // smem pixel index of this lane's quad
 
         const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
-        const float* __restrict__ gt = a.gt[view] + (size_t)b * plane * 3;
+        const float* __restrict__ gt = a.gt[view] + (size_t)b * (size_t)gh * gw * 3;
         const float* __restrict__ conf = a.conf[view] ? a.conf[view] + (size_t)b * plane : nullptr;
         const float* __restrict__ th = a.thermal[view] + (size_t)b * (REP ? 3 : TCH) * plane;
+        // resampled gt: the strip's source segment [s0, s0 + seg_px) covers the x-taps of columns c0 .. c1-1
+        RsCtx rs = {0, gw, sx};
+        uint32_t seg_bytes = 0;
+        if (SEG) {
+            rs.s0 = btap(c0, gw, sx).i0 & ~3;
+            seg_bytes = (uint32_t)(((btap(c1 - 1, gw, sx).i1 + 4) & ~3) - rs.s0) * 12u;
+        }
         // running output pointers of this lane's quad (row i_lo; advanced by one row per iteration)
         float* dp_ptr = BWD ? a.dpred[view] + ((size_t)b * plane + (size_t)i_lo * W + j) * 3 : nullptr;
         float* dc_ptr = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane + (size_t)i_lo * W + j : nullptr;
@@ -226,7 +270,8 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
         // NaN / Inf thermal pixels make the reference loss NaN (clamp(NaN) = NaN): poison the task's sums
         const bool thermal_bad = !(inv_mx > 0.f && inv_mx <= 1.0e5f && inv_my > 0.f && inv_my <= 1.0e5f);
         const float m = (view == 0) ? 0.4f : 0.5f;       // utils/loss.py:253-256
-        const uint32_t row_bytes = (uint32_t)npx * (24u + 4u * TCH) + (conf ? (uint32_t)own_n * 4u : 0u);
+        const uint32_t row_bytes = SEG ? (uint32_t)npx * (12u + 4u * TCH) + 2u * seg_bytes + (conf ? (uint32_t)own_n * 4u : 0u)
+                                       : (uint32_t)npx * (24u + 4u * TCH) + (conf ? (uint32_t)own_n * 4u : 0u);
 
         auto issue_row = [&](int ri) {                    // lane 0 only
             const uint32_t p = pos + (uint32_t)ri;
@@ -237,7 +282,13 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
             mbar_arrive_expect_tx(bar, row_bytes + (with_dz ? (uint32_t)own_n * 2u : 0u));
             if (with_dz) bulk_g2s(st + St::kDz, dz2_strip + (size_t)((i_lo + ri) >> 1) * w2, (uint32_t)own_n * 2u, bar);
             bulk_g2s(st + St::kPred, pred + (rowpix + c0) * 3, (uint32_t)npx * 12u, bar);
-            bulk_g2s(st + St::kGt, gt + (rowpix + c0) * 3, (uint32_t)npx * 12u, bar);
+            if (SEG) {
+                const BTap ty = btap(i_lo + ri, gh, sy);
+                bulk_g2s(st + St::kSrc, gt + ((size_t)ty.i0 * gw + rs.s0) * 3, seg_bytes, bar);
+                bulk_g2s(st + St::kSrc + SEG * 3, gt + ((size_t)ty.i1 * gw + rs.s0) * 3, seg_bytes, bar);
+            } else {
+                bulk_g2s(st + St::kGt, gt + (rowpix + c0) * 3, (uint32_t)npx * 12u, bar);
+            }
             if (conf) bulk_g2s(st + St::kConf, conf + rowpix + col0, (uint32_t)own_n * 4u, bar);
 #pragma unroll
             for (int c = 0; c < TCH; ++c)
@@ -247,6 +298,14 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
         auto wait_row = [&](int ri) {
             const uint32_t p = pos + (uint32_t)ri;
             mbar_wait(&bars[p % NS], (p / NS) & 1u);
+        };
+        auto load = [&](const float* stg, int ri, RowRegs& r) {
+            if constexpr (SEG > 0) load_row_rs<TCH, REP, SEG>(stg, idx, j, W - 1, rs, btap(i_lo + ri, gh, sy), r);
+            else load_row<TCH, REP>(stg, idx, r);
+        };
+        auto gt_z = [&](const float* stg, int ri, int px) {          // gt z of smem pixel px of row i_lo + ri
+            if constexpr (SEG > 0) return gt_rs<SEG>(stg + St::kSrc, c0 + px, 2, rs, btap(i_lo + ri, gh, sy));
+            else return stg[St::kGt + px * 3 + 2];
         };
 
         if (lane == 0) {
@@ -268,7 +327,7 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
             if (has_below) {
                 wait_row(ri + 1);
                 stn = stage_of(ri + 1);
-                load_row<TCH, REP>(stn, idx, nxt);
+                load(stn, ri + 1, nxt);
             } else {                                      // zero-padded last image row: dy == 0
 #pragma unroll
                 for (int e = 0; e < 4; ++e) { nxt.P[3 * e + 2] = cur.P[3 * e + 2]; nxt.G[3 * e + 2] = cur.G[3 * e + 2]; nxt.g[e] = cur.g[e]; }
@@ -281,7 +340,7 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
             if (last_lane) {
                 if (right_in_image) {                     // the strip's right halo pixel
                     zr = st[St::kPred + (idx + 4) * 3 + 2];
-                    gzr = st[St::kGt + (idx + 4) * 3 + 2];
+                    gzr = gt_z(st, ri, idx + 4);
                     gr = gray_px<TCH, REP>(st + St::kTh, idx + 4);
                 } else { zr = cur.P[11]; gzr = cur.G[11]; gr = cur.g[3]; }
             }
@@ -306,7 +365,7 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
                 qxl = 0.f;
                 if (col0 > 0) {                           // pixel col0-1 is in the halo (idx - 1)
                     const float zl = st[St::kPred + (idx - 1) * 3 + 2];
-                    const float gzl = st[St::kGt + (idx - 1) * 3 + 2];
+                    const float gzl = gt_z(st, ri, idx - 1);
                     const float gl = gray_px<TCH, REP>(st + St::kTh, idx - 1);
                     const float gln = has_below ? gray_px<TCH, REP>(stn + St::kTh, idx - 1) : gl;
                     const float wl = edge_w(fabsf(gx[0] - gl), fabsf(gln - gl), inv_mx, inv_my, m);
@@ -366,7 +425,7 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
 
         RowRegs A, Bq;
         wait_row(0);
-        load_row<TCH, REP>(stage_of(0), idx, A);
+        load(stage_of(0), 0, A);
         const int n_cur = rb - i_lo;                      // rows that are "current" at some iteration
         for (int ri = 0; ri < n_cur; ri += 2) {           // ping-pong the two register sets: no row copies
             step(A, Bq, ri);
@@ -385,6 +444,15 @@ __global__ void __launch_bounds__((TCH == 3) ? 320 : 384, 1) loss_march_kernel(c
             o[1] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
     }
+}
+
+template <int TCH, bool REP, bool BWD, bool S2, int NS, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, 1) loss_march_kernel(const MarchArgs a) {
+    march_body<TCH, REP, BWD, S2, 0, NS, WARPS>(a);
+}
+template <int TCH, bool REP, bool BWD, int SEG, int NS, int WARPS>
+__global__ void __launch_bounds__(WARPS * 32, 1) loss_march_rs_kernel(const MarchArgs a) {
+    march_body<TCH, REP, BWD, false, SEG, NS, WARPS>(a);
 }
 
 // ====================================================================== multi-scale in ONE pass
@@ -794,7 +862,51 @@ int launch(const MarchArgs& a, cudaStream_t st) {
     return T3D_OK;
 }
 
+// Resampled gt: the marching kernel stages the gt source rows only while a strip's segment (t3d_loss_march_rs_span)
+// is at most kSegMax pixels -- gt_w = W, e.g. 512x384 <- 512x512: 364 us against 696 us on the tile kernel (batch 64).
+// Wider segments (gt_w up to 2.3 W, e.g. 224x224 <- 512x512) measured slower than the tile kernel with its fused taps
+// (92 vs 77 us at batch 8: a third of the warps of a 320-pixel ring, a grid far from full) and stay there (DESIGN §4).
+// 8 warps x 4 stages: the backward instances need ~230 registers (the taps), 8 warps of them fit an SM without spilling.
+constexpr int kSegMax = 144;
+template <int TCH, bool REP, bool BWD>
+int launch_rs(const MarchArgs& a, cudaStream_t st) {
+    constexpr int NS = 4, WARPS = 8;
+    constexpr size_t smem = (size_t)WARPS * NS * Stage<TCH, false, kSegMax>::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
+    static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
+    static bool attr_done[kT3dMaxDevices] = {};
+    bool& attr_set = attr_done[t3d_device_slot()];
+    if (!attr_set) {
+        T3D_CUDA(cudaFuncSetAttribute(loss_march_rs_kernel<TCH, REP, BWD, kSegMax, NS, WARPS>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        attr_set = true;
+    }
+    T3D_LAUNCH("loss_march_rs_kernel", st,
+               loss_march_rs_kernel<TCH, REP, BWD, kSegMax, NS, WARPS><<<t3d_sm_count(), WARPS * 32, smem, st>>>(a));
+    return T3D_OK;
+}
+
 }  // namespace
+
+// the kernel's segment arithmetic (march_body), evaluated on the host with the same roundings (btap)
+int t3d_loss_march_rs_span(int W, int gt_w) {
+    const float sx = bscale(gt_w, W);
+    int span = 0;
+    for (int col0 = 0; col0 < W; col0 += kStripPx) {
+        const int c0 = max(col0 - 4, 0), c1 = min(col0 + kStripPx + 4, W);
+        const int s0 = btap(c0, gt_w, sx).i0 & ~3, s1 = (btap(c1 - 1, gt_w, sx).i1 + 4) & ~3;
+        span = max(span, s1 - s0);
+    }
+    return span;
+}
+
+bool t3d_loss_march_rs_fits(int span) { return span <= kSegMax; }
+
+int t3d_launch_loss_march_rs(const MarchArgs& a, int span, bool bwd, cudaStream_t st) {
+    T3D_REQUIRE(t3d_loss_march_rs_fits(span), "gt segment of %d pixels does not fit the resampling kernel", span);
+    if (a.tch == 3 && a.replicated) return bwd ? launch_rs<1, true, true>(a, st) : launch_rs<1, true, false>(a, st);
+    if (a.tch == 3) return bwd ? launch_rs<3, false, true>(a, st) : launch_rs<3, false, false>(a, st);
+    return bwd ? launch_rs<1, false, true>(a, st) : launch_rs<1, false, false>(a, st);
+}
 
 // multi-scale in one pass; requires what t3d_launch_loss_march does, plus: tch == 1 or replicated planes, H >= 4,
 // rows_l and rows_s even

@@ -11,6 +11,7 @@
 #include "t3d_preprocess_internal.cuh"
 #include <atomic>
 #include "t3d_select.cuh"
+#include "t3d_bilinear.cuh"
 
 namespace {
 
@@ -818,11 +819,10 @@ __global__ void __launch_bounds__(256) fixed_range_kernel(const float* __restric
 // ------------------------------------------------------------------ torch bilinear resample (align_corners=False)
 // F.interpolate(x, size, mode='bilinear', align_corners=False) as train_thermal_dustr.py:234-271,465-481 applies
 // it to the pseudo-GT pointmaps ([H,W,3] AoS -> permuted to NCHW there; here read and written in place as AoS)
-// and confidences.  ATen: scale = in / out (fp32); src = max(scale * (dst + 0.5) - 0.5, 0); i0 = (int)src;
-// i1 = i0 + (i0 < in - 1); l1 = src - i0; l0 = 1 - l1; out = l0y (l0x v00 + l1x v01) + l1y (l0x v10 + l1x v11).
+// and confidences.  Taps and weights: btap / blerp (t3d_bilinear.cuh).
 __global__ void __launch_bounds__(256) interp_bilinear_kernel(const float* __restrict__ src, float* __restrict__ dst,
                                                               int B, int C, int sh, int sw, int dh, int dw) {
-    const float ry = (float)sh / (float)dh, rx = (float)sw / (float)dw;
+    const float ry = bscale(sh, dh), rx = bscale(sw, dw);
     const size_t total = (size_t)B * dh * dw;
     for (size_t idx = (size_t)blockIdx.x * blockDim.x + threadIdx.x; idx < total;
          idx += (size_t)gridDim.x * blockDim.x) {
@@ -830,15 +830,12 @@ __global__ void __launch_bounds__(256) interp_bilinear_kernel(const float* __res
         const size_t t = idx / dw;
         const int y = (int)(t % dh);
         const int b = (int)(t / dh);
-        const float fy = fmaxf(ry * ((float)y + 0.5f) - 0.5f, 0.f), fx = fmaxf(rx * ((float)x + 0.5f) - 0.5f, 0.f);
-        const int y0 = (int)fy, x0 = (int)fx;
-        const int y1 = y0 + ((y0 < sh - 1) ? 1 : 0), x1 = x0 + ((x0 < sw - 1) ? 1 : 0);
-        const float ly1 = fy - (float)y0, ly0 = 1.f - ly1, lx1 = fx - (float)x0, lx0 = 1.f - lx1;
+        const BTap ty = btap(y, sh, ry), tx = btap(x, sw, rx);
         const float* p = src + (size_t)b * sh * sw * C;
         for (int c = 0; c < C; ++c) {
-            const float v00 = __ldg(p + ((size_t)y0 * sw + x0) * C + c), v01 = __ldg(p + ((size_t)y0 * sw + x1) * C + c);
-            const float v10 = __ldg(p + ((size_t)y1 * sw + x0) * C + c), v11 = __ldg(p + ((size_t)y1 * sw + x1) * C + c);
-            dst[idx * C + c] = ly0 * (lx0 * v00 + lx1 * v01) + ly1 * (lx0 * v10 + lx1 * v11);
+            const float v00 = __ldg(p + ((size_t)ty.i0 * sw + tx.i0) * C + c), v01 = __ldg(p + ((size_t)ty.i0 * sw + tx.i1) * C + c);
+            const float v10 = __ldg(p + ((size_t)ty.i1 * sw + tx.i0) * C + c), v11 = __ldg(p + ((size_t)ty.i1 * sw + tx.i1) * C + c);
+            dst[idx * C + c] = blerp(v00, v01, v10, v11, ty, tx);
         }
     }
 }

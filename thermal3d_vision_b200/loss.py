@@ -88,7 +88,8 @@ def _launch(bwd, p1, p2, g1, g2, c1, c2, t1, t2, need_dconf, alpha, ew, sw, dw, 
     dp1 = dp2 = dc1 = dc2 = None
     if resampled:
         # pseudo-GT (and its confidence) at another resolution: bilinear taps inside the loss kernel's loads
-        # (train_thermal_dustr.py:234-271); a confidence at the GT's size never takes a gradient
+        # (train_thermal_dustr.py:234-271); a confidence at the GT's size never takes a gradient.  The thermal
+        # statistics of the preprocessing are honoured as on the same-size path.
         gh, gw = int(g1.shape[1]), int(g1.shape[2])
         ch, cw = (int(c1.shape[1]), int(c1.shape[2])) if c1 is not None else (H, W)
         if bwd:
@@ -101,12 +102,13 @@ def _launch(bwd, p1, p2, g1, g2, c1, c2, t1, t2, need_dconf, alpha, ew, sw, dw, 
             if need_dconf[1] and (ch, cw) == (H, W):
                 dc2 = out.get("dconf2")
                 dc2 = torch.empty(B, H, W, dtype=torch.float32, device=dev) if dc2 is None else dc2
-        rc = lib.t3d_loss_fwd_bwd_resampled(
+        rc = lib.t3d_loss_fwd_bwd_resampled_stats(
             _lib.ptr(p1), _lib.ptr(p2), _lib.ptr(g1), _lib.ptr(g2), gh, gw, _lib.ptr(c1), _lib.ptr(c2), ch, cw,
-            _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
+            _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(st1), _lib.ptr(st2), st_tiles,
+            _lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
             B, H, W, flags, alpha, ew, sw, dw, grad_scale,
             _lib.ptr(per_sample), _lib.ptr(batch), _lib.ptr(f64), _lib.ptr(ws), ws.numel(), stream)
-        _lib.check(rc, "t3d_loss_fwd_bwd_resampled")
+        _lib.check(rc, "t3d_loss_fwd_bwd_resampled_stats")
         if bwd and rescale_invalid:
             rc = lib.t3d_loss_rescale_invalid(_lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
                                               _lib.ptr(per_sample), _lib.ptr(batch), B, H, W, stream)

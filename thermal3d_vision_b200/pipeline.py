@@ -44,8 +44,11 @@ class HotPathStep:
 
     def __init__(self, B: int, H: int, W: int, raw_hw=(512, 640), device=None, multi_scale: bool = False,
                  alpha=0.2, edge_weight=0.5, smoothness_weight=0.3, detail_weight=0.4, distributed: bool = False,
-                 exchange: str = "peer", pipelined: bool = False, sobel: bool = False):
+                 exchange: str = "peer", pipelined: bool = False, sobel: bool = False, gt_hw=None):
         self.B, self.H, self.W, self.raw_hw = B, H, W, tuple(raw_hw)
+        # pseudo-GT at its stored resolution (e.g. 512x512, scripts/pseudo_gt.py:620): the loss resamples it bilinearly
+        # to (H, W) as train_thermal_dustr.py:234-271 does; None: the GT comes at (H, W)
+        self.gt_hw = tuple(int(v) for v in gt_hw) if gt_hw is not None else None
         self.sobel = bool(sobel)
         self.device = torch.device(device if device is not None else "cuda")
         if self.device.index is None:
@@ -71,6 +74,9 @@ class HotPathStep:
             "dpred1": torch.empty(B, H, W, 3, **f32), "dpred2": torch.empty(B, H, W, 3, **f32),
             "dconf1": torch.empty(B, H, W, **f32), "dconf2": torch.empty(B, H, W, **f32),
         } for _ in range(2)]
+        # what the step exposes as its loss outputs, per set: the set itself, or -- a step whose confidences take no
+        # gradient (pseudo-GT confidences at gt_hw, or none) -- the set without the dconf buffers the loss left unwritten
+        self.loss_views = list(self.loss_sets)
         # both views are preprocessed by ONE call when the caller hands them over as the two halves of a single
         # [2B,...] tensor (what run_host's staging does): outputs are halves of one buffer as well
         self.pre_sets = [{
@@ -198,9 +204,11 @@ class HotPathStep:
     def algorithmic_bytes(self) -> Dict[str, int]:
         B, n = self.B, self.H * self.W
         raw = self.raw_hw[0] * self.raw_hw[1]
+        # read 2x12 gt; with gt_hw: the source rows the bilinear y-taps touch, each read once
+        gt = 24 * n if self.gt_hw is None else 24 * rows_touched(self.gt_hw[0], self.H) * self.gt_hw[1]
         return {
-            # read 2x12 pred, 2x12 gt, 2x4 conf, 2x4 thermal (the 3 planes are replicas: one is read), write 32
-            "loss": 96 * B * n,
+            # read 2x12 pred, the gt, 2x4 conf, 2x4 thermal (the 3 planes are replicas: one is read), write 32
+            "loss": B * (72 * n + gt),
             "preprocess": 2 * B * (2 * raw + 12 * n),          # u16 frame in, 3 fp32 planes out
             "metrics": B * (12 * n + 4 * n + 64),              # pointmap (AoS sectors) + GT in, 64 B out
         }
@@ -221,13 +229,15 @@ class HotPathStep:
     def _run_device(self, raw1, raw2, pred1, pred2, gt1, gt2, conf1, conf2, gt_depth, ready, sobel_dout=None):
         size = (self.W, self.H)
         B = self.B
+        conf_grad = self._check_gt_hw(gt1, gt2, conf1, conf2) if self.gt_hw is not None else True
         lib = _lib.lib()
         main = torch.cuda.current_stream(self.device)
         i = self.calls & 1
         step_no = self.calls
         self.calls += 1
         lo, pre, met = self.loss_sets[i], self.pre_sets[i], self.met_sets[i]
-        self.loss_out, self.pre_both, self.met_out = lo, pre, met
+        self.loss_views[i] = lo if conf_grad else dict(lo, dconf1=None, dconf2=None)
+        self.loss_out, self.pre_both, self.met_out = self.loss_views[i], pre, met
         # fork: the inputs are ready on the caller's stream as of now (or, from run_host, when the H2D copies are done)
         if ready is None:
             ready = self.ev_ready[i]
@@ -330,7 +340,7 @@ class HotPathStep:
                     self.ev_main[i].record(self.s_loss)          # creates the CUDA event behind the torch object
                     self._main_recorded[i] = True
                 lib.t3d_loss_set_main_done_event(self.ev_main[i].cuda_event)
-            _loss.fused_thermal_loss_fwd_bwd(pred1, pred2, gt1, gt2, conf1, conf2, t1, t2,
+            _loss.fused_thermal_loss_fwd_bwd(pred1, pred2, gt1, gt2, conf1, conf2, t1, t2, conf_grad=conf_grad,
                                              out=lo, thermal_stats=stats, thermal_stats_scales=stats_scales,
                                              thermal_replicated=True,   # preprocess_thermal_batch wrote 3 identical planes
                                              grad_scale=_dist.global_grad_scale(self.B) if self.distributed else None,
@@ -338,7 +348,7 @@ class HotPathStep:
                                              **self.kw)
             self.s_loss.wait_event(self.ev_met[i])
             stream = _lib.current_stream_ptr()
-            grads = [_lib.ptr(lo[k]) for k in ("dpred1", "dpred2", "dconf1", "dconf2")]
+            grads = [_lib.ptr(self.loss_views[i][k]) for k in ("dpred1", "dpred2", "dconf1", "dconf2")]
             if self.exchange == "peer":
                 # reduce(step - 1) is enqueued before epilogue(step): the order that makes the two mailbox slots reusable
                 self._reduce_pending()
@@ -373,6 +383,22 @@ class HotPathStep:
             self._join(main)
         return self.result
 
+    def _check_gt_hw(self, gt1, gt2, conf1, conf2) -> bool:
+        """Shapes of a step with gt_hw; returns whether the confidences are predicted ones (at (H, W): they take a
+        gradient) -- at gt_hw they are pseudo-GT confidences (train_thermal_dustr.py:274-275), None means ones."""
+        B, H, W = self.B, self.H, self.W
+        want = (B,) + self.gt_hw + (3,)
+        for name, g in (("gt1", gt1), ("gt2", gt2)):
+            if tuple(g.shape) != want:
+                raise ValueError(f"{name} must be {want} (gt_hw={self.gt_hw}), got {tuple(g.shape)}")
+        if conf1 is None and conf2 is None:
+            return False
+        shapes = {None if c is None else tuple(c.shape) for c in (conf1, conf2)}
+        if len(shapes) != 1 or shapes.pop() not in ((B, H, W), (B,) + self.gt_hw):
+            raise ValueError(f"conf1 / conf2 must both be [B,H,W]={B, H, W} or [B,*gt_hw]={(B,) + self.gt_hw}, got "
+                             f"{None if conf1 is None else tuple(conf1.shape)} / {None if conf2 is None else tuple(conf2.shape)}")
+        return tuple(conf1.shape[1:3]) == (H, W)
+
     def _join(self, main):
         """Order `main` after every step it has not been ordered after yet (not after their pending reductions)."""
         for k in range(2):
@@ -404,7 +430,7 @@ class HotPathStep:
             with torch.cuda.graph(graph):
                 r = self.run_device(*args)
         self.pipelined = pipelined
-        sets = (self.loss_sets[0], self.pre_sets[0], self.met_sets[0])
+        sets = (self.loss_views[0], self.pre_sets[0], self.met_sets[0])
 
         def replay():
             graph.replay()
@@ -425,7 +451,7 @@ class HotPathStep:
             for i in sorted(range(2), key=lambda k: self.step_of[k]):
                 if self.reduced[i]:
                     continue
-                lo = self.loss_sets[i]
+                lo = self.loss_views[i]
                 grads = [_lib.ptr(lo[k]) for k in ("dpred1", "dpred2", "dconf1", "dconf2")]
                 if self.exchange == "peer":
                     rc = lib.t3d_mailbox_reduce(_lib.ptr(self.mailbox), world, self.step_of[i], _lib.ptr(self.results[i]),
@@ -506,6 +532,18 @@ class HotPathStep:
     @staticmethod
     def summarize(result_host: torch.Tensor) -> Dict[str, float]:
         return _dist.summarize(result_host.tolist())
+
+
+def rows_touched(src: int, dst: int) -> int:
+    """Source rows that the bilinear y-taps of `dst` output rows read (F.interpolate, align_corners=False; the fp32
+    tap arithmetic of t3d_bilinear.cuh, one rounding for scale * (y + 0.5) - 0.5)."""
+    import numpy as np
+    scale = float(np.float32(src) / np.float32(dst))
+    y = np.arange(dst, dtype=np.float64)
+    f = np.maximum((scale * (y + 0.5) - 0.5).astype(np.float32), np.float32(0))   # exact in fp64, then one rounding
+    i0 = f.astype(np.int64)
+    i1 = i0 + (i0 < src - 1)
+    return int(np.unique(np.concatenate([i0, i1])).size)
 
 
 class EvalStep:
