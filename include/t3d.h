@@ -40,7 +40,7 @@ typedef enum {
     T3D_ERR_DEVICE = -4       /* not an sm_100 device */
 } t3d_status;
 
-#define T3D_ABI_VERSION 2
+#define T3D_ABI_VERSION 3
 
 /* ------------------------------------------------------------------ library */
 int t3d_version(void);
@@ -73,7 +73,7 @@ int t3d_profile_timeline(char* names, int name_stride, double* start_ms, double*
  * batched over B independent samples (the reference is called once per sample,
  * train_thermal_dustr.py:182-293; B = 1 reproduces that call).
  *
- * Layout of `out_sample` [B][8] float32, written by t3d_loss_fwd_bwd:
+ * Layout of `out_sample` [B][8] float32:
  *   0 total  1 basic  2 edge  3 smoothness  4 detail   (unweighted components,
  *   utils/loss.py:298-303)   5 valid (1.0 iff total is finite and > 0,
  *   train_thermal_dustr.py:320)   6,7 reserved.
@@ -91,41 +91,52 @@ int t3d_profile_timeline(char* names, int name_stride, double* start_ms, double*
                                     * "original loss calculation" of train_thermal_dustr.py:278-279,305-318, which
                                     * never goes through utils/loss.py's clamp(conf, 1e-5, 10) */
 #define T3D_LOSS_STATS_TWO_SCALES 0x4 /* the caller's thermal_stats hold the half-resolution sums too ([..][2], [3];
-                                    * t3d_preprocess_set_stats_scales): with T3D_LOSS_MULTI_SCALE they are used instead
-                                    * of a statistics pass (without this flag, multi-scale ignores thermal_stats) */
+                                    * t3d_preprocess_train_u16 with stats_scales 2): with T3D_LOSS_MULTI_SCALE they are
+                                    * used instead of a statistics pass (without this flag, multi-scale ignores
+                                    * thermal_stats) */
 size_t t3d_loss_workspace_bytes(int B, int H, int W, int flags);
 
-/* Thermal-gradient statistics (utils/loss.py:184-201,239-249): for every
- * sample, view and scale, mean|Dx gray| and mean|Dy gray| over all h*w entries
- * of the zero-padded forward differences.  out_stats [B][2 views][2 scales][2]
- * float32 = the means (scale-2 slots are 0 when multi_scale == 0).
- * thermal_channels is 1 or 3 (gray = 0.299 c0 + 0.587 c1 + 0.114 c2 in fp32,
- * utils/loss.py:119-124).  In the loss entry points 3 may be OR-ed with
- * T3D_THERMAL_REPLICATED: the caller guarantees that the three planes of every
- * image are bit-identical (what enhance_thermal_contrast always returns,
- * utils/preprocessing.py:22-28; t3d_preprocess_train_u16 with out_channels 3
- * produces exactly that), so the kernel reads plane 0 only and evaluates
- * gray3(v, v, v) -- the same bits, a third of the thermal traffic. */
+/* thermal_channels is 1 or 3 (gray = 0.299 c0 + 0.587 c1 + 0.114 c2 in fp32, utils/loss.py:119-124); 3 may be
+ * OR-ed with T3D_THERMAL_REPLICATED: the caller guarantees that the three planes of every image are bit-identical
+ * (what enhance_thermal_contrast always returns, utils/preprocessing.py:22-28; t3d_preprocess_train_u16 with
+ * out_channels 3 produces exactly that), so the kernel reads plane 0 only and evaluates gray3(v, v, v) -- the same
+ * bits, a third of the thermal traffic. */
 #define T3D_THERMAL_REPLICATED 0x100
-int t3d_thermal_grad_stats(const float* thermal1, const float* thermal2, int thermal_channels,
-                           int B, int H, int W, int multi_scale,
-                           float* out_stats, void* workspace, size_t workspace_bytes,
-                           void* stream);
 
-/* Fused forward + backward.  Launches: thermal statistics -> fused tile kernel
- * (loss partials + all gradients in one pass) -> deterministic second-stage
- * reduction.  conf1/conf2 may be NULL (-> ones, utils/loss.py:85-88);
- * thermal1/thermal2 may both be NULL (-> basic loss only, utils/loss.py:116);
- * dconf1/dconf2 may be NULL (confidence without grad).
- * thermal_stats1/2 (nullable) [B][stats_tiles][4]: partial sums of |Dx gray|, |Dy gray|
- * of each thermal image as t3d_preprocess_train_u16 emits them; when given (and
- * multi_scale == 0) the statistics pass over the thermal images is skipped.
- * Gradients are those of  grad_scale * loss_b  for every sample b (pass 1/B for
- * a batch mean); t3d_loss_rescale_invalid turns them into the gradients of the
- * mean over VALID samples without a host sync. */
+/* Fused forward + backward.  Launches: thermal statistics -> main kernel (loss partials + all gradients in one
+ * pass) -> deterministic second-stage reduction.
+ *  - gt1/gt2 [B,gt_h,gt_w,3]: gt_h x gt_w == H x W is a pseudo-GT at the prediction's size.  At ANOTHER
+ *    resolution -- the normal case in training: 512x512 pseudo-GT (scripts/pseudo_gt.py:620) against 224x224
+ *    predictions -- the reference resamples it to the prediction's size first (train_thermal_dustr.py:234-271:
+ *    F.interpolate(mode='bilinear', align_corners=False) on [1,3,H,W] / [1,1,H,W] views); here the four bilinear
+ *    taps are evaluated inside the loss kernel's loads (same ATen arithmetic), so the resampled pointmaps are never
+ *    written or re-read.
+ *  - conf1/conf2 [B,conf_h,conf_w]: conf_h x conf_w = H x W for a predicted confidence, which may take a gradient,
+ *    = gt_h x gt_w for a pseudo-GT confidence, which never does.  Both NULL -> ones (utils/loss.py:85-88), and
+ *    conf_h / conf_w are ignored.
+ *  - thermal1/thermal2 may both be NULL (-> basic loss only, utils/loss.py:116).
+ *  - thermal_stats1/2 (nullable) [B][stats_tiles][4]: partial sums of |Dx gray|, |Dy gray| of each thermal image
+ *    as t3d_preprocess_train_u16 emits them; when given (and single scale, or T3D_LOSS_STATS_TWO_SCALES) the
+ *    statistics pass over the thermal images is skipped.
+ *  - dpred1/dpred2 both NULL -> forward only (no gradient writes; dconf1/dconf2 and grad_scale are ignored);
+ *    exactly one NULL is rejected.  dconf1/dconf2 may be NULL (confidence without grad).
+ *  - Gradients are those of  grad_scale * loss_b  for every sample b (pass 1/B for a batch mean);
+ *    t3d_loss_rescale_invalid turns them into the gradients of the mean over VALID samples without a host sync.
+ *  - main_done_event (a cudaEvent_t, nullable) is recorded on `stream` right behind the main kernel, i.e. BEFORE
+ *    the small second-stage reduction: the moment the machine is free again.  A caller that overlaps consecutive
+ *    steps lets the next batch's preprocessing wait for it instead of for the end of the call.  It is recorded only
+ *    when the call gets that far.
+ * Main kernel: the TMA-fed marching kernel where thermal is on, single scale or multi-scale with H, W >= 4, no
+ * T3D_LOSS_CONF_MIN_ONLY, W % 4 == 0 and 16-byte aligned arrays, and the gt either at the prediction's size or
+ * downsampled (gt_h >= H, gt_w >= W, gt_w % 4 == 0, single scale, no confidence or one at the prediction's size)
+ * with a 128-pixel strip's gt source segment of at most 144 pixels (gt_w = W, e.g. 512x384 <- 512x512): that
+ * kernel resamples the gt rows as it stages them (loss_march_rs_kernel), bit-identical to t3d_interp_bilinear_f32
+ * followed by this call at the prediction's size.  Everything else (wider segments such as 224x224 <- 512x512,
+ * where the tile kernel measured faster; upsampled gt, a gt-sized confidence, unaligned data) runs on the general
+ * tile kernel. */
 int t3d_loss_fwd_bwd(const float* pred1, const float* pred2,
-                     const float* gt1, const float* gt2,
-                     const float* conf1, const float* conf2,
+                     const float* gt1, const float* gt2, int gt_h, int gt_w,
+                     const float* conf1, const float* conf2, int conf_h, int conf_w,
                      const float* thermal1, const float* thermal2, int thermal_channels,
                      const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
                      float* dpred1, float* dpred2, float* dconf1, float* dconf2,
@@ -133,65 +144,8 @@ int t3d_loss_fwd_bwd(const float* pred1, const float* pred2,
                      float alpha, float edge_weight, float smoothness_weight, float detail_weight,
                      float grad_scale,
                      float* out_sample, float* out_batch, double* out_sample_f64,
+                     void* main_done_event,
                      void* workspace, size_t workspace_bytes, void* stream);
-
-/* The same with the pseudo-GT (and, optionally, its confidence) at ANOTHER resolution than the prediction -- the normal
- * case in training: 512x512 pseudo-GT (scripts/pseudo_gt.py:620) against 224x224 predictions.  The reference resamples
- * both to the prediction's size first (train_thermal_dustr.py:234-271: F.interpolate(mode='bilinear',
- * align_corners=False) on [1,3,H,W] / [1,1,H,W] views); here the four bilinear taps are evaluated inside the loss
- * kernel's loads (same ATen arithmetic), so the resampled pointmaps are never written or re-read.
- * gt1/gt2 [B,gt_h,gt_w,3]; conf1/conf2 [B,conf_h,conf_w] (NULL -> ones; conf_h x conf_w = H x W for a predicted
- * confidence, which may take a gradient, = gt_h x gt_w for a pseudo-GT confidence, which never does).
- * dpred1/dpred2 NULL -> forward only.
- * Kernel: a downsampled gt (gt_h >= H, gt_w >= W, gt_w % 4 == 0) with thermal on, single scale, no
- * T3D_LOSS_CONF_MIN_ONLY, no confidence or one at the prediction's size, W % 4 == 0 and 16-byte aligned arrays runs on
- * the TMA-fed marching kernel, which resamples the gt rows as it stages them (loss_march_rs_kernel), when a 128-pixel
- * strip's gt source segment is at most 144 pixels (gt_w = W, e.g. 512x384 <- 512x512) -- bit-identical to
- * t3d_interp_bilinear_f32 followed by t3d_loss_fwd_bwd.  Everything else (wider segments such as 224x224 <- 512x512,
- * where the tile kernel measured faster; multi-scale, upsampled gt, a gt-sized confidence, unaligned data) runs on
- * the general tile kernel. */
-int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2,
-                               const float* gt1, const float* gt2, int gt_h, int gt_w,
-                               const float* conf1, const float* conf2, int conf_h, int conf_w,
-                               const float* thermal1, const float* thermal2, int thermal_channels,
-                               float* dpred1, float* dpred2, float* dconf1, float* dconf2,
-                               int B, int H, int W, int flags,
-                               float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                               float grad_scale,
-                               float* out_sample, float* out_batch, double* out_sample_f64,
-                               void* workspace, size_t workspace_bytes, void* stream);
-
-/* t3d_loss_fwd_bwd_resampled with the thermal-gradient statistics of the preprocessing (thermal_stats1/2,
- * stats_tiles and T3D_LOSS_STATS_TWO_SCALES as in t3d_loss_fwd_bwd): when given, the statistics pass is skipped.
- * t3d_loss_fwd_bwd_resampled is this call with NULL statistics. */
-int t3d_loss_fwd_bwd_resampled_stats(const float* pred1, const float* pred2,
-                                     const float* gt1, const float* gt2, int gt_h, int gt_w,
-                                     const float* conf1, const float* conf2, int conf_h, int conf_w,
-                                     const float* thermal1, const float* thermal2, int thermal_channels,
-                                     const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
-                                     float* dpred1, float* dpred2, float* dconf1, float* dconf2,
-                                     int B, int H, int W, int flags,
-                                     float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                                     float grad_scale,
-                                     float* out_sample, float* out_batch, double* out_sample_f64,
-                                     void* workspace, size_t workspace_bytes, void* stream);
-
-/* Scheduling hook: `cuda_event` (a cudaEvent_t, or NULL to cancel) is recorded on the stream of the NEXT
- * t3d_loss_fwd_bwd / t3d_loss_fwd call of the calling thread right behind its main kernel, i.e. BEFORE the small
- * second-stage reduction: the moment the machine is free again.  A caller that overlaps consecutive steps lets the
- * next batch's preprocessing wait for this event instead of for the end of the call.  One-shot. */
-int t3d_loss_set_main_done_event(void* cuda_event);
-
-/* Forward only (no gradient writes): same outputs as above. */
-int t3d_loss_fwd(const float* pred1, const float* pred2,
-                 const float* gt1, const float* gt2,
-                 const float* conf1, const float* conf2,
-                 const float* thermal1, const float* thermal2, int thermal_channels,
-                 const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
-                 int B, int H, int W, int flags,
-                 float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                 float* out_sample, float* out_batch, double* out_sample_f64,
-                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* Per-sample validity fix-up (train_thermal_dustr.py:320,359): multiplies the
  * gradients of sample b by  valid_b * B / n_valid  (read from out_sample /
@@ -255,28 +209,24 @@ size_t t3d_preprocess_workspace_bytes(int B, int dst_h, int dst_w);
  * of the resized frame); percentiles [B,2] float64.
  * grad_stats (nullable) [B][t3d_preprocess_stats_tiles()][4] float32: partial sums of
  * |Dx gray|, |Dy gray| of the OUTPUT image (utils/loss.py:184-201), produced while the
- * output is written; hand them to t3d_loss_fwd_bwd to skip its statistics pass. */
+ * output is written; hand them to t3d_loss_fwd_bwd to skip its statistics pass.
+ * stats_scales (1 or 2): with 2, grad_stats[..][2], [3] also receive the sums of |Dx|, |Dy| of the 2x2
+ * average-pooled gray image (the multi-scale loss, utils/loss.py:133-174) where t3d_preprocess_stats_scales(dst_h,
+ * dst_w) returns 2; elsewhere those slots stay 0 and the loss computes its own statistics.  Pass such statistics to
+ * t3d_loss_fwd_bwd with T3D_LOSS_STATS_TWO_SCALES.
+ * shared != 0 is a scheduling hint: the caller runs other kernels concurrently (another stream), so the issue-bound
+ * resize kernel leaves registers on every SM for them.  Results do not depend on it.
+ * phase (T3D_PHASE_*, see t3d_depth_metrics; phases other than T3D_PHASE_ALL need hist == NULL): T3D_PHASE_SAMPLE
+ * launches only the window-sampling kernel (its outputs stay in `workspace`), T3D_PHASE_REST everything after it. */
 int t3d_preprocess_train_u16(const uint16_t* raw, int B, int src_h, int src_w, int dst_h, int dst_w,
                              float* out, int out_channels, unsigned int* hist, double* percentiles,
-                             float* grad_stats, void* workspace, size_t workspace_bytes, void* stream);
-/* The same call in phases (hist == NULL only; see T3D_PHASE_* at t3d_depth_metrics_phase): T3D_PHASE_SAMPLE launches
- * only the window-sampling kernel (its outputs stay in `workspace`), T3D_PHASE_REST everything after it. */
-int t3d_preprocess_train_u16_phase(const uint16_t* raw, int B, int src_h, int src_w, int dst_h, int dst_w,
-                                   float* out, int out_channels, unsigned int* hist, double* percentiles,
-                                   float* grad_stats, void* workspace, size_t workspace_bytes, int phase, void* stream);
+                             float* grad_stats, int stats_scales, int shared,
+                             void* workspace, size_t workspace_bytes, int phase, void* stream);
 /* Number of statistic partials per frame written to grad_stats (0: not available for this shape). */
 int t3d_preprocess_stats_tiles(int dst_h, int dst_w);
-/* Half-resolution statistics for the multi-scale loss (utils/loss.py:133-174).  t3d_preprocess_set_stats_scales(2)
- * makes the following t3d_preprocess_train_u16 calls OF THE CALLING THREAD also leave the sums of |Dx|, |Dy| of the
- * 2x2 average-pooled gray image in grad_stats[..][2], [3] -- where t3d_preprocess_stats_scales(dst_h, dst_w)
- * returns 2 (else those slots stay 0 and the loss computes its own statistics).  Pass such statistics to
- * t3d_loss_fwd_bwd with T3D_LOSS_STATS_TWO_SCALES. */
-int t3d_preprocess_set_stats_scales(int scales);
+/* 2 where t3d_preprocess_train_u16 with stats_scales 2 writes the half-resolution statistics, else 1 (0: no
+ * statistics for this shape). */
 int t3d_preprocess_stats_scales(int dst_h, int dst_w);
-/* Scheduling hint (process-wide, default 0): shared != 0 says the caller runs other kernels
- * concurrently with t3d_preprocess_train_u16 (another stream), so its issue-bound resize
- * kernel leaves registers on every SM for them.  Results do not depend on it. */
-int t3d_preprocess_set_shared(int shared);
 
 /* Diagnostics of the last t3d_preprocess_train_u16 call with hist == NULL on `workspace`: the number of frames
  * whose percentile ranks fell outside the sampled value windows and were found by the exact per-frame select
@@ -323,17 +273,12 @@ size_t t3d_depth_metrics_workspace_bytes(int B, int H, int W);
  * out [B][8] float32: abs_rel, sq_rel, rmse, rmse_log, acc_1, acc_2, acc_3,
  * n_valid (n_valid == 0 -> NaN,NaN,NaN,NaN,0,0,0 as :34-43); out_f64 (nullable)
  * the same in double (acc_k are float64 in numpy); out_medians (nullable)
- * [B][2] = median(gt), median(pred). */
-int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
-                      const float* gt, int gt_h, int gt_w, const unsigned char* mask,
-                      int B, int H, int W, int median_scaling,
-                      float* out, double* out_f64, float* out_medians,
-                      void* workspace, size_t workspace_bytes, void* stream);
-
-/* The two side chains in phases (extensions for pipeline.HotPathStep): T3D_PHASE_SAMPLE launches only the chain's
- * sampling kernel (the value windows / brackets the streaming passes classify against), as a thin CTA shape that fits
- * beside other kernels; T3D_PHASE_REST everything after it.  A caller that knows step i+1's inputs while step i is still
- * running samples them ahead of time, off the step's critical path; results are identical to T3D_PHASE_ALL.
+ * [B][2] = median(gt), median(pred).
+ * Phases (T3D_PHASE_ALL: the whole call; also taken by t3d_preprocess_train_u16): T3D_PHASE_SAMPLE launches only
+ * the sampling kernel (the value windows / brackets the streaming passes classify against), as a thin CTA shape
+ * that fits beside other kernels; T3D_PHASE_REST everything after it.  A caller that knows step i+1's inputs while
+ * step i is still running samples them ahead of time, off the step's critical path; results are identical to
+ * T3D_PHASE_ALL.
  * `state` (t3d_depth_metrics_state_bytes(B) bytes, 16-byte aligned, nullable): where the sampling pass leaves its
  * outputs (brackets, zeroed counters) -- per step, so that the big scratch in `workspace` can be shared by steps in
  * flight; NULL = inside `workspace`.  Both phases of a step take the same workspace / state, and T3D_PHASE_REST
@@ -344,11 +289,11 @@ int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
 #define T3D_PHASE_SAMPLE 1
 #define T3D_PHASE_REST 2
 size_t t3d_depth_metrics_state_bytes(int B);
-int t3d_depth_metrics_phase(const float* pred, int pred_stride, int pred_offset,
-                            const float* gt, int gt_h, int gt_w, const unsigned char* mask,
-                            int B, int H, int W, int median_scaling,
-                            float* out, double* out_f64, float* out_medians,
-                            void* workspace, size_t workspace_bytes, void* state, int phase, void* stream);
+int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
+                      const float* gt, int gt_h, int gt_w, const unsigned char* mask,
+                      int B, int H, int W, int median_scaling,
+                      float* out, double* out_f64, float* out_medians,
+                      void* workspace, size_t workspace_bytes, void* state, int phase, void* stream);
 
 /* Dataset accumulator of utils/metrics.py:128-136 (evaluate_thermal_depth): state[0..6] += the finite
  * per-image metrics of metrics_f64 [B][8] (t3d_depth_metrics' out_f64), state[7] += B (non-finite values are
@@ -427,13 +372,10 @@ int t3d_hwc_to_chw_clip01(const float* hwc, int H, int W, float* chw, void* stre
  *   [16..23] parameter gradients riding along (data-parallel training sums parameter gradients over the ranks --
  *   DDP's gradient all-reduce; on this path the only parameters are ThermalDUSt3R's two scalars edge_weight and
  *   temp_scale, thermal_dustr_model.py:104-107: slots 16, 17), else 0.
- * This is the one vector a data-parallel job sums over its ranks per step.
- * t3d_pack_step_result: either input may be NULL; slots 15.. are 0. */
+ * This is the one vector a data-parallel job sums over its ranks per step. */
 #define T3D_RESULT_SIZE 24
-int t3d_pack_step_result(const float* loss_per_sample, const double* metrics_f64, int B, int n_images,
-                         double* out_vec, void* stream);
-/* t3d_loss_rescale_invalid + t3d_pack_step_result as ONE launch (the tail of a training step,
- * train_thermal_dustr.py:320,359-360): out_vec as above; when some samples are invalid their
+/* t3d_loss_rescale_invalid + the packing of that vector as ONE launch (the tail of a training step,
+ * train_thermal_dustr.py:320,359-360): out_vec as above (metrics_f64 may be NULL); when some samples are invalid their
  * gradients are zeroed and the others rescaled by B / n_valid (dconf may be NULL).
  * defer_rescale != 0 (data parallel, the batch spans several ranks): only the zeroing happens here; after the
  * vector has been summed over the ranks, t3d_rescale_global multiplies this rank's gradients by

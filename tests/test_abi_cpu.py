@@ -32,14 +32,27 @@ def test_python_binding_lists_every_declared_symbol(lib_built):
     lib_built.lib()     # argtypes/restype set for each; raises if one is absent
 
 
-def test_bad_arguments_are_rejected_without_a_gpu(lib_built):
+def test_single_entry_points_reject_bad_arguments_without_a_gpu(lib_built):
     lib = lib_built.lib()
     assert lib.t3d_loss_workspace_bytes(0, 4, 4, 0) == 0
     assert lib.t3d_loss_workspace_bytes(2, 384, 512, 1) > 0
-    rc = lib.t3d_loss_fwd_bwd(*([None] * 8), 3, None, None, 0, *([None] * 4), 1, 8, 8, 0, 0.2, 0.5, 0.3, 0.4, 1.0,
-                              None, None, None, None, 0, None)
+    rc = lib.t3d_loss_fwd_bwd(*([None] * 4), 8, 8, None, None, 8, 8, None, None, 3, None, None, 0, *([None] * 4),
+                              1, 8, 8, 0, 0.2, 0.5, 0.3, 0.4, 1.0, None, None, None, None, None, 0, None)
     assert rc == -1
     assert b"NULL" in lib.t3d_last_error()
+    # the library checks its arguments before any CUDA call: dummy non-NULL pointers never get dereferenced
+    p = 256
+    rc = lib.t3d_loss_fwd_bwd(p, p, p, p, 8, 8, None, None, 8, 8, None, None, 0, None, None, 0, p, None, None, None,
+                              1, 8, 8, 0, 0.2, 0.5, 0.3, 0.4, 1.0, p, p, None, None, p, 1 << 20, None)
+    assert rc == -1                     # exactly one dpred NULL
+    assert b"NULL" in lib.t3d_last_error()
+    for stats_scales, phase, what in ((3, 0, b"stats_scales"), (1, 7, b"phase")):
+        rc = lib.t3d_preprocess_train_u16(p, 1, 8, 8, 8, 8, p, 3, None, p, None, stats_scales, 0, p, 1 << 20, phase, None)
+        assert rc == -1
+        assert what in lib.t3d_last_error()
+    rc = lib.t3d_depth_metrics(p, 1, 0, p, 8, 8, None, 1, 8, 8, 0, p, None, None, p, 1 << 20, None, 7, None)
+    assert rc == -1
+    assert b"phase" in lib.t3d_last_error()
 
 
 def _runtime_strings(py_source):

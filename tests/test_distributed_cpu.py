@@ -1,6 +1,6 @@
 """CPU, world_size 2 over gloo: the N>1 host logic (sharding by image, ONE packed all-reduce, summary)
 reproduces the single-process result.  The per-rank numbers come from the oracle (no GPU here); the
-packing layout is the one t3d_pack_step_result writes on the device (include/t3d.h)."""
+packing layout is the one t3d_step_epilogue writes on the device (include/t3d.h)."""
 import os
 import socket
 
@@ -16,7 +16,7 @@ KW = dict(alpha=0.2, edge_weight=0.5, smoothness_weight=0.3, detail_weight=0.4, 
 
 
 def _pack(rows, valid, metrics):
-    """Host mirror of the device packing (test helper, same layout as t3d_pack_step_result)."""
+    """Host mirror of the device packing (test helper, same layout as t3d_step_epilogue)."""
     from thermal3d_vision_b200.distributed import RESULT_SIZE
     v = np.zeros(RESULT_SIZE)
     for r, ok in zip(rows, valid):

@@ -153,6 +153,11 @@ def test_reference_parity(dev):
     (tot / B).backward()
     for got, ref in ((res["dpred1"], p1.grad), (res["dpred2"], p2.grad), (res["dconf1"], c1.grad), (res["dconf2"], c2.grad)):
         torch.testing.assert_close(got.cpu(), ref, rtol=1e-4, atol=1e-6)
+    # forward only (no gradient buffers, detached inputs) on the same GT gives the same numbers
+    from thermal3d_vision_b200 import loss as t3d
+    f, names = _launched(lambda: t3d.fused_thermal_loss(*args, **KW))
+    assert "loss_march_rs_kernel" in names
+    assert torch.equal(f.per_sample, res["per_sample"])
 
 
 @pytest.mark.parametrize("case", ["multi_scale", "upsampled", "gt_sized_conf", "wide_segment"])

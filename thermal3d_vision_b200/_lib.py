@@ -15,7 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libt3d_sm100.so")
 CSRC_DIR = os.path.join(_HERE, "csrc")
 
-ABI_VERSION = 2    # T3D_ABI_VERSION of include/t3d.h
+ABI_VERSION = 3    # T3D_ABI_VERSION of include/t3d.h
 _lock = threading.Lock()
 _lib = None
 
@@ -34,18 +34,9 @@ _SIGNATURES = {
     "t3d_profile_timeline": (C.c_int, [C.c_char_p, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double), C.c_int,
                                        C.POINTER(C.c_int)]),
     "t3d_loss_workspace_bytes": (C.c_size_t, [C.c_int] * 4),
-    "t3d_loss_set_main_done_event": (C.c_int, [c_ptr]),
-    "t3d_thermal_grad_stats": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
-                                         c_ptr, c_ptr, C.c_size_t, c_ptr]),
-    "t3d_loss_fwd_bwd": (C.c_int, [c_ptr] * 8 + [C.c_int] + [c_ptr, c_ptr, C.c_int] + [c_ptr] * 4 + [C.c_int] * 4
-                         + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
-    "t3d_loss_fwd_bwd_resampled": (C.c_int, [c_ptr] * 4 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int]
-                                   + [c_ptr] * 4 + [C.c_int] * 4 + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
-    "t3d_loss_fwd_bwd_resampled_stats": (C.c_int, [c_ptr] * 4 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int] * 2 + [c_ptr] * 2
-                                         + [C.c_int] + [c_ptr, c_ptr, C.c_int] + [c_ptr] * 4 + [C.c_int] * 4
-                                         + [C.c_float] * 5 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
-    "t3d_loss_fwd": (C.c_int, [c_ptr] * 8 + [C.c_int] + [c_ptr, c_ptr, C.c_int] + [C.c_int] * 4 + [C.c_float] * 4
-                     + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
+    "t3d_loss_fwd_bwd": (C.c_int, [c_ptr] * 4 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int] * 2 + [c_ptr] * 2 + [C.c_int]
+                         + [c_ptr, c_ptr, C.c_int] + [c_ptr] * 4 + [C.c_int] * 4 + [C.c_float] * 5 + [c_ptr] * 4
+                         + [c_ptr, C.c_size_t, c_ptr]),
     "t3d_loss_v1_workspace_bytes": (C.c_size_t, [C.c_int] * 3),
     "t3d_loss_v1_fwd_bwd": (C.c_int, [c_ptr] * 8 + [C.c_int] + [c_ptr] * 4 + [C.c_int] * 3 + [C.c_float] * 4
                             + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
@@ -55,14 +46,10 @@ _SIGNATURES = {
     "t3d_resize_nearest_f32": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 5 + [c_ptr]),
     "t3d_interp_bilinear_f32": (C.c_int, [c_ptr, c_ptr] + [C.c_int] * 6 + [c_ptr]),
     "t3d_preprocess_workspace_bytes": (C.c_size_t, [C.c_int] * 3),
-    "t3d_preprocess_train_u16": (C.c_int, [c_ptr] + [C.c_int] * 5 + [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr,
-                                                                    c_ptr, C.c_size_t, c_ptr]),
-    "t3d_preprocess_train_u16_phase": (C.c_int, [c_ptr] + [C.c_int] * 5 + [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr,
-                                                                          c_ptr, C.c_size_t, C.c_int, c_ptr]),
+    "t3d_preprocess_train_u16": (C.c_int, [c_ptr] + [C.c_int] * 5 + [c_ptr, C.c_int, c_ptr, c_ptr, c_ptr, C.c_int, C.c_int,
+                                                                    c_ptr, C.c_size_t, C.c_int, c_ptr]),
     "t3d_preprocess_stats_tiles": (C.c_int, [C.c_int, C.c_int]),
-    "t3d_preprocess_set_stats_scales": (C.c_int, [C.c_int]),
     "t3d_preprocess_stats_scales": (C.c_int, [C.c_int, C.c_int]),
-    "t3d_preprocess_set_shared": (C.c_int, [C.c_int]),
     "t3d_preprocess_fallback_count": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_uint), c_ptr]),
     "t3d_contrast_normalize_workspace_bytes": (C.c_size_t, [C.c_int]),
     "t3d_contrast_normalize_f32": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, C.c_int,
@@ -71,10 +58,8 @@ _SIGNATURES = {
     "t3d_fixed_range_normalize": (C.c_int, [c_ptr, c_ptr, C.c_size_t, C.c_size_t, c_ptr, C.c_int, c_ptr]),
     "t3d_depth_metrics_workspace_bytes": (C.c_size_t, [C.c_int] * 3),
     "t3d_depth_metrics": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, C.c_int, C.c_int, c_ptr]
-                          + [C.c_int] * 4 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr]),
+                          + [C.c_int] * 4 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr, C.c_int, c_ptr]),
     "t3d_depth_metrics_state_bytes": (C.c_size_t, [C.c_int]),
-    "t3d_depth_metrics_phase": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, C.c_int, C.c_int, c_ptr]
-                                + [C.c_int] * 4 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr, C.c_int, c_ptr]),
     "t3d_metrics_accumulate": (C.c_int, [c_ptr, C.c_int, c_ptr, c_ptr]),
     "t3d_pointmap_to_depth": (C.c_int, [c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "t3d_estimate_focal": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, C.c_int, c_ptr, c_ptr]),
@@ -96,7 +81,6 @@ _SIGNATURES = {
     "t3d_fire_adv_u8": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, c_ptr, c_ptr]),
     "t3d_fire_adv_compose": (C.c_int, [c_ptr, C.c_int, C.c_int, C.c_double, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr, c_ptr]),
     "t3d_hwc_to_chw_clip01": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, c_ptr]),
-    "t3d_pack_step_result": (C.c_int, [c_ptr, c_ptr, C.c_int, C.c_int, c_ptr, c_ptr]),
     "t3d_step_epilogue": (C.c_int, [c_ptr] * 7 + [C.c_int] * 5 + [c_ptr, C.c_int] + [c_ptr, c_ptr]),
     "t3d_rescale_global": (C.c_int, [c_ptr] * 6 + [C.c_int] * 3 + [c_ptr]),
     "t3d_mailbox_bytes": (C.c_size_t, []),

@@ -277,20 +277,6 @@ __global__ void __launch_bounds__(kSMWarps * 32, (MODE == 1) ? 3 : 6) thermal_st
         *reinterpret_cast<float4*>(a.partials + (((size_t)view * a.B + b) * per_img + t) * 4) = make_float4(s[0], s[1], s[2], s[3]);
 }
 
-// out_stats[B][2][2][2] = means (public API of t3d_thermal_grad_stats)
-__global__ void thermal_stats_finalize_kernel(const float* __restrict__ partials, int stiles, int B,
-                                              int H, int W, int multi, float* __restrict__ out) {
-    const int img = blockIdx.x;      // 2 b + view
-    const int k = threadIdx.x;  // 0..3
-    if (k >= 4) return;
-    double s = 0.0;
-    const size_t base = ((size_t)(img & 1) * B + (img >> 1)) * stiles;
-    for (int t = 0; t < stiles; ++t) s += (double)partials[(base + t) * 4 + k];
-    const double n1 = (double)H * W, n2 = (double)(H >> 1) * (W >> 1);
-    double m = (k < 2) ? s / n1 : ((multi && n2 > 0) ? s / n2 : 0.0);
-    out[(size_t)img * 4 + k] = (float)m;
-}
-
 // ------------------------------------------------------------------ fused loss tile kernel
 constexpr int kTH = 16, kTW = 128, kThreads = 256;
 constexpr int kPW = kTW + 8;          // raw plane row stride: col j -> c = j - j0 + 4
@@ -936,7 +922,7 @@ struct WsLayout {
     int sm_bands, sm_strips;           // work items per image-view of the marching statistics kernel
 };
 
-WsLayout ws_layout(int B, int H, int W, int multi = 0) {
+WsLayout ws_layout(int B, int H, int W, int multi) {
     WsLayout L;
     L.stiles_x = (W + kSTW - 1) / kSTW; L.stiles_y = (H + kSTH - 1) / kSTH;
     L.tiles_x = (W + kTW - 1) / kTW;    L.tiles_y = (H + kTH - 1) / kTH;
@@ -958,9 +944,6 @@ WsLayout ws_layout(int B, int H, int W, int multi = 0) {
 }
 
 inline float __int_as_float_host(unsigned int u) { float f; memcpy(&f, &u, sizeof(f)); return f; }
-
-// optional event recorded right behind the main (marching / tile) kernel of the next loss call of this thread
-thread_local cudaEvent_t g_main_done_event = nullptr;
 
 int check_dims(int B, int H, int W) {
     T3D_REQUIRE(B >= 1 && H >= 1 && W >= 1, "bad dims B=%d H=%d W=%d", B, H, W);
@@ -1020,9 +1003,8 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
               const float* conf1, const float* conf2, const float* thermal1, const float* thermal2,
               int tch, const float* ustats1, const float* ustats2, int ustats_tiles, float* dpred1, float* dpred2, float* dconf1, float* dconf2,
               int B, int H, int W, int flags, float alpha, float ew, float sw, float dw, float gscale,
-              float* out_sample, float* out_batch, double* out_f64,
-              void* workspace, size_t ws_bytes, void* stream,
-              int gt_h = 0, int gt_w = 0, int conf_h = 0, int conf_w = 0) {
+              float* out_sample, float* out_batch, double* out_f64, cudaEvent_t main_done,
+              void* workspace, size_t ws_bytes, void* stream, int gt_h, int gt_w, int conf_h, int conf_w) {
     if (int rc = check_dims(B, H, W)) return rc;
     T3D_REQUIRE((flags & ~(T3D_LOSS_MULTI_SCALE | T3D_LOSS_CONF_MIN_ONLY | T3D_LOSS_STATS_TWO_SCALES)) == 0, "unknown loss flags 0x%x", flags);
     if (gt_h == H && gt_w == W) gt_h = gt_w = 0;                    // same size: direct reads
@@ -1151,10 +1133,7 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         else    rc = vec ? launch_loss<false, true, false>(la, st) : launch_loss<false, false, false>(la, st);
     }
     if (rc) return rc;
-    if (g_main_done_event) {            // t3d_loss_set_main_done_event: lets a caller overlap the second stage with other work
-        T3D_CUDA(cudaEventRecord(g_main_done_event, st));
-        g_main_done_event = nullptr;
-    }
+    if (main_done) T3D_CUDA(cudaEventRecord(main_done, st));   // lets a caller overlap the second stage with other work
 
     FinalizeArgs fa;
     fa.partials = loss_partials; fa.out_sample = out_sample; fa.out_batch = out_batch; fa.out_f64 = out_f64;
@@ -1170,93 +1149,32 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
 // ====================================================================== C ABI
 extern "C" {
 
-int t3d_loss_set_main_done_event(void* cuda_event) {
-    g_main_done_event = reinterpret_cast<cudaEvent_t>(cuda_event);
-    return T3D_OK;
-}
-
 size_t t3d_loss_workspace_bytes(int B, int H, int W, int flags) {
     if (B < 1 || H < 1 || W < 1) return 0;
     return ws_layout(B, H, W, (flags & T3D_LOSS_MULTI_SCALE) ? 1 : 0).total;
 }
 
-int t3d_thermal_grad_stats(const float* thermal1, const float* thermal2, int thermal_channels,
-                           int B, int H, int W, int multi_scale, float* out_stats,
-                           void* workspace, size_t workspace_bytes, void* stream) {
-    if (int rc = check_dims(B, H, W)) return rc;
-    T3D_REQUIRE(thermal1 && thermal2 && out_stats && workspace, "NULL pointer");
-    T3D_REQUIRE(thermal_channels == 1 || thermal_channels == 3, "thermal_channels must be 1 or 3");
-    const WsLayout L = ws_layout(B, H, W);
-    if (workspace_bytes < L.total) { t3d_set_error("workspace too small"); return T3D_ERR_WORKSPACE; }
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    float* partials = reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + L.stats_partials);
-    int stiles = 0;
-    if (int rc = run_stats(thermal1, thermal2, thermal_channels, B, H, W, multi_scale, partials, L, st, 0, &stiles)) return rc;
-    T3D_LAUNCH("thermal_stats_finalize_kernel", st, thermal_stats_finalize_kernel<<<B * 2, 32, 0, st>>>(partials, stiles, B, H, W, multi_scale, out_stats));
-    return T3D_OK;
-}
-
-int t3d_loss_fwd_bwd(const float* pred1, const float* pred2, const float* gt1, const float* gt2,
-                     const float* conf1, const float* conf2,
+int t3d_loss_fwd_bwd(const float* pred1, const float* pred2, const float* gt1, const float* gt2, int gt_h, int gt_w,
+                     const float* conf1, const float* conf2, int conf_h, int conf_w,
                      const float* thermal1, const float* thermal2, int thermal_channels,
                      const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
                      float* dpred1, float* dpred2, float* dconf1, float* dconf2,
-                     int B, int H, int W, int multi_scale,
+                     int B, int H, int W, int flags,
                      float alpha, float edge_weight, float smoothness_weight, float detail_weight,
                      float grad_scale, float* out_sample, float* out_batch, double* out_sample_f64,
-                     void* workspace, size_t workspace_bytes, void* stream) {
-    return loss_impl(true, pred1, pred2, gt1, gt2, conf1, conf2, thermal1, thermal2, thermal_channels,
-                     thermal_stats1, thermal_stats2, stats_tiles, dpred1, dpred2, dconf1, dconf2, B, H, W, multi_scale, alpha, edge_weight,
-                     smoothness_weight, detail_weight, grad_scale, out_sample, out_batch, out_sample_f64,
-                     workspace, workspace_bytes, stream);
-}
-
-int t3d_loss_fwd_bwd_resampled_stats(const float* pred1, const float* pred2, const float* gt1, const float* gt2,
-                                     int gt_h, int gt_w, const float* conf1, const float* conf2, int conf_h, int conf_w,
-                                     const float* thermal1, const float* thermal2, int thermal_channels,
-                                     const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
-                                     float* dpred1, float* dpred2, float* dconf1, float* dconf2,
-                                     int B, int H, int W, int flags,
-                                     float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                                     float grad_scale, float* out_sample, float* out_batch, double* out_sample_f64,
-                                     void* workspace, size_t workspace_bytes, void* stream) {
+                     void* main_done_event, void* workspace, size_t workspace_bytes, void* stream) {
+    T3D_REQUIRE((dpred1 == nullptr) == (dpred2 == nullptr), "dpred1 / dpred2: both or neither may be NULL");
+    const bool bwd = dpred1 != nullptr;
+    if (!bwd) { dconf1 = dconf2 = nullptr; grad_scale = 1.0f; }          // forward only: no gradient writes
+    if (!conf1 && !conf2) { conf_h = H; conf_w = W; }                   // ones
     T3D_REQUIRE(gt_h >= 1 && gt_w >= 1, "bad gt size");
-    T3D_REQUIRE((conf1 == nullptr && conf2 == nullptr) || (conf_h >= 1 && conf_w >= 1), "bad conf size");
+    T3D_REQUIRE(conf_h >= 1 && conf_w >= 1, "bad conf size");
     T3D_REQUIRE(!(dconf1 || dconf2) || (conf_h == H && conf_w == W), "a confidence that takes a gradient has the prediction's size");
-    const bool bwd = dpred1 != nullptr && dpred2 != nullptr;
     return loss_impl(bwd, pred1, pred2, gt1, gt2, conf1, conf2, thermal1, thermal2, thermal_channels,
                      thermal_stats1, thermal_stats2, stats_tiles, dpred1, dpred2, dconf1, dconf2, B, H, W, flags, alpha,
                      edge_weight, smoothness_weight, detail_weight, grad_scale, out_sample, out_batch, out_sample_f64,
-                     workspace, workspace_bytes, stream, gt_h, gt_w, conf1 ? conf_h : 0, conf1 ? conf_w : 0);
-}
-
-int t3d_loss_fwd_bwd_resampled(const float* pred1, const float* pred2, const float* gt1, const float* gt2, int gt_h, int gt_w,
-                               const float* conf1, const float* conf2, int conf_h, int conf_w,
-                               const float* thermal1, const float* thermal2, int thermal_channels,
-                               float* dpred1, float* dpred2, float* dconf1, float* dconf2,
-                               int B, int H, int W, int flags,
-                               float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                               float grad_scale, float* out_sample, float* out_batch, double* out_sample_f64,
-                               void* workspace, size_t workspace_bytes, void* stream) {
-    return t3d_loss_fwd_bwd_resampled_stats(pred1, pred2, gt1, gt2, gt_h, gt_w, conf1, conf2, conf_h, conf_w,
-                                            thermal1, thermal2, thermal_channels, nullptr, nullptr, 0,
-                                            dpred1, dpred2, dconf1, dconf2, B, H, W, flags, alpha, edge_weight,
-                                            smoothness_weight, detail_weight, grad_scale, out_sample, out_batch,
-                                            out_sample_f64, workspace, workspace_bytes, stream);
-}
-
-int t3d_loss_fwd(const float* pred1, const float* pred2, const float* gt1, const float* gt2,
-                 const float* conf1, const float* conf2,
-                 const float* thermal1, const float* thermal2, int thermal_channels,
-                 const float* thermal_stats1, const float* thermal_stats2, int stats_tiles,
-                 int B, int H, int W, int multi_scale,
-                 float alpha, float edge_weight, float smoothness_weight, float detail_weight,
-                 float* out_sample, float* out_batch, double* out_sample_f64,
-                 void* workspace, size_t workspace_bytes, void* stream) {
-    return loss_impl(false, pred1, pred2, gt1, gt2, conf1, conf2, thermal1, thermal2, thermal_channels,
-                     thermal_stats1, thermal_stats2, stats_tiles, nullptr, nullptr, nullptr, nullptr, B, H, W, multi_scale, alpha, edge_weight,
-                     smoothness_weight, detail_weight, 1.0f, out_sample, out_batch, out_sample_f64,
-                     workspace, workspace_bytes, stream);
+                     reinterpret_cast<cudaEvent_t>(main_done_event), workspace, workspace_bytes, stream,
+                     gt_h, gt_w, conf_h, conf_w);
 }
 
 static int scale_common(int mode, float* dpred1, float* dpred2, float* dconf1, float* dconf2,

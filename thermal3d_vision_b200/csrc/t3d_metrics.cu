@@ -809,16 +809,7 @@ int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
                       const float* gt, int gt_h, int gt_w, const unsigned char* mask,
                       int B, int H, int W, int median_scaling,
                       float* out, double* out_f64, float* out_medians,
-                      void* workspace, size_t workspace_bytes, void* stream) {
-    return t3d_depth_metrics_phase(pred, pred_stride, pred_offset, gt, gt_h, gt_w, mask, B, H, W, median_scaling,
-                                   out, out_f64, out_medians, workspace, workspace_bytes, nullptr, T3D_PHASE_ALL, stream);
-}
-
-int t3d_depth_metrics_phase(const float* pred, int pred_stride, int pred_offset,
-                            const float* gt, int gt_h, int gt_w, const unsigned char* mask,
-                            int B, int H, int W, int median_scaling,
-                            float* out, double* out_f64, float* out_medians,
-                            void* workspace, size_t workspace_bytes, void* state, int phase, void* stream) {
+                      void* workspace, size_t workspace_bytes, void* state, int phase, void* stream) {
     T3D_REQUIRE(phase == T3D_PHASE_ALL || phase == T3D_PHASE_SAMPLE || phase == T3D_PHASE_REST, "bad phase %d", phase);
     T3D_REQUIRE(pred && gt && (out || phase == T3D_PHASE_SAMPLE) && workspace, "NULL pointer");
     T3D_REQUIRE(B >= 1 && H >= 1 && W >= 1 && gt_h >= 1 && gt_w >= 1, "bad dims");

@@ -8,51 +8,6 @@
 
 namespace {
 
-__global__ void __launch_bounds__(128) pack_step_result_kernel(const float* __restrict__ loss_per_sample,
-                                                               const double* __restrict__ metrics_f64, int B,
-                                                               int n_images, double* __restrict__ out) {
-    __shared__ double red[4][14];
-    const int tid = threadIdx.x;
-    double v[14];
-#pragma unroll
-    for (int k = 0; k < 14; ++k) v[k] = 0.0;
-    if (loss_per_sample) {
-        for (int b = tid; b < B; b += 128) {
-            const float* o = loss_per_sample + (size_t)b * T3D_LOSS_OUT_STRIDE;
-            if (o[5] != 0.f) {
-#pragma unroll
-                for (int k = 0; k < 5; ++k) v[k] += (double)o[k];
-                v[5] += 1.0;
-            }
-        }
-    }
-    if (metrics_f64) {
-        for (int b = tid; b < n_images; b += 128) {
-            const double* m = metrics_f64 + (size_t)b * 8;
-#pragma unroll
-            for (int k = 0; k < 7; ++k) if (isfinite(m[k])) v[7 + k] += m[k];
-        }
-    }
-    // fixed butterfly per warp, fixed order over the 4 warps: deterministic
-    const int lane = tid & 31, wrp = tid >> 5;
-#pragma unroll
-    for (int k = 0; k < 14; ++k) {
-        const double r = warp_sum(v[k]);
-        if (lane == 0) red[wrp][k] = r;
-    }
-    __syncthreads();
-    if (tid < 14) red[0][tid] = (red[0][tid] + red[1][tid]) + (red[2][tid] + red[3][tid]);
-    __syncthreads();
-    if (tid < T3D_RESULT_SIZE) {
-        double r;
-        if (tid == 6) r = loss_per_sample ? (double)B : 0.0;
-        else if (tid == 14) r = metrics_f64 ? (double)n_images : 0.0;
-        else if (tid >= 15) r = 0.0;
-        else r = red[0][tid];
-        out[tid] = r;
-    }
-}
-
 // pack + the validity fix-up of the loss gradients (scale_grads_kernel<0> of t3d_loss.cu) as ONE launch: block 0
 // packs, every block then checks the batch's valid count and returns at once when all samples are valid.
 // Peer-memory exchange of the packed vector (one process per GPU on one NVLink / NVSwitch node): every rank owns a
@@ -280,15 +235,5 @@ extern "C" int t3d_rescale_global(float* dpred1, float* dpred2, float* dconf1, f
     a.out_sample = loss_per_sample; a.B = B; a.plane = (size_t)H * W;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     T3D_LAUNCH("rescale_global_kernel", st, rescale_global_kernel<<<t3d_sm_count() * 4, 128, 0, st>>>(a));
-    return T3D_OK;
-}
-
-extern "C" int t3d_pack_step_result(const float* loss_per_sample, const double* metrics_f64, int B, int n_images,
-                                    double* out16, void* stream) {
-    T3D_REQUIRE(out16, "NULL pointer");
-    T3D_REQUIRE(B >= 0 && n_images >= 0, "bad dims");
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    T3D_LAUNCH("pack_step_result_kernel", st,
-               pack_step_result_kernel<<<1, 128, 0, st>>>(loss_per_sample, metrics_f64, B, n_images, out16));
     return T3D_OK;
 }

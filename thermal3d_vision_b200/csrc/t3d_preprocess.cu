@@ -9,7 +9,6 @@
 // numpy/OpenCV (IPP off): no FMA contraction in the interpolation, fp64 in
 // the normalisation, integer histograms.
 #include "t3d_preprocess_internal.cuh"
-#include <atomic>
 #include "t3d_select.cuh"
 #include "t3d_bilinear.cuh"
 
@@ -524,8 +523,6 @@ __global__ void __launch_bounds__(256) normalize_u16_kernel(const uint16_t* __re
 constexpr int kNormBands = 24;       // CTAs per frame == statistic partials per frame (T3D_STATS_TILES)
 constexpr int kNormThreads = 256;
 constexpr int kNormStageMax = 24 * 1024;  // staged band bytes: LUT 32 KB + band <= 56 KB per CTA, 4 CTAs per SM
-// t3d_preprocess_set_stats_scales: 2 = the next calls of this thread also leave the half-resolution sums in grad_stats
-thread_local int g_pre_stats_scales = 1;
 // shapes whose bands the half-resolution pass handles: even bands of <= 16 rows, W / 2 columns <= one per thread,
 // the band + two rows below fit the staging area
 static bool norm_s2_supported(int H, int W) {
@@ -880,15 +877,10 @@ size_t t3d_preprocess_workspace_bytes(int B, int dst_h, int dst_w) {
 
 int t3d_preprocess_train_u16(const uint16_t* raw, int B, int src_h, int src_w, int dst_h, int dst_w,
                              float* out, int out_channels, unsigned int* hist, double* percentiles,
-                             float* grad_stats, void* workspace, size_t workspace_bytes, void* stream) {
-    return t3d_preprocess_train_u16_phase(raw, B, src_h, src_w, dst_h, dst_w, out, out_channels, hist, percentiles,
-                                          grad_stats, workspace, workspace_bytes, T3D_PHASE_ALL, stream);
-}
-
-int t3d_preprocess_train_u16_phase(const uint16_t* raw, int B, int src_h, int src_w, int dst_h, int dst_w,
-                                   float* out, int out_channels, unsigned int* hist, double* percentiles,
-                                   float* grad_stats, void* workspace, size_t workspace_bytes, int phase, void* stream) {
+                             float* grad_stats, int stats_scales, int shared,
+                             void* workspace, size_t workspace_bytes, int phase, void* stream) {
     T3D_REQUIRE(phase == T3D_PHASE_ALL || phase == T3D_PHASE_SAMPLE || phase == T3D_PHASE_REST, "bad phase %d", phase);
+    T3D_REQUIRE(stats_scales == 1 || stats_scales == 2, "stats_scales must be 1 or 2, got %d", stats_scales);
     T3D_REQUIRE(phase == T3D_PHASE_ALL || hist == nullptr, "phases are a feature of the sampled-window path (hist == NULL)");
     T3D_REQUIRE(raw && out && percentiles && workspace, "NULL pointer");
     T3D_REQUIRE(B >= 1 && src_h >= 1 && src_w >= 1 && dst_h >= 1 && dst_w >= 1, "bad dims");
@@ -909,7 +901,7 @@ int t3d_preprocess_train_u16_phase(const uint16_t* raw, int B, int src_h, int sr
     const int rep3 = (out_channels == 3);
     if (hist == nullptr) {
         // percentiles from sampled value windows: no per-pixel histogram atomic (t3d_preprocess_bracket.cu)
-        if (int rc = t3d_launch_bracket_percentiles(raw, B, src_h, src_w, dst_h, dst_w, same, w, rep3, percentiles, st, phase)) return rc;
+        if (int rc = t3d_launch_bracket_percentiles(raw, B, src_h, src_w, dst_h, dst_w, same, w, rep3, percentiles, shared != 0, phase, st)) return rc;
         if (phase == T3D_PHASE_SAMPLE) return T3D_OK;
     } else {
         // exact 65 536-bin histogram (an output) -> percentiles
@@ -961,8 +953,8 @@ int t3d_preprocess_train_u16_phase(const uint16_t* raw, int B, int src_h, int sr
         constexpr int kNormCtasPerSm = 32;
         const int nitems = B * kNormBands;
         const int grid = min(nitems, t3d_sm_count() * kNormCtasPerSm);
-        // half-resolution sums too (t3d_preprocess_set_stats_scales(2)) where the shape allows: two rows below the band
-        const bool s2 = grad_stats && g_pre_stats_scales == 2 && norm_s2_supported(dst_h, dst_w);
+        // half-resolution sums too (stats_scales == 2) where the shape allows: two rows below the band
+        const bool s2 = grad_stats && stats_scales == 2 && norm_s2_supported(dst_h, dst_w);
         if (s2) T3D_REQUIRE(t3d_aligned16(nsrc), "half-resolution statistics need 16-byte aligned frames");
         const int band_rows = (dst_h + kNormBands - 1) / kNormBands + (s2 ? 2 : 1);  // + the row(s) below (gradient statistics)
         const size_t stage_bytes = (size_t)band_rows * dst_w * sizeof(uint16_t);
@@ -996,15 +988,6 @@ int t3d_preprocess_fallback_count(const void* workspace, int B, int dst_h, int d
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     T3D_CUDA(cudaMemcpyAsync(count_host, w.brhist + (size_t)B * 2 * kBrSlots, sizeof(unsigned int), cudaMemcpyDeviceToHost, st));
     T3D_CUDA(cudaStreamSynchronize(st));
-    return T3D_OK;
-}
-
-static std::atomic<int> g_pre_shared{0};
-int t3d_preprocess_set_shared(int shared) { g_pre_shared.store(shared ? 1 : 0, std::memory_order_relaxed); return T3D_OK; }
-
-int t3d_preprocess_set_stats_scales(int scales) {
-    T3D_REQUIRE(scales == 1 || scales == 2, "scales must be 1 or 2");
-    g_pre_stats_scales = scales;
     return T3D_OK;
 }
 
@@ -1108,5 +1091,3 @@ int t3d_interp_bilinear_f32(const float* src, float* dst, int B, int channels_la
 }
 
 }  // extern "C"
-
-bool t3d_preprocess_shared() { return g_pre_shared.load(std::memory_order_relaxed) != 0; }

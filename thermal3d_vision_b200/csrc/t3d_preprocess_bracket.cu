@@ -553,7 +553,7 @@ percentile_from_brackets_kernel(const uint16_t* __restrict__ frames, int n, cons
 }  // namespace
 
 int t3d_launch_bracket_percentiles(const uint16_t* raw, int B, int sh, int sw, int dh, int dw, bool same,
-                                   const PreWs& w, int rep3, double* percentiles, cudaStream_t st, int phase) {
+                                   const PreWs& w, int rep3, double* percentiles, bool shared, int phase, cudaStream_t st) {
     const int n = dh * dw;
     if (phase == T3D_PHASE_SAMPLE) {            // ahead of time, beside other kernels: the thin form
         T3D_LAUNCH("bracket_sample_kernel", st, bracket_sample_kernel<256><<<B, 256, 0, st>>>(
@@ -591,11 +591,11 @@ int t3d_launch_bracket_percentiles(const uint16_t* raw, int B, int sh, int sw, i
                 T3D_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&max_ctas[di], fn, kRzThreads, smem));
                 if (max_ctas[di] < 1) max_ctas[di] = 1;
             }
-            // Shared machine (t3d_preprocess_set_shared(1): the caller runs other kernels concurrently, as
+            // Shared machine (`shared`: the caller runs other kernels concurrently, as
             // pipeline.HotPathStep does with the metric pipeline): 2 of the 3 CTAs per SM that fit -- the registers
             // left over let the memory-bound kernels of the other stream co-reside with this issue-bound one
             // (436.6 -> 432.9 us per step); alone, 3 CTAs per SM are faster (56.7 vs 65.8 us).
-            const int ctas = min(max_ctas[di], t3d_preprocess_shared() ? 2 : max_ctas[di]);
+            const int ctas = min(max_ctas[di], shared ? 2 : max_ctas[di]);
             const long long total = (long long)B * nstrips * dh;
             long long grid = (long long)t3d_sm_count() * ctas;
             if (grid * kRzWarps > total) grid = (total + kRzWarps - 1) / kRzWarps;

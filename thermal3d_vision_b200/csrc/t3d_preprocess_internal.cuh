@@ -72,8 +72,6 @@ __device__ __forceinline__ void build_norm_lut(int b, double p2, double p98, int
     if (threadIdx.x == 0) lutmeta[b] = make_int2(lom1, use ? range : 0);
 }
 
-bool t3d_preprocess_shared();      // t3d_preprocess_set_shared(): other kernels run concurrently with the preprocessing
-
 // ------------------------------------------------------------------ percentile brackets (t3d_preprocess_bracket.cu)
 constexpr int kBrBins = 2048;        // bins of each windowed histogram (p2 window, p98 window)
 constexpr int kBrSlots = kBrBins + 32;  // + the below / above slot (t3d_preprocess_bracket.cu: kBrStride)
@@ -111,5 +109,6 @@ static inline PreWs pre_ws_layout(void* base, int B, int dh, int dw) {
 // around the p2 / p98 ranks -> one pass that resizes, counts the pixels below each bracket and histograms only
 // the few percent inside -> exact order statistics, np.percentile lerp, normalisation LUT.
 // `same` : source and destination sizes are equal (no resize; `resized` is not written, the raw frame is used).
+// `shared`: other kernels run concurrently with the preprocessing (t3d_preprocess_train_u16's `shared`).
 int t3d_launch_bracket_percentiles(const uint16_t* raw, int B, int sh, int sw, int dh, int dw, bool same,
-                                   const PreWs& w, int rep3, double* percentiles, cudaStream_t st, int phase = 0 /* T3D_PHASE_* */);
+                                   const PreWs& w, int rep3, double* percentiles, bool shared, int phase, cudaStream_t st);

@@ -2,7 +2,7 @@
 
 The path shards by image: rank r owns a contiguous slice of the batch / dataset and runs the
 kernels on it with no data-path collective.  The only exchange per step is ONE all-reduce (SUM)
-of the packed result vector (RESULT_SIZE doubles) that ``t3d_pack_step_result`` produces on the device
+of the packed result vector (RESULT_SIZE doubles) that ``t3d_step_epilogue`` produces on the device
 (SURVEY.md section 8e): sums of valid losses / components / counts and sums of finite metrics /
 image count, i.e. exactly the accumulators of train_thermal_dustr.py:320,359 and
 utils/metrics.py:128-136.  Gradients w.r.t. pointmaps stay local to the rank.

@@ -48,8 +48,10 @@ def _prep(t: Optional[torch.Tensor], device) -> Optional[torch.Tensor]:
 @_lib.on_tensor_device
 def _launch(bwd, p1, p2, g1, g2, c1, c2, t1, t2, need_dconf, alpha, ew, sw, dw, multi, grad_scale,
             rescale_invalid, out=None, thermal_stats=None, thermal_replicated=False, conf_min_only=False,
-            thermal_stats_scales=1):
-    """Raw call into the C ABI on already-prepared [B,H,W,3] CUDA tensors."""
+            thermal_stats_scales=1, main_done_event=None):
+    """Raw call into the C ABI on already-prepared [B,H,W,3] CUDA tensors.  The pseudo-GT (and its confidence) may
+    come at another resolution: bilinear taps inside the loss kernel's loads (train_thermal_dustr.py:234-271); a
+    confidence at the GT's size never takes a gradient."""
     lib = _lib.lib()
     B, H, W, _ = p1.shape
     dev = p1.device
@@ -84,68 +86,31 @@ def _launch(bwd, p1, p2, g1, g2, c1, c2, t1, t2, need_dconf, alpha, ew, sw, dw, 
             st1 = st2 = None
     if multi and st1 is not None:
         flags |= LOSS_STATS_TWO_SCALES     # the statistics carry the half-resolution sums (thermal_stats_scales == 2)
-    resampled = tuple(g1.shape[1:3]) != (H, W) or (c1 is not None and tuple(c1.shape[1:3]) != (H, W))
+    gh, gw = int(g1.shape[1]), int(g1.shape[2])
+    ch, cw = (int(c1.shape[1]), int(c1.shape[2])) if c1 is not None else (H, W)
     dp1 = dp2 = dc1 = dc2 = None
-    if resampled:
-        # pseudo-GT (and its confidence) at another resolution: bilinear taps inside the loss kernel's loads
-        # (train_thermal_dustr.py:234-271); a confidence at the GT's size never takes a gradient.  The thermal
-        # statistics of the preprocessing are honoured as on the same-size path.
-        gh, gw = int(g1.shape[1]), int(g1.shape[2])
-        ch, cw = (int(c1.shape[1]), int(c1.shape[2])) if c1 is not None else (H, W)
-        if bwd:
-            dp1 = out.get("dpred1"); dp2 = out.get("dpred2")
-            dp1 = torch.empty_like(p1) if dp1 is None else dp1
-            dp2 = torch.empty_like(p2) if dp2 is None else dp2
-            if need_dconf[0] and (ch, cw) == (H, W):
-                dc1 = out.get("dconf1")
-                dc1 = torch.empty(B, H, W, dtype=torch.float32, device=dev) if dc1 is None else dc1
-            if need_dconf[1] and (ch, cw) == (H, W):
-                dc2 = out.get("dconf2")
-                dc2 = torch.empty(B, H, W, dtype=torch.float32, device=dev) if dc2 is None else dc2
-        rc = lib.t3d_loss_fwd_bwd_resampled_stats(
-            _lib.ptr(p1), _lib.ptr(p2), _lib.ptr(g1), _lib.ptr(g2), gh, gw, _lib.ptr(c1), _lib.ptr(c2), ch, cw,
-            _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(st1), _lib.ptr(st2), st_tiles,
-            _lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
-            B, H, W, flags, alpha, ew, sw, dw, grad_scale,
-            _lib.ptr(per_sample), _lib.ptr(batch), _lib.ptr(f64), _lib.ptr(ws), ws.numel(), stream)
-        _lib.check(rc, "t3d_loss_fwd_bwd_resampled_stats")
-        if bwd and rescale_invalid:
-            rc = lib.t3d_loss_rescale_invalid(_lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
-                                              _lib.ptr(per_sample), _lib.ptr(batch), B, H, W, stream)
-            _lib.check(rc, "t3d_loss_rescale_invalid")
-        return per_sample, batch, dp1, dp2, dc1, dc2
     if bwd:
         dp1 = out.get("dpred1"); dp2 = out.get("dpred2")
-        if dp1 is None:
-            dp1 = torch.empty_like(p1)
-        if dp2 is None:
-            dp2 = torch.empty_like(p2)
-        if need_dconf[0]:
+        dp1 = torch.empty_like(p1) if dp1 is None else dp1
+        dp2 = torch.empty_like(p2) if dp2 is None else dp2
+        if need_dconf[0] and (ch, cw) == (H, W):
             dc1 = out.get("dconf1")
-            if dc1 is None:
-                dc1 = torch.empty(B, H, W, dtype=torch.float32, device=dev)
-        if need_dconf[1]:
+            dc1 = torch.empty(B, H, W, dtype=torch.float32, device=dev) if dc1 is None else dc1
+        if need_dconf[1] and (ch, cw) == (H, W):
             dc2 = out.get("dconf2")
-            if dc2 is None:
-                dc2 = torch.empty(B, H, W, dtype=torch.float32, device=dev)
-        rc = lib.t3d_loss_fwd_bwd(
-            _lib.ptr(p1), _lib.ptr(p2), _lib.ptr(g1), _lib.ptr(g2), _lib.ptr(c1), _lib.ptr(c2),
-            _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(st1), _lib.ptr(st2), st_tiles,
-            _lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
-            B, H, W, flags, alpha, ew, sw, dw, grad_scale,
-            _lib.ptr(per_sample), _lib.ptr(batch), _lib.ptr(f64), _lib.ptr(ws), ws.numel(), stream)
-        _lib.check(rc, "t3d_loss_fwd_bwd")
-        if rescale_invalid:
-            rc = lib.t3d_loss_rescale_invalid(_lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
-                                              _lib.ptr(per_sample), _lib.ptr(batch), B, H, W, stream)
-            _lib.check(rc, "t3d_loss_rescale_invalid")
-    else:
-        rc = lib.t3d_loss_fwd(
-            _lib.ptr(p1), _lib.ptr(p2), _lib.ptr(g1), _lib.ptr(g2), _lib.ptr(c1), _lib.ptr(c2),
-            _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(st1), _lib.ptr(st2), st_tiles,
-            B, H, W, flags, alpha, ew, sw, dw,
-            _lib.ptr(per_sample), _lib.ptr(batch), _lib.ptr(f64), _lib.ptr(ws), ws.numel(), stream)
-        _lib.check(rc, "t3d_loss_fwd")
+            dc2 = torch.empty(B, H, W, dtype=torch.float32, device=dev) if dc2 is None else dc2
+    rc = lib.t3d_loss_fwd_bwd(
+        _lib.ptr(p1), _lib.ptr(p2), _lib.ptr(g1), _lib.ptr(g2), gh, gw, _lib.ptr(c1), _lib.ptr(c2), ch, cw,
+        _lib.ptr(t1), _lib.ptr(t2), tch, _lib.ptr(st1), _lib.ptr(st2), st_tiles,
+        _lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
+        B, H, W, flags, alpha, ew, sw, dw, grad_scale,
+        _lib.ptr(per_sample), _lib.ptr(batch), _lib.ptr(f64),
+        None if main_done_event is None else main_done_event.cuda_event, _lib.ptr(ws), ws.numel(), stream)
+    _lib.check(rc, "t3d_loss_fwd_bwd")
+    if bwd and rescale_invalid:
+        rc = lib.t3d_loss_rescale_invalid(_lib.ptr(dp1), _lib.ptr(dp2), _lib.ptr(dc1), _lib.ptr(dc2),
+                                          _lib.ptr(per_sample), _lib.ptr(batch), B, H, W, stream)
+        _lib.check(rc, "t3d_loss_rescale_invalid")
     return per_sample, batch, dp1, dp2, dc1, dc2
 
 
@@ -253,7 +218,8 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
                                thermal_img1=None, thermal_img2=None, *, alpha=0.2, edge_weight=0.5,
                                smoothness_weight=0.3, detail_weight=0.3, multi_scale=True,
                                conf_grad=True, out=None, thermal_stats=None, grad_scale=None,
-                               thermal_replicated=False, rescale_invalid=True, thermal_stats_scales=1):
+                               thermal_replicated=False, rescale_invalid=True, thermal_stats_scales=1,
+                               main_done_event=None):
     """Functional (no autograd) fused step on prepared contiguous fp32 CUDA tensors.
 
     Returns dict(per_sample, batch, dpred1, dpred2, dconf1, dconf2); gradients are those of the
@@ -267,7 +233,9 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
     image are bit-identical (ThermalBatch.replicated; what enhance_thermal_contrast always returns): the
     kernel then reads one plane instead of three, same results.  ``rescale_invalid=False`` leaves the
     validity fix-up of the gradients to the caller (pipeline.HotPathStep: t3d_step_epilogue does it together
-    with the result packing in one launch).
+    with the result packing in one launch).  ``main_done_event`` (a ``torch.cuda.Event`` recorded at least once:
+    torch creates the CUDA event on its first record) is recorded right behind the loss's main kernel, before its
+    small second-stage reduction (pipeline.HotPathStep gates the next step's preprocessing on it).
     """
     _lib.require_cuda(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidences1, confidences2, thermal_img1, thermal_img2)
     if thermal_replicated and DEBUG_CHECKS and not torch.cuda.is_current_stream_capturing():
@@ -278,7 +246,8 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
         True, pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidences1, confidences2, thermal_img1, thermal_img2,
         need_dconf, float(alpha), float(edge_weight), float(smoothness_weight), float(detail_weight),
         bool(multi_scale), (1.0 / B) if grad_scale is None else float(grad_scale), rescale_invalid=bool(rescale_invalid), out=out,
-        thermal_stats=thermal_stats, thermal_replicated=thermal_replicated, thermal_stats_scales=int(thermal_stats_scales))
+        thermal_stats=thermal_stats, thermal_replicated=thermal_replicated, thermal_stats_scales=int(thermal_stats_scales),
+        main_done_event=main_done_event)
     return {"per_sample": ps, "batch": bt, "dpred1": dp1, "dpred2": dp2, "dconf1": dc1, "dconf2": dc2}
 
 

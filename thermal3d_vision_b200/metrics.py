@@ -91,10 +91,10 @@ def compute_depth_metrics_batch(pred, gt_depth, mask=None, median_scaling=True, 
     if med is None:
         med = torch.empty(B, 2, dtype=torch.float32, device=dev)
     state = out.get("state")
-    rc = lib.t3d_depth_metrics_phase(_lib.ptr(pred), stride, offset, _lib.ptr(gt), gt.shape[1], gt.shape[2], _lib.ptr(m),
+    rc = lib.t3d_depth_metrics(_lib.ptr(pred), stride, offset, _lib.ptr(gt), gt.shape[1], gt.shape[2], _lib.ptr(m),
                                B, H, W, 1 if median_scaling else 0, _lib.ptr(res), _lib.ptr(res64), _lib.ptr(med),
                                _lib.ptr(ws), ws.numel(), _lib.ptr(state), int(phase), _lib.current_stream_ptr())
-    _lib.check(rc, "t3d_depth_metrics_phase")
+    _lib.check(rc, "t3d_depth_metrics")
     if phase == PHASE_SAMPLE:
         return None
     return {"metrics": res, "metrics_f64": res64, "medians": med}

@@ -248,7 +248,6 @@ class HotPathStep:
         stacked = (raw1.is_contiguous() and raw2.is_contiguous() and raw1.shape == raw2.shape and
                    raw1.untyped_storage().data_ptr() == raw2.untyped_storage().data_ptr() and
                    raw2.storage_offset() == raw1.storage_offset() + raw1.numel())      # halves of one tensor
-        lib.t3d_preprocess_set_shared(1)            # the metric chain runs beside the preprocessing
         if self.histogram and "histogram" not in pre:
             pre["histogram"] = torch.empty(2 * B, 65536, dtype=torch.int32, device=self.device)
 
@@ -273,7 +272,7 @@ class HotPathStep:
                 self.s_samp_p.wait_event(ready)
                 self.s_samp_p.wait_event(self.ev_pre[i])
                 _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=False,
-                                              half_res_stats=self.multi_scale, phase=_metrics.PHASE_SAMPLE)
+                                              half_res_stats=self.multi_scale, phase=_metrics.PHASE_SAMPLE, shared=True)
                 self.ev_sp[i].record(self.s_samp_p)
         phase = _metrics.PHASE_REST if ahead else _metrics.PHASE_ALL
         s_met = self.s_met_alt if (i & 1) else self.s_met
@@ -286,7 +285,7 @@ class HotPathStep:
             me = _metrics.compute_depth_metrics_batch(pred1, gt_depth, out=met if ahead else {k: v for k, v in met.items() if k != "state"},
                                                       phase=phase)
             self.ev_met[i].record(s_met)
-        with torch.cuda.stream(self.s_pre):
+        with torch.cuda.stream(self.s_pre):                 # shared=True: the metric chain runs beside the preprocessing
             self.s_pre.wait_event(ready)
             if gate is not None:
                 self.s_pre.wait_event(gate)
@@ -294,7 +293,7 @@ class HotPathStep:
                 self.s_pre.wait_event(self.ev_sp[i])
             if stacked:
                 tb = _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=self.histogram,
-                                                   half_res_stats=self.multi_scale, phase=phase)
+                                                   half_res_stats=self.multi_scale, phase=phase, shared=True)
                 gs = tb.grad_stats
                 stats_scales = tb.stats_scales
                 (t1, t2), stats = (tb.thermal[:B], tb.thermal[B:]), ((None, None) if gs is None else (gs[:B], gs[B:]))
@@ -304,9 +303,9 @@ class HotPathStep:
                                             torch.empty(lib.t3d_preprocess_workspace_bytes(B, self.H, self.W), dtype=torch.uint8,
                                                         device=self.device) for k, v in pre.items()} for h in range(2)]
                 a = _pre.preprocess_thermal_batch(raw1, size, path="train", out=self._pre_halves[i][0], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale)
+                                                  half_res_stats=self.multi_scale, shared=True)
                 b = _pre.preprocess_thermal_batch(raw2, size, path="train", out=self._pre_halves[i][1], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale)
+                                                  half_res_stats=self.multi_scale, shared=True)
                 (t1, t2), stats = (a.thermal, b.thermal), (a.grad_stats, b.grad_stats)
                 stats_scales = min(a.stats_scales, b.stats_scales)
             pgrads, n_pgrads = None, 0
@@ -335,13 +334,12 @@ class HotPathStep:
             self.s_loss.wait_event(ready)                   # pred / gt / conf
             self.s_loss.wait_event(self.ev_pre[i])
             # the normalisation kernel already summed the thermal gradients: the loss skips its statistics pass
-            if self.pipelined:
-                if not self._main_recorded[i]:
-                    self.ev_main[i].record(self.s_loss)          # creates the CUDA event behind the torch object
-                    self._main_recorded[i] = True
-                lib.t3d_loss_set_main_done_event(self.ev_main[i].cuda_event)
+            if self.pipelined and not self._main_recorded[i]:
+                self.ev_main[i].record(self.s_loss)              # creates the CUDA event behind the torch object
+                self._main_recorded[i] = True
             _loss.fused_thermal_loss_fwd_bwd(pred1, pred2, gt1, gt2, conf1, conf2, t1, t2, conf_grad=conf_grad,
                                              out=lo, thermal_stats=stats, thermal_stats_scales=stats_scales,
+                                             main_done_event=self.ev_main[i] if self.pipelined else None,
                                              thermal_replicated=True,   # preprocess_thermal_batch wrote 3 identical planes
                                              grad_scale=_dist.global_grad_scale(self.B) if self.distributed else None,
                                              rescale_invalid=False,     # done by the epilogue below
@@ -587,7 +585,6 @@ class EvalStep:
         self.ev_met_done = [torch.cuda.Event() for _ in range(2)]
         self._next = 0
         self._prefetched = []          # [(raw ptr, pointmap ptr or None, set)], oldest first
-        lib.t3d_preprocess_set_shared(1)            # the metric pipeline runs beside the preprocessing (run_batch)
 
     def algorithmic_bytes(self) -> int:
         """Per batch: u16 frame in + 3 fp32 planes out, AoS pointmap + GT depth in (SURVEY.md 8d)."""
@@ -612,7 +609,7 @@ class EvalStep:
                 self.s_samp_p.wait_event(self.ev_ready[j])
                 self.s_samp_p.wait_event(self.ev_pre_done[j])          # the last batch on this set is done with it
                 _pre.preprocess_thermal_batch(raw, (self.W, self.H), path="train", out=self.pre_sets[j], histogram=False,
-                                              phase=_metrics.PHASE_SAMPLE)
+                                              phase=_metrics.PHASE_SAMPLE, shared=True)
                 self.ev_sp[j].record(self.s_samp_p)
             if pointmap is not None:
                 with torch.cuda.stream(self.s_samp_m):
@@ -649,7 +646,9 @@ class EvalStep:
                 self.join.record(self.side)
                 self.ev_met_done[j].record(self.side)
             main.wait_event(self.ev_sp[j])                   # likewise for the preprocessing's sampling state
-            tb = _pre.preprocess_thermal_batch(raw, (self.W, self.H), path=self.path, out=pre, histogram=False, phase=pre_phase)
+            # shared=True: the metric pipeline runs beside the preprocessing (side stream)
+            tb = _pre.preprocess_thermal_batch(raw, (self.W, self.H), path=self.path, out=pre, histogram=False, phase=pre_phase,
+                                               shared=True)
             self.ev_pre_done[j].record(main)
             main.wait_event(self.join)
             self.acc.update(me["metrics_f64"])

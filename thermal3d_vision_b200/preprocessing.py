@@ -82,7 +82,8 @@ class ThermalBatch(NamedTuple):
 @_lib.on_tensor_device
 def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: str = "train",
                              out_channels: int = 3, out: Optional[dict] = None,
-                             histogram: bool = True, half_res_stats: bool = False, phase: int = 0) -> ThermalBatch:
+                             histogram: bool = True, half_res_stats: bool = False, phase: int = 0,
+                             shared: bool = False) -> ThermalBatch:
     """16-bit radiometric frames [B,Hs,Ws] -> normalised thermal [B,3,h,w].
 
     img_size is (W, H) in cv2 order like the reference's --img_size.  path='train':
@@ -94,7 +95,9 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
     half_res_stats=True (train path): grad_stats also carries the thermal-gradient sums of the 2x2 average-pooled image
     the multi-scale loss needs (utils/loss.py:133-174), where the shape allows (ThermalBatch.stats_scales == 2).
     phase (train path, histogram=False; pipeline.HotPathStep): 1 = launch only the window-sampling kernel for these frames
-    (outputs stay in out["workspace"]), 2 = everything after it, on the same `out`; 0 = the whole call."""
+    (outputs stay in out["workspace"]), 2 = everything after it, on the same `out`; 0 = the whole call.
+    shared=True (train path) is a scheduling hint: other kernels run concurrently on another stream (the metric chain
+    of pipeline.HotPathStep / EvalStep), so the resize kernel leaves them room on every SM.  Same results."""
     x = _to_cuda(raw_u16).contiguous()
     if x.dtype != torch.uint16:
         raise ValueError(f"raw frames must be uint16, got {x.dtype}")
@@ -131,15 +134,10 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
         scales = 1
         if half_res_stats and stats is not None and lib.t3d_preprocess_stats_scales(dh, dw) == 2:
             scales = 2
-        lib.t3d_preprocess_set_stats_scales(scales)          # thread-local: applies to this thread's next call
-        try:
-            rc = lib.t3d_preprocess_train_u16_phase(_lib.ptr(x), B, sh, sw, dh, dw, _lib.ptr(thermal), out_channels,
-                                                    _lib.ptr(hist), _lib.ptr(pct), _lib.ptr(stats), _lib.ptr(ws), ws.numel(),
-                                                    int(phase), stream)
-        finally:
-            if scales != 1:
-                lib.t3d_preprocess_set_stats_scales(1)
-        _lib.check(rc, "t3d_preprocess_train_u16_phase")
+        rc = lib.t3d_preprocess_train_u16(_lib.ptr(x), B, sh, sw, dh, dw, _lib.ptr(thermal), out_channels,
+                                          _lib.ptr(hist), _lib.ptr(pct), _lib.ptr(stats), scales, int(bool(shared)),
+                                          _lib.ptr(ws), ws.numel(), int(phase), stream)
+        _lib.check(rc, "t3d_preprocess_train_u16")
         return ThermalBatch(thermal, pct, hist, stats, scales)
     if path == "inference":
         resized = torch.empty(B, dh, dw, dtype=torch.float32, device=dev)

@@ -42,9 +42,9 @@ def loss_bytes(B, H, W, gt_hw):
 
 def parent_handle(path):
     h = C.CDLL(os.path.abspath(path))
-    name = "t3d_loss_fwd_bwd_resampled"
-    res, args = _lib._SIGNATURES[name]
-    getattr(h, name).restype, getattr(h, name).argtypes = res, args
+    f, p, i = h.t3d_loss_fwd_bwd_resampled, C.c_void_p, C.c_int      # the parent's C ABI (version 2)
+    f.restype, f.argtypes = i, ([p] * 4 + [i] * 2 + [p] * 2 + [i] * 2 + [p] * 2 + [i] + [p] * 4 + [i] * 4
+                                + [C.c_float] * 5 + [p] * 3 + [p, C.c_size_t, p])
     h.t3d_last_error.restype = C.c_char_p
     return h
 
