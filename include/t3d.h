@@ -133,7 +133,13 @@ size_t t3d_loss_workspace_bytes(int B, int H, int W, int flags);
  * kernel resamples the gt rows as it stages them (loss_march_rs_kernel), bit-identical to t3d_interp_bilinear_f32
  * followed by this call at the prediction's size.  Everything else (wider segments such as 224x224 <- 512x512,
  * where the tile kernel measured faster; upsampled gt, a gt-sized confidence, unaligned data) runs on the general
- * tile kernel. */
+ * tile kernel.  With no thermal images (both NULL: the basic term alone, e.g. with T3D_LOSS_CONF_MIN_ONLY the plain
+ * confidence-weighted loss), W % 4 == 0, 16-byte aligned arrays, the confidence absent or at the prediction's size and
+ * the gt at the prediction's size or downsampled with a strip's source segment of at most 144 pixels (gt_w = W, e.g.
+ * 512x384 <- 512x512), the main kernel is loss_basic_kernel, a persistent per-pixel stream whose gradients are
+ * bit-identical to the tile kernel's (with a downsampled gt: to t3d_interp_bilinear_f32 followed by the same-size
+ * call).  Wider segments (224x224 <- 512x512, measured faster on the tile kernel), an upsampled gt and a gt-sized
+ * confidence keep the tile kernel's fused bilinear taps. */
 int t3d_loss_fwd_bwd(const float* pred1, const float* pred2,
                      const float* gt1, const float* gt2, int gt_h, int gt_w,
                      const float* conf1, const float* conf2, int conf_h, int conf_w,

@@ -350,6 +350,29 @@ __device__ __forceinline__ float edge_weight_of(float tx, float ty, float inv_mx
     return expf(-kThermalFactor * cx) * expf(-kThermalFactor * cy);
 }
 
+// The confidence-weighted L1 term of one pixel (utils/loss.py:81-98) and its closed-form gradient: the tile kernel's
+// per-pixel expressions, which loss_basic_kernel evaluates so that both write the same gradient bits.  p, g: the
+// pixel's xyz; craw: its raw confidence; the term is added to `sum`.  Returns d/dpred xyz and d/dconf (BWD).
+struct BasicGrad { float gx, gy, gz, dc; };
+template <bool BWD>
+__device__ __forceinline__ BasicGrad basic_px(float px, float py, float pz, float gx, float gy, float gz, float craw,
+                                              float conf_max, float alpha, float kb, float kc, float& sum) {
+    BasicGrad r = {0.f, 0.f, 0.f, 0.f};
+    const float dx = px - gx, dy = py - gy, dz = pz - gz;
+    const float l = ((fabsf(dx) + fabsf(dy)) + fabsf(dz)) / 3.0f;                 // utils/loss.py:82
+    const float cc = (craw < kConfMin) ? kConfMin : ((craw > conf_max) ? conf_max : craw);   // :91, NaN passes
+    sum += cc * l - alpha * logf(cc);                                              // :95
+    if (BWD) {
+        const float kc3 = cc * kb;
+        r.gx = sgnf(dx) * kc3;
+        r.gy = sgnf(dy) * kc3;
+        r.gz = sgnf(dz) * kc3;
+        const bool inside = (craw >= kConfMin) && (craw <= conf_max);              // clamp grad mask (inclusive)
+        r.dc = inside ? (l - alpha / cc) * kc : 0.f;
+    }
+    return r;
+}
+
 template <bool MULTI, bool VEC, bool BWD>
 __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(const LossArgs a) {
     constexpr int HALO = MULTI ? 2 : 1;
@@ -454,6 +477,8 @@ __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(cons
             float dc[4];
 #pragma unroll
             for (int e = 0; e < 4; ++e) {
+                // (basic_px, written out: through the helper, ptxas allocates the registers of the two unaligned
+                // backward instances differently)
                 const float dx = p[3 * e] - g[3 * e], dy = p[3 * e + 1] - g[3 * e + 1], dz = p[3 * e + 2] - g[3 * e + 2];
                 const float l = ((fabsf(dx) + fabsf(dy)) + fabsf(dz)) / 3.0f;             // utils/loss.py:82
                 const float craw = c[e];
@@ -683,6 +708,129 @@ __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(cons
 #pragma unroll
         for (int w = 0; w < kThreads / 32; ++w) s += red[w][tid];
         a.partials[((size_t)img * tiles + tile) * kNTerms + tid] = s;
+    }
+}
+
+// ------------------------------------------------------------------ basic term only (no thermal images)
+// loss_basic_kernel: the confidence-weighted L1 term alone -- train_thermal_dustr.py:305-318 (the loss without
+// --use_thermal_aware_loss), the validation loss (:465-492), confidence_weighted_regression_loss.  No stencil: a pure
+// per-pixel stream with one sum per sample.  Persistent grid; a warp pulls work items (one image-view, one band of
+// rows, one 128-pixel strip) from a queue, the large bands of the whole batch first and the short tail bands behind
+// them as loss_march_kernel does.  Each lane owns 4 pixels of a row: three 128-bit loads each of pred and gt (AoS),
+// one of the confidence, 128-bit streaming stores of d/dpred and d/dconf; one row per lane in flight, the latency is
+// covered by 20 (backward) / 32 (forward) resident warps per SM.  One partial per item (fixed butterfly), so a sample's
+// sums depend neither on its position in the batch nor on the batch size.
+// RS: the gt is downsampled (gt_h >= H, gt_w >= W), read through the bilinear taps of t3d_bilinear.cuh -- the
+// arithmetic of interp_bilinear_kernel, so the result is bit-identical to resampling first.
+struct BasicArgs {
+    const float* pred[2]; const float* gt[2]; const float* conf[2];
+    float* dpred[2]; float* dconf[2];
+    float* partials;              // [B*2][nbands*nstrips][kNTerms]: basic, 0 ...
+    unsigned int* queue;          // work-item counter, zero on entry
+    int B, H, W;
+    int rows_l, nbands_l, rows_s, nbands_s, nstrips;
+    float alpha, kb, kc, conf_max;
+    int gt_h, gt_w;               // RS: size of the gt arrays
+};
+// 4-warp CTAs: the backward instance needs 87 registers (5 CTAs = 20 warps per SM without spilling), forward 64 (32);
+// with the gt taps (RS) 166 / 128: 3 / 4 CTAs
+constexpr int kBWarps = 4;
+template <bool BWD, bool RS> constexpr int basic_blocks_per_sm() { return RS ? (BWD ? 3 : 4) : (BWD ? 5 : 8); }
+
+template <bool BWD, bool RS>
+__global__ void __launch_bounds__(kBWarps * 32, basic_blocks_per_sm<BWD, RS>()) loss_basic_kernel(const BasicArgs a) {
+    const int lane = threadIdx.x & 31;
+    const int H = a.H, W = a.W;
+    const size_t plane = (size_t)H * W;
+    const int nbands = a.nbands_l + a.nbands_s;
+    const int n_large = a.B * 2 * a.nbands_l * a.nstrips;
+    const int ntasks = a.B * 2 * nbands * a.nstrips;
+    const float conf_max = a.conf_max, alpha = a.alpha, kb = a.kb, kc = a.kc;
+    const float gsy = RS ? bscale(a.gt_h, H) : 1.f, gsx = RS ? bscale(a.gt_w, W) : 1.f;
+
+    for (;;) {
+        int task = 0;
+        if (lane == 0) task = (int)atomicAdd(a.queue, 1u);
+        task = __shfl_sync(0xffffffffu, task, 0);
+        if (task >= ntasks) break;
+        const bool large = task < n_large;
+        const int t1 = large ? task : task - n_large;
+        const int nb = large ? a.nbands_l : a.nbands_s;
+        const int s = t1 % a.nstrips;
+        const int t2 = t1 / a.nstrips;
+        const int k = t2 % nb;
+        const int img = t2 / nb;
+        const int b = img >> 1, view = img & 1;
+        const int ra = large ? k * a.rows_l : a.nbands_l * a.rows_l + k * a.rows_s;
+        const int rb = large ? ra + a.rows_l : min(ra + a.rows_s, H);
+        const int pidx = (img * nbands + (large ? k : a.nbands_l + k)) * a.nstrips + s;
+        const int x0 = s * 128 + 4 * lane;
+
+        float sum = 0.f;
+        if (x0 < W) {                                  // W % 4 == 0: a lane's 4 pixels are all inside or all outside
+            const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
+            const float* __restrict__ gt = a.gt[view] + (size_t)b * (RS ? (size_t)a.gt_h * a.gt_w : plane) * 3;
+            BTap gtx[4];
+            if (RS) {
+#pragma unroll
+                for (int e = 0; e < 4; ++e) gtx[e] = btap(x0 + e, a.gt_w, gsx);
+            }
+            const float* __restrict__ conf = a.conf[view] ? a.conf[view] + (size_t)b * plane : nullptr;
+            float* __restrict__ dpred = BWD ? a.dpred[view] + (size_t)b * plane * 3 : nullptr;
+            float* __restrict__ dconf = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane : nullptr;
+            auto load = [&](int y, float p[12], float g[12], float c[4]) {
+                const size_t pix = (size_t)y * W + x0;
+                const float4 p0 = ldg_stream_f4(pred + pix * 3), p1 = ldg_stream_f4(pred + pix * 3 + 4),
+                             p2 = ldg_stream_f4(pred + pix * 3 + 8);
+                p[0] = p0.x; p[1] = p0.y; p[2] = p0.z; p[3] = p0.w; p[4] = p1.x; p[5] = p1.y;
+                p[6] = p1.z; p[7] = p1.w; p[8] = p2.x; p[9] = p2.y; p[10] = p2.z; p[11] = p2.w;
+                if (!RS) {
+                    const float4 g0 = ldg_stream_f4(gt + pix * 3), g1 = ldg_stream_f4(gt + pix * 3 + 4),
+                                 g2 = ldg_stream_f4(gt + pix * 3 + 8);
+                    g[0] = g0.x; g[1] = g0.y; g[2] = g0.z; g[3] = g0.w; g[4] = g1.x; g[5] = g1.y;
+                    g[6] = g1.z; g[7] = g1.w; g[8] = g2.x; g[9] = g2.y; g[10] = g2.z; g[11] = g2.w;
+                } else {                               // bilinear taps (every tap is read, zero weights included)
+                    const BTap gty = btap(y, a.gt_h, gsy);
+#pragma unroll
+                    for (int e = 0; e < 4; ++e)
+#pragma unroll
+                        for (int ch = 0; ch < 3; ++ch) g[3 * e + ch] = bsample(gt, a.gt_w, 3, ch, gty, gtx[e]);
+                }
+                if (!conf) { c[0] = c[1] = c[2] = c[3] = 1.f; }
+                else {
+                    const float4 cc = ldg_stream_f4(conf + pix);
+                    c[0] = cc.x; c[1] = cc.y; c[2] = cc.z; c[3] = cc.w;
+                }
+            };
+            auto eval = [&](int y, const float p[12], const float g[12], const float c[4]) {
+                float gq[12], dc[4];
+#pragma unroll
+                for (int e = 0; e < 4; ++e) {
+                    const BasicGrad bg = basic_px<BWD>(p[3 * e], p[3 * e + 1], p[3 * e + 2], g[3 * e], g[3 * e + 1],
+                                                       g[3 * e + 2], c[e], conf_max, alpha, kb, kc, sum);
+                    gq[3 * e] = bg.gx; gq[3 * e + 1] = bg.gy; gq[3 * e + 2] = bg.gz; dc[e] = bg.dc;
+                }
+                if (BWD) {
+                    const size_t pix = (size_t)y * W + x0;
+                    float* o = dpred + pix * 3;
+                    stg_stream_f4(o, make_float4(gq[0], gq[1], gq[2], gq[3]));
+                    stg_stream_f4(o + 4, make_float4(gq[4], gq[5], gq[6], gq[7]));
+                    stg_stream_f4(o + 8, make_float4(gq[8], gq[9], gq[10], gq[11]));
+                    if (dconf) stg_stream_f4(dconf + pix, make_float4(dc[0], dc[1], dc[2], dc[3]));
+                }
+            };
+            for (int y = ra; y < rb; ++y) {
+                float p[12], g[12], c[4];
+                load(y, p, g, c);
+                eval(y, p, g, c);
+            }
+        }
+        sum = warp_sum(sum);
+        if (lane == 0) {
+            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)pidx * kNTerms);
+            o[0] = make_float4(sum, 0.f, 0.f, 0.f);
+            o[1] = make_float4(0.f, 0.f, 0.f, 0.f);
+        }
     }
 }
 
@@ -999,6 +1147,32 @@ int launch_loss(const LossArgs& la, cudaStream_t st) {
     return T3D_OK;
 }
 
+// Work items of the persistent loss kernels: nbands_l bands of rows_l rows from the top, then the last ~1/tail_div of
+// the image in bands of rows_s rows (queued behind all the large ones: a shorter tail of the persistent grid).  An
+// image too short for a tail has its ragged last large band handled as one small band of rows_l rows.
+struct Bands { int rows_l, nbands_l, rows_s, nbands_s; };
+Bands plan_bands(int H, int rows_l, int rows_s, int tail_div) {
+    Bands bd;
+    const int small_rows = ((H / tail_div + rows_s - 1) / rows_s) * rows_s;
+    bd.rows_l = rows_l; bd.rows_s = rows_s;
+    bd.nbands_l = (small_rows > 0) ? max(0, H - small_rows) / rows_l : (H + rows_l - 1) / rows_l;
+    if (small_rows == 0) { bd.nbands_s = 0;
+        if (bd.nbands_l * rows_l > H) { bd.nbands_l -= 1; bd.rows_s = rows_l; bd.nbands_s = 1; } }
+    else bd.nbands_s = (H - bd.nbands_l * rows_l + rows_s - 1) / rows_s;
+    return bd;
+}
+
+// 32-row bands with an 8-row tail: at most (H + 7) / 8 bands per strip, what the workspace reserves for the partials
+constexpr int kBasicRows = 32, kBasicTailRows = 8, kBasicTailDiv = 8;
+
+template <bool BWD, bool RS>
+int launch_basic(const BasicArgs& ba, cudaStream_t st) {
+    const int items = ba.B * 2 * (ba.nbands_l + ba.nbands_s) * ba.nstrips;
+    const int grid = min(t3d_sm_count() * basic_blocks_per_sm<BWD, RS>(), (items + kBWarps - 1) / kBWarps);
+    T3D_LAUNCH("loss_basic_kernel", st, loss_basic_kernel<BWD, RS><<<grid, kBWarps * 32, 0, st>>>(ba));
+    return T3D_OK;
+}
+
 int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1, const float* gt2,
               const float* conf1, const float* conf2, const float* thermal1, const float* thermal2,
               int tch, const float* ustats1, const float* ustats2, int ustats_tiles, float* dpred1, float* dpred2, float* dconf1, float* dconf2,
@@ -1079,7 +1253,31 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
     const bool march_rs = vec && thermal_on && !conf_min_only && !ms && gt_h != 0 && conf_h == 0 &&
                           gt_h >= H && gt_w >= W && gt_w % 4 == 0 && t3d_aligned16(gt1) && t3d_aligned16(gt2) &&
                           t3d_loss_march_rs_fits(rs_span = t3d_loss_march_rs_span(W, gt_w));
-    if (vec && thermal_on && !conf_min_only && (!resampled || march_rs) && (!ms || (H >= 4 && W >= 4))) {
+    // no thermal images: the basic term alone, a per-pixel stream (loss_basic_kernel) -- with the GT at the prediction's
+    // size, or downsampled with a strip's source segment of at most 144 px (gt_w ~ W: bilinear taps in its loads), and
+    // the confidence absent or at the prediction's size.  Measured on a B200 at 1000 W (tools/plain_loss_time.py):
+    // 384x512 <- 512x512, batch 64: 321.5 us against 341.1 us on the tile kernel; 224x224 <- 512x512, batch 8: 88.1 us
+    // against 41.0 us, so wider segments keep the tile kernel's fused taps, as do an upsampled GT and a GT-sized
+    // confidence
+    const bool basic_rs = gt_h != 0 && gt_h >= H && gt_w >= W && t3d_loss_march_rs_fits(t3d_loss_march_rs_span(W, gt_w));
+    const bool basic = vec && !thermal_on && conf_h == 0 && (gt_h == 0 || basic_rs);
+    if (basic) {
+        BasicArgs ba;
+        for (int v = 0; v < 2; ++v) {
+            ba.pred[v] = la.pred[v]; ba.gt[v] = la.gt[v]; ba.conf[v] = la.conf[v];
+            ba.dpred[v] = la.dpred[v]; ba.dconf[v] = la.dconf[v];
+        }
+        ba.partials = loss_partials; ba.queue = counter + 1;
+        ba.B = B; ba.H = H; ba.W = W;
+        const Bands bd = plan_bands(H, kBasicRows, kBasicTailRows, kBasicTailDiv);
+        ba.rows_l = bd.rows_l; ba.nbands_l = bd.nbands_l; ba.rows_s = bd.rows_s; ba.nbands_s = bd.nbands_s;
+        ba.nstrips = (W + 127) / 128;
+        ba.alpha = alpha; ba.kb = la.kb; ba.kc = la.kc; ba.conf_max = la.conf_max;
+        ba.gt_h = gt_h; ba.gt_w = gt_w;
+        n_partials = (ba.nbands_l + ba.nbands_s) * ba.nstrips;
+        if (basic_rs) rc = bwd ? launch_basic<true, true>(ba, st) : launch_basic<false, true>(ba, st);
+        else rc = bwd ? launch_basic<true, false>(ba, st) : launch_basic<false, false>(ba, st);
+    } else if (vec && thermal_on && !conf_min_only && (!resampled || march_rs) && (!ms || (H >= 4 && W >= 4))) {
         // fast path: TMA-fed warp-marching kernel (t3d_loss_march.cu); multi-scale: the half-resolution terms run
         // first as their own pass (t3d_loss_scale2.cu) and hand their gradient to the marching kernel
         MarchArgs ma;
@@ -1111,13 +1309,8 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         // heights and tails: DESIGN §4 experiment 12 and §5
         constexpr int kMarchRows = 32, kMarchTailDiv = 8;
         // (one-pass multi-scale: a band brings 4 halo rows instead of 2 and must start on an even row: 16-row tail bands)
-        const int rows_l = kMarchRows, rows_s = fused_ms ? 16 : 8;
-        const int small_rows = ((H / kMarchTailDiv + rows_s - 1) / rows_s) * rows_s;
-        ma.rows_l = rows_l; ma.rows_s = rows_s;
-        ma.nbands_l = (small_rows > 0) ? max(0, H - small_rows) / rows_l : (H + rows_l - 1) / rows_l;
-        if (small_rows == 0) { ma.nbands_s = 0; /* the last large band may be ragged: handle it as one small band */
-            if (ma.nbands_l * rows_l > H) { ma.nbands_l -= 1; ma.rows_s = rows_l; ma.nbands_s = 1; } }
-        else ma.nbands_s = (H - ma.nbands_l * rows_l + rows_s - 1) / rows_s;
+        const Bands bd = plan_bands(H, kMarchRows, fused_ms ? 16 : 8, kMarchTailDiv);
+        ma.rows_l = bd.rows_l; ma.nbands_l = bd.nbands_l; ma.rows_s = bd.rows_s; ma.nbands_s = bd.nbands_s;
         ma.nstrips = (W + 127) / 128;
         ma.alpha = alpha; ma.kb = la.kb; ma.kc = la.kc; ma.kE = la.kE[0]; ma.kS = la.kS[0]; ma.kD = la.kD[0];
         ma.kE2 = la.kE[1]; ma.kS2 = la.kS[1]; ma.kD2 = la.kD[1];

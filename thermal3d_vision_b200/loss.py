@@ -219,7 +219,7 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
                                smoothness_weight=0.3, detail_weight=0.3, multi_scale=True,
                                conf_grad=True, out=None, thermal_stats=None, grad_scale=None,
                                thermal_replicated=False, rescale_invalid=True, thermal_stats_scales=1,
-                               main_done_event=None):
+                               main_done_event=None, conf_min_only=False):
     """Functional (no autograd) fused step on prepared contiguous fp32 CUDA tensors.
 
     Returns dict(per_sample, batch, dpred1, dpred2, dconf1, dconf2); gradients are those of the
@@ -236,6 +236,8 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
     with the result packing in one launch).  ``main_done_event`` (a ``torch.cuda.Event`` recorded at least once:
     torch creates the CUDA event on its first record) is recorded right behind the loss's main kernel, before its
     small second-stage reduction (pipeline.HotPathStep gates the next step's preprocessing on it).
+    ``conf_min_only``: clamp the confidence from below only, as `fused_thermal_loss` (with no thermal images: the
+    training loss without --use_thermal_aware_loss, train_thermal_dustr.py:305-318).
     """
     _lib.require_cuda(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidences1, confidences2, thermal_img1, thermal_img2)
     if thermal_replicated and DEBUG_CHECKS and not torch.cuda.is_current_stream_capturing():
@@ -247,7 +249,7 @@ def fused_thermal_loss_fwd_bwd(pred_pts1, pred_pts2, gt_pts1, gt_pts2, confidenc
         need_dconf, float(alpha), float(edge_weight), float(smoothness_weight), float(detail_weight),
         bool(multi_scale), (1.0 / B) if grad_scale is None else float(grad_scale), rescale_invalid=bool(rescale_invalid), out=out,
         thermal_stats=thermal_stats, thermal_replicated=thermal_replicated, thermal_stats_scales=int(thermal_stats_scales),
-        main_done_event=main_done_event)
+        main_done_event=main_done_event, conf_min_only=bool(conf_min_only))
     return {"per_sample": ps, "batch": bt, "dpred1": dp1, "dpred2": dp2, "dconf1": dc1, "dconf2": dc2}
 
 

@@ -40,11 +40,22 @@ class HotPathStep:
     Every step still does all of its work on its own inputs; results are bit-identical to the plain step's.  With ``pipelined=False`` (default) the caller's stream
     waits for the step before `run_device` returns: plain stream semantics.  `loss_out`, `pre_both`, `met_out` and
     `result` always name the set of the latest call.
+
+    Loss.  ``use_thermal_aware_loss=True`` (default) trains on the thermal-aware loss of utils/loss.py:100-305.
+    ``False`` is train_thermal_dustr.py's other branch (:278-279,305-318, the run without --use_thermal_aware_loss):
+    the plain confidence-weighted L1 with the confidence clamped from below only.  The thermal batches are still
+    produced (they are the model's input) but the loss does not read them, and the preprocessing computes no
+    thermal-gradient statistics; edge_weight / smoothness_weight / detail_weight do not apply and the packed vector's
+    slots 2-4 are 0.  It has no multi-scale form.
     """
 
     def __init__(self, B: int, H: int, W: int, raw_hw=(512, 640), device=None, multi_scale: bool = False,
                  alpha=0.2, edge_weight=0.5, smoothness_weight=0.3, detail_weight=0.4, distributed: bool = False,
-                 exchange: str = "peer", pipelined: bool = False, sobel: bool = False, gt_hw=None):
+                 exchange: str = "peer", pipelined: bool = False, sobel: bool = False, gt_hw=None,
+                 use_thermal_aware_loss: bool = True):
+        if not use_thermal_aware_loss and multi_scale:
+            raise ValueError("multi_scale is a form of the thermal-aware loss: use_thermal_aware_loss=False has none")
+        self.use_thermal_aware_loss = bool(use_thermal_aware_loss)
         self.B, self.H, self.W, self.raw_hw = B, H, W, tuple(raw_hw)
         # pseudo-GT at its stored resolution (e.g. 512x512, scripts/pseudo_gt.py:620): the loss resamples it bilinearly
         # to (H, W) as train_thermal_dustr.py:234-271 does; None: the GT comes at (H, W)
@@ -56,6 +67,10 @@ class HotPathStep:
         self.multi_scale = bool(multi_scale)
         self.kw = dict(alpha=alpha, edge_weight=edge_weight, smoothness_weight=smoothness_weight,
                        detail_weight=detail_weight, multi_scale=multi_scale)
+        if not self.use_thermal_aware_loss:
+            # train_thermal_dustr.py:305-318: no thermal terms, the confidence clamped from below only (:278-279)
+            self.kw = dict(alpha=alpha, edge_weight=0.0, smoothness_weight=0.0, detail_weight=0.0, multi_scale=False,
+                           conf_min_only=True)
         self.distributed = distributed
         self.pipelined = bool(pipelined)
         dev = self.device
@@ -82,9 +97,11 @@ class HotPathStep:
         self.pre_sets = [{
             "thermal": torch.empty(2 * B, 3, H, W, **f32),
             "percentiles": torch.empty(2 * B, 2, dtype=torch.float64, device=dev),
-            "grad_stats": torch.empty(2 * B, max(lib.t3d_preprocess_stats_tiles(H, W), 1), 4, **f32),
             "workspace": torch.empty(lib.t3d_preprocess_workspace_bytes(2 * B, H, W), dtype=torch.uint8, device=dev),
         } for _ in range(2)]
+        if self.use_thermal_aware_loss:      # the thermal-gradient sums the loss reads (the plain loss reads none)
+            for p in self.pre_sets:
+                p["grad_stats"] = torch.empty(2 * B, max(lib.t3d_preprocess_stats_tiles(H, W), 1), 4, **f32)
         self._pre_halves = [None, None]      # separate-view fallback: allocated on first use
         self.met_sets = [{
             "workspace": torch.empty(lib.t3d_depth_metrics_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev),
@@ -206,9 +223,11 @@ class HotPathStep:
         raw = self.raw_hw[0] * self.raw_hw[1]
         # read 2x12 gt; with gt_hw: the source rows the bilinear y-taps touch, each read once
         gt = 24 * n if self.gt_hw is None else 24 * rows_touched(self.gt_hw[0], self.H) * self.gt_hw[1]
+        # read 2x12 pred, the gt, 2x4 conf, 2x4 thermal (the 3 planes are replicas: one is read), write 32; the plain
+        # loss reads no thermal
+        per_px = 72 if self.use_thermal_aware_loss else 64
         return {
-            # read 2x12 pred, the gt, 2x4 conf, 2x4 thermal (the 3 planes are replicas: one is read), write 32
-            "loss": B * (72 * n + gt),
+            "loss": B * (per_px * n + gt),
             "preprocess": 2 * B * (2 * raw + 12 * n),          # u16 frame in, 3 fp32 planes out
             "metrics": B * (12 * n + 4 * n + 64),              # pointmap (AoS sectors) + GT in, 64 B out
         }
@@ -272,7 +291,8 @@ class HotPathStep:
                 self.s_samp_p.wait_event(ready)
                 self.s_samp_p.wait_event(self.ev_pre[i])
                 _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=False,
-                                              half_res_stats=self.multi_scale, phase=_metrics.PHASE_SAMPLE, shared=True)
+                                              half_res_stats=self.multi_scale, phase=_metrics.PHASE_SAMPLE, shared=True,
+                                              grad_stats=self.use_thermal_aware_loss)
                 self.ev_sp[i].record(self.s_samp_p)
         phase = _metrics.PHASE_REST if ahead else _metrics.PHASE_ALL
         s_met = self.s_met_alt if (i & 1) else self.s_met
@@ -293,7 +313,8 @@ class HotPathStep:
                 self.s_pre.wait_event(self.ev_sp[i])
             if stacked:
                 tb = _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=self.histogram,
-                                                   half_res_stats=self.multi_scale, phase=phase, shared=True)
+                                                   half_res_stats=self.multi_scale, phase=phase, shared=True,
+                                                   grad_stats=self.use_thermal_aware_loss)
                 gs = tb.grad_stats
                 stats_scales = tb.stats_scales
                 (t1, t2), stats = (tb.thermal[:B], tb.thermal[B:]), ((None, None) if gs is None else (gs[:B], gs[B:]))
@@ -303,9 +324,11 @@ class HotPathStep:
                                             torch.empty(lib.t3d_preprocess_workspace_bytes(B, self.H, self.W), dtype=torch.uint8,
                                                         device=self.device) for k, v in pre.items()} for h in range(2)]
                 a = _pre.preprocess_thermal_batch(raw1, size, path="train", out=self._pre_halves[i][0], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale, shared=True)
+                                                  half_res_stats=self.multi_scale, shared=True,
+                                                  grad_stats=self.use_thermal_aware_loss)
                 b = _pre.preprocess_thermal_batch(raw2, size, path="train", out=self._pre_halves[i][1], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale, shared=True)
+                                                  half_res_stats=self.multi_scale, shared=True,
+                                                  grad_stats=self.use_thermal_aware_loss)
                 (t1, t2), stats = (a.thermal, b.thermal), (a.grad_stats, b.grad_stats)
                 stats_scales = min(a.stats_scales, b.stats_scales)
             pgrads, n_pgrads = None, 0
@@ -337,7 +360,9 @@ class HotPathStep:
             if self.pipelined and not self._main_recorded[i]:
                 self.ev_main[i].record(self.s_loss)              # creates the CUDA event behind the torch object
                 self._main_recorded[i] = True
-            _loss.fused_thermal_loss_fwd_bwd(pred1, pred2, gt1, gt2, conf1, conf2, t1, t2, conf_grad=conf_grad,
+            # (the plain loss: the thermal batches are the model's input only)
+            lt1, lt2 = (t1, t2) if self.use_thermal_aware_loss else (None, None)
+            _loss.fused_thermal_loss_fwd_bwd(pred1, pred2, gt1, gt2, conf1, conf2, lt1, lt2, conf_grad=conf_grad,
                                              out=lo, thermal_stats=stats, thermal_stats_scales=stats_scales,
                                              main_done_event=self.ev_main[i] if self.pipelined else None,
                                              thermal_replicated=True,   # preprocess_thermal_batch wrote 3 identical planes

@@ -83,7 +83,7 @@ class ThermalBatch(NamedTuple):
 def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: str = "train",
                              out_channels: int = 3, out: Optional[dict] = None,
                              histogram: bool = True, half_res_stats: bool = False, phase: int = 0,
-                             shared: bool = False) -> ThermalBatch:
+                             shared: bool = False, grad_stats: bool = True) -> ThermalBatch:
     """16-bit radiometric frames [B,Hs,Ws] -> normalised thermal [B,3,h,w].
 
     img_size is (W, H) in cv2 order like the reference's --img_size.  path='train':
@@ -97,7 +97,9 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
     phase (train path, histogram=False; pipeline.HotPathStep): 1 = launch only the window-sampling kernel for these frames
     (outputs stay in out["workspace"]), 2 = everything after it, on the same `out`; 0 = the whole call.
     shared=True (train path) is a scheduling hint: other kernels run concurrently on another stream (the metric chain
-    of pipeline.HotPathStep / EvalStep), so the resize kernel leaves them room on every SM.  Same results."""
+    of pipeline.HotPathStep / EvalStep), so the resize kernel leaves them room on every SM.  Same results.
+    grad_stats=False (train path): no thermal-gradient sums (ThermalBatch.grad_stats is None), for a loss that does not
+    use the thermal images; the thermal planes are the same."""
     x = _to_cuda(raw_u16).contiguous()
     if x.dtype != torch.uint16:
         raise ValueError(f"raw frames must be uint16, got {x.dtype}")
@@ -125,7 +127,7 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
         ws = out.get("workspace")
         if ws is None or ws.numel() < ws_bytes:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        tiles = lib.t3d_preprocess_stats_tiles(dh, dw)
+        tiles = lib.t3d_preprocess_stats_tiles(dh, dw) if grad_stats else 0
         stats = None
         if tiles > 0:
             stats = out.get("grad_stats")
