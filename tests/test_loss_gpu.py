@@ -29,6 +29,26 @@ def _oracle_sample(p1, p2, g1, g2, c1, c2, t1, t2, multi, **kw):
     return loss.item(), comp, a[0].grad, a[1].grad, None if a[4] is None else a[4].grad, None if a[5] is None else a[5].grad
 
 
+def _launched(fn):
+    """(fn(), names of the library's loss kernels it launched, the second stage left out)."""
+    from thermal3d_vision_b200 import _lib
+    torch.cuda.synchronize()
+    _lib.profile_begin("loss_", 256)
+    out = fn()
+    torch.cuda.synchronize()
+    names = {n for n, _, _ in _lib.profile_timeline(256)} - {"loss_finalize_kernel"}
+    _lib.profile_end()
+    return out, names
+
+
+def _misaligned(t):
+    """A contiguous copy at element offset 1 of its storage: not 16-byte aligned."""
+    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
+    v = buf[1:].view(t.shape)
+    v.copy_(t)
+    return v
+
+
 def _check_grad(name, got, ref32, ref64):
     got = got.detach().cpu()
     torch.testing.assert_close(got, ref32, rtol=1e-4, atol=1e-6, msg=lambda m: f"{name} vs fp32 oracle: {m}")
@@ -264,10 +284,18 @@ def test_marching_kernel_edge_shapes(cuda_device, H, W):
     d = [x.to(cuda_device) for x in (P1, P2, G1, G2, C1, C2, T1, T2)]
     for k in (0, 1, 4, 5):
         d[k].requires_grad_()
-    res = t3d.fused_thermal_loss(*d, multi_scale=False, **KW)
+    res, names = _launched(lambda: t3d.fused_thermal_loss(*d, multi_scale=False, **KW))
+    assert names == {"loss_march_kernel"}, names
     res.loss.backward()
     np.testing.assert_allclose(res.per_sample[:, :5].cpu().numpy(), rows, rtol=1e-5)
     for got, ref in ((d[0].grad, Pa.grad), (d[1].grad, Pb.grad), (d[4].grad, Ca.grad), (d[5].grad, Cb.grad)):
+        torch.testing.assert_close(got.cpu(), ref, rtol=1e-4, atol=1e-6)
+    # a misaligned thermal image: the tile kernel, same loss
+    args = [x.detach() for x in d[:7]] + [_misaligned(d[7])]
+    out, names = _launched(lambda: t3d.fused_thermal_loss_fwd_bwd(*args, multi_scale=False, **KW))
+    assert names == {"loss_tile_kernel"}, names
+    np.testing.assert_allclose(out["per_sample"][:, :5].cpu().numpy(), rows, rtol=1e-5)
+    for got, ref in ((out["dpred1"], Pa.grad), (out["dpred2"], Pb.grad), (out["dconf1"], Ca.grad), (out["dconf2"], Cb.grad)):
         torch.testing.assert_close(got.cpu(), ref, rtol=1e-4, atol=1e-6)
 
 
@@ -353,13 +381,17 @@ def test_multi_scale_march_paths_edge_shapes(cuda_device, H, W, planes):
     d = [x.to(cuda_device) for x in (P1, P2, G1, G2, C1, C2, T1, T2)]
     for k in (0, 1, 4, 5):
         d[k].requires_grad_()
+    expect = {"loss_scale2_kernel", "loss_march_kernel"} if planes == "three" else {"loss_march_ms_kernel"}
     if planes == "replicated":          # the functional entry takes the caller's promise that the planes are replicas
-        out = t3d.fused_thermal_loss_fwd_bwd(*(x.detach() for x in d), multi_scale=True, thermal_replicated=True, **KW)
+        out, names = _launched(lambda: t3d.fused_thermal_loss_fwd_bwd(*(x.detach() for x in d), multi_scale=True,
+                                                                      thermal_replicated=True, **KW))
+        assert names == expect, names
         np.testing.assert_allclose(out["per_sample"][:, :5].cpu().numpy(), rows, rtol=1e-5)
         for got, ref in ((out["dpred1"], Pa.grad), (out["dpred2"], Pb.grad), (out["dconf1"], Ca.grad), (out["dconf2"], Cb.grad)):
             torch.testing.assert_close(got.cpu(), ref, rtol=1e-4, atol=1e-6)
         return
-    res = t3d.fused_thermal_loss(*d, multi_scale=True, **KW)
+    res, names = _launched(lambda: t3d.fused_thermal_loss(*d, multi_scale=True, **KW))
+    assert names == expect, names
     res.loss.backward()
     np.testing.assert_allclose(res.per_sample[:, :5].cpu().numpy(), rows, rtol=1e-5)
     for got, ref in ((d[0].grad, Pa.grad), (d[1].grad, Pb.grad), (d[4].grad, Ca.grad), (d[5].grad, Cb.grad)):

@@ -50,6 +50,19 @@ int t3d_sm_count();   // cached per process (current device at first call; every
 constexpr int kT3dMaxDevices = 64;
 int t3d_device_slot();
 
+// cudaFuncSetAttribute(Kernel, MaxDynamicSharedMemorySize, bytes) once per device.  The flag is keyed on the kernel
+// itself (not on its type: instantiations with the same signature each need their own); benign race: idempotent.
+template <auto Kernel>
+int t3d_set_max_dynamic_smem(int bytes) {
+    static bool done[kT3dMaxDevices] = {};
+    bool& set = done[t3d_device_slot()];
+    if (!set) {
+        T3D_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        set = true;
+    }
+    return T3D_OK;
+}
+
 // Optional per-kernel CUDA-event timing (t3d_profile_begin / t3d_profile_end in include/t3d.h).
 bool t3d_prof_before(const char* name, cudaStream_t st);
 void t3d_prof_after(cudaStream_t st);

@@ -17,12 +17,6 @@
 
 namespace {
 
-constexpr float kEps = 1e-5f;          // utils/loss.py:240
-constexpr float kThermalFactor = 8.0f; // utils/loss.py:252
-constexpr float kHuber = 0.1f;         // utils/loss.py:267
-constexpr float kConfMin = 1e-5f, kConfMax = 10.0f;  // utils/loss.py:91-92
-constexpr float kScale2Weight = 0.35f; // 0.7 / scale, utils/loss.py:288
-
 // ------------------------------------------------------------------ stats
 constexpr int kSTH = 16, kSTW = 256, kSThreads = 256;
 constexpr int kSPW = kSTW + 4;  // row stride of the gray plane (2 halo cols + pad)
@@ -282,19 +276,14 @@ constexpr int kTH = 16, kTW = 128, kThreads = 256;
 constexpr int kPW = kTW + 8;          // raw plane row stride: col j -> c = j - j0 + 4
 constexpr int kQPT = kTH * kTW / 4 / kThreads;  // quads per thread (2)
 constexpr int kP2H = kTH / 2 + 2, kP2W = kTW / 2 + 4;  // pooled planes: (I,J) -> R = I-I0+1, C = J-J0+1
-constexpr int kNTerms = 8;            // basic, E1, S1, D1, E2, S2, D2, (pad)
 
 struct LossArgs {
-    const float* pred[2]; const float* gt[2]; const float* conf[2]; const float* thermal[2];
-    float* dpred[2]; float* dconf[2];
+    LossOperands op;
+    const float* thermal[2];
     const float* stats[2];        // per view: [B][stiles][4]
     float* partials;              // [B*2][tiles][kNTerms]
     int B, H, W, tch, tiles_x, tiles_y, stiles;
-    float alpha;
-    float kb;                     // grad_scale / (3 H W)
-    float kc;                     // grad_scale / (H W)
     float kE[2], kS[2], kD[2];    // grad_scale * lambda_s * weight / n_s
-    float conf_max;               // upper clamp of the confidence: 10 (utils/loss.py:91), +inf with T3D_LOSS_CONF_MIN_ONLY
     // GT (and GT confidence) at another resolution: bilinear taps fused into the loads (train_thermal_dustr.py:234-271)
     int gt_h, gt_w;               // size of the gt arrays; 0 = the prediction's size (read directly)
     int conf_h, conf_w;           // size of the conf arrays; 0 = the prediction's size
@@ -401,15 +390,15 @@ __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(cons
     const size_t plane = (size_t)H * W;
     const bool thermal_on = a.tch != 0;
 
-    const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
+    const float* __restrict__ pred = a.op.pred[view] + (size_t)b * plane * 3;
     const bool gt_rs = a.gt_h != 0, conf_rs = a.conf_h != 0;        // block-uniform: bilinear taps instead of direct reads
-    const float* __restrict__ gt = a.gt[view] + (size_t)b * (gt_rs ? (size_t)a.gt_h * a.gt_w : plane) * 3;
-    const float* __restrict__ conf = a.conf[view] ? a.conf[view] + (size_t)b * (conf_rs ? (size_t)a.conf_h * a.conf_w : plane) : nullptr;
+    const float* __restrict__ gt = a.op.gt[view] + (size_t)b * (gt_rs ? (size_t)a.gt_h * a.gt_w : plane) * 3;
+    const float* __restrict__ conf = a.op.conf[view] ? a.op.conf[view] + (size_t)b * (conf_rs ? (size_t)a.conf_h * a.conf_w : plane) : nullptr;
     const float gsy = gt_rs ? (float)a.gt_h / (float)H : 1.f, gsx = gt_rs ? (float)a.gt_w / (float)W : 1.f;
     const float csy = conf_rs ? (float)a.conf_h / (float)H : 1.f, csx = conf_rs ? (float)a.conf_w / (float)W : 1.f;
     const float* __restrict__ th = thermal_on ? a.thermal[view] + (size_t)b * a.tch * plane : nullptr;
-    float* __restrict__ dpred = BWD ? a.dpred[view] + (size_t)b * plane * 3 : nullptr;
-    float* __restrict__ dconf = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane : nullptr;
+    float* __restrict__ dpred = BWD ? a.op.dpred[view] + (size_t)b * plane * 3 : nullptr;
+    float* __restrict__ dconf = (BWD && a.op.dconf[view]) ? a.op.dconf[view] + (size_t)b * plane : nullptr;
 
     // 1/(mean + eps) of the thermal gradients of this image (fixed-order sum of the stats partials)
     if (thermal_on && tid < 4) {
@@ -482,18 +471,18 @@ __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(cons
                 const float dx = p[3 * e] - g[3 * e], dy = p[3 * e + 1] - g[3 * e + 1], dz = p[3 * e + 2] - g[3 * e + 2];
                 const float l = ((fabsf(dx) + fabsf(dy)) + fabsf(dz)) / 3.0f;             // utils/loss.py:82
                 const float craw = c[e];
-                const float cc = (craw < kConfMin) ? kConfMin : ((craw > a.conf_max) ? a.conf_max : craw);   // :91, NaN passes
+                const float cc = (craw < kConfMin) ? kConfMin : ((craw > a.op.conf_max) ? a.op.conf_max : craw);   // :91, NaN passes
                 const bool ok = e < nvalid;
-                if (ok) sum_basic += cc * l - a.alpha * logf(cc);                          // :95
+                if (ok) sum_basic += cc * l - a.op.alpha * logf(cc);                          // :95
                 zq[e] = p[3 * e + 2];
                 gzq[e] = g[3 * e + 2];
                 if (BWD) {
-                    const float kc3 = cc * a.kb;
+                    const float kc3 = cc * a.op.kb;
                     gq[k][3 * e] = sgnf(dx) * kc3;
                     gq[k][3 * e + 1] = sgnf(dy) * kc3;
                     gq[k][3 * e + 2] = sgnf(dz) * kc3;
-                    const bool inside = (craw >= kConfMin) && (craw <= a.conf_max);       // clamp grad mask (inclusive)
-                    dc[e] = inside ? (l - a.alpha / cc) * a.kc : 0.f;
+                    const bool inside = (craw >= kConfMin) && (craw <= a.op.conf_max);       // clamp grad mask (inclusive)
+                    dc[e] = inside ? (l - a.op.alpha / cc) * a.op.kc : 0.f;
                 }
             }
             if (BWD && dconf) {
@@ -714,22 +703,18 @@ __global__ void __launch_bounds__(kThreads, MULTI ? 2 : 3) loss_tile_kernel(cons
 // ------------------------------------------------------------------ basic term only (no thermal images)
 // loss_basic_kernel: the confidence-weighted L1 term alone -- train_thermal_dustr.py:305-318 (the loss without
 // --use_thermal_aware_loss), the validation loss (:465-492), confidence_weighted_regression_loss.  No stencil: a pure
-// per-pixel stream with one sum per sample.  Persistent grid; a warp pulls work items (one image-view, one band of
-// rows, one 128-pixel strip) from a queue, the large bands of the whole batch first and the short tail bands behind
-// them as loss_march_kernel does.  Each lane owns 4 pixels of a row: three 128-bit loads each of pred and gt (AoS),
+// per-pixel stream with one sum per sample.  Persistent grid; a warp pulls work items from the BandQueue
+// (t3d_loss_internal.cuh) as loss_march_kernel does.  Each lane owns 4 pixels of a row: three 128-bit loads each of pred and gt (AoS),
 // one of the confidence, 128-bit streaming stores of d/dpred and d/dconf; one row per lane in flight, the latency is
 // covered by 20 (backward) / 32 (forward) resident warps per SM.  One partial per item (fixed butterfly), so a sample's
 // sums depend neither on its position in the batch nor on the batch size.
 // RS: the gt is downsampled (gt_h >= H, gt_w >= W), read through the bilinear taps of t3d_bilinear.cuh -- the
 // arithmetic of interp_bilinear_kernel, so the result is bit-identical to resampling first.
 struct BasicArgs {
-    const float* pred[2]; const float* gt[2]; const float* conf[2];
-    float* dpred[2]; float* dconf[2];
-    float* partials;              // [B*2][nbands*nstrips][kNTerms]: basic, 0 ...
-    unsigned int* queue;          // work-item counter, zero on entry
+    LossOperands op;
+    float* partials;              // [B*2][bq.per_image_view()][kNTerms]: basic, 0 ...
+    BandQueue bq;
     int B, H, W;
-    int rows_l, nbands_l, rows_s, nbands_s, nstrips;
-    float alpha, kb, kc, conf_max;
     int gt_h, gt_w;               // RS: size of the gt arrays
 };
 // 4-warp CTAs: the backward instance needs 87 registers (5 CTAs = 20 warps per SM without spilling), forward 64 (32);
@@ -742,42 +727,26 @@ __global__ void __launch_bounds__(kBWarps * 32, basic_blocks_per_sm<BWD, RS>()) 
     const int lane = threadIdx.x & 31;
     const int H = a.H, W = a.W;
     const size_t plane = (size_t)H * W;
-    const int nbands = a.nbands_l + a.nbands_s;
-    const int n_large = a.B * 2 * a.nbands_l * a.nstrips;
-    const int ntasks = a.B * 2 * nbands * a.nstrips;
-    const float conf_max = a.conf_max, alpha = a.alpha, kb = a.kb, kc = a.kc;
+    const float conf_max = a.op.conf_max, alpha = a.op.alpha, kb = a.op.kb, kc = a.op.kc;
     const float gsy = RS ? bscale(a.gt_h, H) : 1.f, gsx = RS ? bscale(a.gt_w, W) : 1.f;
 
-    for (;;) {
-        int task = 0;
-        if (lane == 0) task = (int)atomicAdd(a.queue, 1u);
-        task = __shfl_sync(0xffffffffu, task, 0);
-        if (task >= ntasks) break;
-        const bool large = task < n_large;
-        const int t1 = large ? task : task - n_large;
-        const int nb = large ? a.nbands_l : a.nbands_s;
-        const int s = t1 % a.nstrips;
-        const int t2 = t1 / a.nstrips;
-        const int k = t2 % nb;
-        const int img = t2 / nb;
-        const int b = img >> 1, view = img & 1;
-        const int ra = large ? k * a.rows_l : a.nbands_l * a.rows_l + k * a.rows_s;
-        const int rb = large ? ra + a.rows_l : min(ra + a.rows_s, H);
-        const int pidx = (img * nbands + (large ? k : a.nbands_l + k)) * a.nstrips + s;
-        const int x0 = s * 128 + 4 * lane;
+    BandItem it;
+    while (next_band_item(a.bq, a.B, H, lane, it)) {
+        const int b = it.b, view = it.view, ra = it.ra, rb = it.rb;
+        const int x0 = it.strip * 128 + 4 * lane;
 
         float sum = 0.f;
         if (x0 < W) {                                  // W % 4 == 0: a lane's 4 pixels are all inside or all outside
-            const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
-            const float* __restrict__ gt = a.gt[view] + (size_t)b * (RS ? (size_t)a.gt_h * a.gt_w : plane) * 3;
+            const float* __restrict__ pred = a.op.pred[view] + (size_t)b * plane * 3;
+            const float* __restrict__ gt = a.op.gt[view] + (size_t)b * (RS ? (size_t)a.gt_h * a.gt_w : plane) * 3;
             BTap gtx[4];
             if (RS) {
 #pragma unroll
                 for (int e = 0; e < 4; ++e) gtx[e] = btap(x0 + e, a.gt_w, gsx);
             }
-            const float* __restrict__ conf = a.conf[view] ? a.conf[view] + (size_t)b * plane : nullptr;
-            float* __restrict__ dpred = BWD ? a.dpred[view] + (size_t)b * plane * 3 : nullptr;
-            float* __restrict__ dconf = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane : nullptr;
+            const float* __restrict__ conf = a.op.conf[view] ? a.op.conf[view] + (size_t)b * plane : nullptr;
+            float* __restrict__ dpred = BWD ? a.op.dpred[view] + (size_t)b * plane * 3 : nullptr;
+            float* __restrict__ dconf = (BWD && a.op.dconf[view]) ? a.op.dconf[view] + (size_t)b * plane : nullptr;
             auto load = [&](int y, float p[12], float g[12], float c[4]) {
                 const size_t pix = (size_t)y * W + x0;
                 const float4 p0 = ldg_stream_f4(pred + pix * 3), p1 = ldg_stream_f4(pred + pix * 3 + 4),
@@ -827,7 +796,7 @@ __global__ void __launch_bounds__(kBWarps * 32, basic_blocks_per_sm<BWD, RS>()) 
         }
         sum = warp_sum(sum);
         if (lane == 0) {
-            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)pidx * kNTerms);
+            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)it.pidx * kNTerms);
             o[0] = make_float4(sum, 0.f, 0.f, 0.f);
             o[1] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
@@ -1068,6 +1037,7 @@ struct WsLayout {
     size_t s2_partials, s2_dzp;        // multi-scale only (appended: the other offsets do not depend on `multi`)
     int stiles_x, stiles_y, tiles_x, tiles_y, s2_tiles_x, s2_tiles_y;
     int sm_bands, sm_strips;           // work items per image-view of the marching statistics kernel
+    int loss_partials_n;               // partial vectors per image-view the loss_partials hold
 };
 
 WsLayout ws_layout(int B, int H, int W, int multi) {
@@ -1079,8 +1049,9 @@ WsLayout ws_layout(int B, int H, int W, int multi) {
     L.sm_bands = (H + kStatsMarchRows - 1) / kStatsMarchRows; L.sm_strips = (W + 127) / 128;
     const size_t stats_tiles = (size_t)max(L.stiles_x * L.stiles_y, L.sm_bands * L.sm_strips);
     L.stats_partials = off; off += t3d_align_up((size_t)B * 2 * stats_tiles * 4 * sizeof(float), 256);
-    // sized for the tile kernel (16-row tiles) and the marching kernel (>= 8-row bands)
-    L.loss_partials = off;  off += t3d_align_up((size_t)B * 2 * L.tiles_x * ((H + 7) / 8) * kNTerms * sizeof(float), 256);
+    // sized for the tile kernel (16-row tiles) and the persistent kernels (>= 8-row bands; loss_impl checks the plan)
+    L.loss_partials_n = L.tiles_x * ((H + 7) / 8);
+    L.loss_partials = off;  off += t3d_align_up((size_t)B * 2 * L.loss_partials_n * kNTerms * sizeof(float), 256);
     t3d_scale2_tiles(H, W, &L.s2_tiles_x, &L.s2_tiles_y);
     L.s2_partials = L.s2_dzp = off;
     if (multi) {
@@ -1134,43 +1105,89 @@ int run_stats(const float* t1, const float* t2, int tch, int B, int H, int W, in
 
 template <bool MULTI, bool VEC, bool BWD>
 int launch_loss(const LossArgs& la, cudaStream_t st) {
-    static bool attr_done[kT3dMaxDevices] = {};   // per device; benign race: idempotent
-    bool& attr_set = attr_done[t3d_device_slot()];
     constexpr size_t smem = loss_smem_bytes<MULTI>();
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(loss_tile_kernel<MULTI, VEC, BWD>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<loss_tile_kernel<MULTI, VEC, BWD>>((int)smem)) return rc;
     const int grid = la.B * 2 * la.tiles_x * la.tiles_y;
     T3D_LAUNCH("loss_tile_kernel", st, loss_tile_kernel<MULTI, VEC, BWD><<<grid, kThreads, smem, st>>>(la));
     return T3D_OK;
 }
 
-// Work items of the persistent loss kernels: nbands_l bands of rows_l rows from the top, then the last ~1/tail_div of
-// the image in bands of rows_s rows (queued behind all the large ones: a shorter tail of the persistent grid).  An
-// image too short for a tail has its ragged last large band handled as one small band of rows_l rows.
-struct Bands { int rows_l, nbands_l, rows_s, nbands_s; };
-Bands plan_bands(int H, int rows_l, int rows_s, int tail_div) {
-    Bands bd;
+// The persistent kernels' work items (BandQueue): nbands_l bands of rows_l rows from the top, then the last
+// ~1/tail_div of the image in bands of rows_s rows (queued behind all the large ones: a shorter tail of the persistent
+// grid).  An image too short for a tail has its ragged last large band handled as one small band of rows_l rows.
+BandQueue plan_bands(int H, int W, int rows_l, int rows_s, int tail_div, unsigned int* queue) {
+    BandQueue bq;
+    bq.queue = queue;
     const int small_rows = ((H / tail_div + rows_s - 1) / rows_s) * rows_s;
-    bd.rows_l = rows_l; bd.rows_s = rows_s;
-    bd.nbands_l = (small_rows > 0) ? max(0, H - small_rows) / rows_l : (H + rows_l - 1) / rows_l;
-    if (small_rows == 0) { bd.nbands_s = 0;
-        if (bd.nbands_l * rows_l > H) { bd.nbands_l -= 1; bd.rows_s = rows_l; bd.nbands_s = 1; } }
-    else bd.nbands_s = (H - bd.nbands_l * rows_l + rows_s - 1) / rows_s;
-    return bd;
+    bq.rows_l = rows_l; bq.rows_s = rows_s;
+    bq.nbands_l = (small_rows > 0) ? max(0, H - small_rows) / rows_l : (H + rows_l - 1) / rows_l;
+    if (small_rows == 0) { bq.nbands_s = 0;
+        if (bq.nbands_l * rows_l > H) { bq.nbands_l -= 1; bq.rows_s = rows_l; bq.nbands_s = 1; } }
+    else bq.nbands_s = (H - bq.nbands_l * rows_l + rows_s - 1) / rows_s;
+    bq.nstrips = (W + 127) / 128;
+    return bq;
 }
 
-// 32-row bands with an 8-row tail: at most (H + 7) / 8 bands per strip, what the workspace reserves for the partials
+// loss_basic_kernel: 32-row bands, the last ~1/8 of the image in 8-row bands
 constexpr int kBasicRows = 32, kBasicTailRows = 8, kBasicTailDiv = 8;
+// loss_march_kernel: bands of 32 rows (a band re-reads the row above and the row below it: taller = less overfetch),
+// the last ~1/8 of the image in 8-row bands; other band heights and tails: DESIGN §4 experiment 12 and §5.
+// loss_march_ms_kernel: a band brings 4 halo rows instead of 2 and must start on an even row: 16-row tail bands.
+constexpr int kMarchRows = 32, kMarchTailRows = 8, kMarchMsTailRows = 16, kMarchTailDiv = 8;
 
 template <bool BWD, bool RS>
 int launch_basic(const BasicArgs& ba, cudaStream_t st) {
-    const int items = ba.B * 2 * (ba.nbands_l + ba.nbands_s) * ba.nstrips;
+    const int items = ba.B * 2 * ba.bq.per_image_view();
     const int grid = min(t3d_sm_count() * basic_blocks_per_sm<BWD, RS>(), (items + kBWarps - 1) / kBWarps);
     T3D_LAUNCH("loss_basic_kernel", st, loss_basic_kernel<BWD, RS><<<grid, kBWarps * 32, 0, st>>>(ba));
     return T3D_OK;
+}
+
+// The kernels that compute the loss; choose_loss_path picks one per call.
+enum class LossPath {
+    kBasic,         // loss_basic_kernel: no thermal images
+    kBasicTaps,     // loss_basic_kernel<RS>: the same with a downsampled GT read through bilinear taps
+    kMarch,         // loss_march_kernel: thermal-aware, single scale
+    kMarchTaps,     // loss_march_rs_kernel: the same with a downsampled GT resampled as its rows are staged
+    kMarchMs,       // loss_march_ms_kernel: multi-scale, both scales in one pass
+    kScale2March,   // loss_scale2_kernel, then loss_march_kernel adding its gradient: multi-scale in two passes
+    kTile,          // loss_tile_kernel: every other call
+};
+struct LossPathChoice { LossPath path; int span; };   // span: a strip's widest GT source segment (the *Taps paths)
+
+// gt_h == 0 / conf_h == 0: the GT / confidence is at the prediction's size.  vec: W % 4 == 0 and every array the
+// kernels stream is 16-byte aligned (a GT read through taps excepted).  gt_vec: gt_w % 4 == 0 and a 16-byte aligned GT.
+// one_plane: a thermal row stages one plane (one channel, or three bit-identical replicas).  ms: multi-scale with
+// thermal images.
+LossPathChoice choose_loss_path(int H, int W, int gt_h, int gt_w, int conf_h, bool vec, bool gt_vec, bool thermal_on,
+                                bool one_plane, bool ms, bool conf_min_only) {
+    const LossPathChoice tile = {LossPath::kTile, 0};
+    // The persistent kernels stream 4 pixels per lane with 128-bit loads or bulk copies, and read the confidence at
+    // the prediction's size only: unaligned arrays, W % 4 != 0 and a GT-sized confidence take the tile kernel.
+    if (!vec || conf_h != 0) return tile;
+    // A downsampled GT is read through bilinear taps by the persistent kernels only while a strip's source segment is
+    // at most 144 px (gt_w ~ W, t3d_loss_march_rs_fits).  Measured on a B200 at 1000 W against the tile kernel's fused
+    // taps: 384x512 <- 512x512 at batch 64, 364 us against 696 us thermal-aware (loss_march_rs_kernel) and 321.5 us
+    // against 341.1 us without thermal images (loss_basic_kernel, tools/plain_loss_time.py); 224x224 <- 512x512 at
+    // batch 8, 92 us against 77 us and 88.1 us against 41.0 us.  Wider segments and an upsampled GT keep the tile
+    // kernel (DESIGN §4).
+    int span = 0;
+    if (gt_h != 0) {
+        if (gt_h < H || gt_w < W) return tile;
+        span = t3d_loss_march_rs_span(W, gt_w);
+        if (!t3d_loss_march_rs_fits(span)) return tile;
+    }
+    if (!thermal_on) return {gt_h != 0 ? LossPath::kBasicTaps : LossPath::kBasic, span};
+    // the marching kernels clamp the confidence to [kConfMin, kConfMax]: the lower clamp alone takes the tile kernel
+    if (conf_min_only) return tile;
+    // the marching kernel bulk-copies the GT source rows; the one-pass multi-scale kernel has no registers left for
+    // the taps (DESIGN §8)
+    if (gt_h != 0) return (gt_vec && !ms) ? LossPathChoice{LossPath::kMarchTaps, span} : tile;
+    if (!ms) return {LossPath::kMarch, 0};
+    if (H < 4 || W < 4) return tile;     // the marching multi-scale paths need at least 2 x 2 pooled cells
+    // One staged thermal plane: both scales in one pass over the rows.  Three distinct planes would leave no shared
+    // memory for that kernel's deeper ring: the half-resolution terms run first as their own pass (DESIGN §4).
+    return {one_plane ? LossPath::kMarchMs : LossPath::kScale2March, 0};
 }
 
 int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1, const float* gt2,
@@ -1179,12 +1196,12 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
               int B, int H, int W, int flags, float alpha, float ew, float sw, float dw, float gscale,
               float* out_sample, float* out_batch, double* out_f64, cudaEvent_t main_done,
               void* workspace, size_t ws_bytes, void* stream, int gt_h, int gt_w, int conf_h, int conf_w) {
+    // ---- validate and normalise
     if (int rc = check_dims(B, H, W)) return rc;
     T3D_REQUIRE((flags & ~(T3D_LOSS_MULTI_SCALE | T3D_LOSS_CONF_MIN_ONLY | T3D_LOSS_STATS_TWO_SCALES)) == 0, "unknown loss flags 0x%x", flags);
     if (gt_h == H && gt_w == W) gt_h = gt_w = 0;                    // same size: direct reads
     if (conf_h == H && conf_w == W) conf_h = conf_w = 0;
     T3D_REQUIRE((gt_h == 0) == (gt_w == 0) && gt_h >= 0 && (conf_h == 0) == (conf_w == 0) && conf_h >= 0, "bad gt / conf size");
-    const bool resampled = gt_h != 0 || conf_h != 0;
     const int multi = (flags & T3D_LOSS_MULTI_SCALE) ? 1 : 0;
     const bool conf_min_only = (flags & T3D_LOSS_CONF_MIN_ONLY) != 0;
     T3D_REQUIRE(pred1 && pred2 && gt1 && gt2, "pred/gt pointers must not be NULL");
@@ -1200,11 +1217,33 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         return T3D_ERR_WORKSPACE;
     }
     T3D_REQUIRE(t3d_aligned16(workspace), "workspace must be 16-byte aligned");
+    const bool ms = multi && thermal_on;
+    const bool vec = (W % 4 == 0) && t3d_aligned16(pred1) && t3d_aligned16(pred2) && (gt_h != 0 || (t3d_aligned16(gt1) &&
+                     t3d_aligned16(gt2))) && (conf_h != 0 || (t3d_aligned16(conf1) && t3d_aligned16(conf2))) &&
+                     t3d_aligned16(thermal1) && t3d_aligned16(thermal2) && t3d_aligned16(dpred1) &&
+                     t3d_aligned16(dpred2) && t3d_aligned16(dconf1) && t3d_aligned16(dconf2);
+    const bool gt_vec = gt_w % 4 == 0 && t3d_aligned16(gt1) && t3d_aligned16(gt2);
+
+    // ---- choose the kernel; the persistent ones get their work items
+    const LossPathChoice choice = choose_loss_path(H, W, gt_h, gt_w, conf_h, vec, gt_vec, thermal_on, tch == 1 || replicated,
+                                                   ms, conf_min_only);
+    const LossPath path = choice.path;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     char* ws = reinterpret_cast<char*>(workspace);
     float* stats_partials = reinterpret_cast<float*>(ws + L.stats_partials);
     float* loss_partials = reinterpret_cast<float*>(ws + L.loss_partials);
     unsigned int* counter = reinterpret_cast<unsigned int*>(ws + L.counter);
+    BandQueue bq = {};
+    int n_partials = L.tiles_x * L.tiles_y;                          // loss_tile_kernel: one per 16 x 128 tile
+    if (path == LossPath::kBasic || path == LossPath::kBasicTaps) {
+        bq = plan_bands(H, W, kBasicRows, kBasicTailRows, kBasicTailDiv, counter + 1);
+        n_partials = bq.per_image_view();
+    } else if (path != LossPath::kTile) {
+        bq = plan_bands(H, W, kMarchRows, path == LossPath::kMarchMs ? kMarchMsTailRows : kMarchTailRows, kMarchTailDiv, counter + 1);
+        n_partials = bq.per_image_view();
+    }
+    T3D_REQUIRE(n_partials <= L.loss_partials_n, "%d partial vectors per image-view do not fit the %d of the workspace",
+                n_partials, L.loss_partials_n);
 
     T3D_CUDA(cudaMemsetAsync(counter, 0, 2 * sizeof(unsigned int), st));   // [0] finalize ticket, [1] work queue
     // thermal-gradient statistics: supplied by the caller (fused into the preprocessing) or computed here
@@ -1217,117 +1256,87 @@ int loss_impl(bool bwd, const float* pred1, const float* pred2, const float* gt1
         stats_v[1] = stats_partials + (size_t)B * stiles * 4;
     }
 
-    LossArgs la;
-    la.pred[0] = pred1; la.pred[1] = pred2; la.gt[0] = gt1; la.gt[1] = gt2;
-    la.conf[0] = conf1; la.conf[1] = conf2;
-    la.thermal[0] = thermal_on ? thermal1 : nullptr; la.thermal[1] = thermal_on ? thermal2 : nullptr;
-    la.dpred[0] = dpred1; la.dpred[1] = dpred2; la.dconf[0] = dconf1; la.dconf[1] = dconf2;
-    la.stats[0] = stats_v[0]; la.stats[1] = stats_v[1]; la.partials = loss_partials;
-    la.B = B; la.H = H; la.W = W; la.tch = thermal_on ? tch : 0;
-    la.tiles_x = L.tiles_x; la.tiles_y = L.tiles_y; la.stiles = stiles;
-    la.alpha = alpha;
-    la.conf_max = conf_min_only ? __int_as_float_host(0x7f800000u) : kConfMax;
-    la.gt_h = gt_h; la.gt_w = gt_w; la.conf_h = conf_h; la.conf_w = conf_w;
+    LossOperands op;
+    op.pred[0] = pred1; op.pred[1] = pred2; op.gt[0] = gt1; op.gt[1] = gt2; op.conf[0] = conf1; op.conf[1] = conf2;
+    op.dpred[0] = dpred1; op.dpred[1] = dpred2; op.dconf[0] = dconf1; op.dconf[1] = dconf2;
+    op.alpha = alpha;
     const double N = (double)H * W, n2 = (double)(H / 2) * (W / 2);
-    la.kb = (float)((double)gscale / (3.0 * N));
-    la.kc = (float)((double)gscale / N);
-    la.kE[0] = (float)((double)gscale * ew / N); la.kS[0] = (float)((double)gscale * sw / N);
-    la.kD[0] = (float)((double)gscale * dw / N);
+    op.kb = (float)((double)gscale / (3.0 * N));
+    op.kc = (float)((double)gscale / N);
+    op.conf_max = conf_min_only ? __int_as_float_host(0x7f800000u) : kConfMax;
     const double l2 = (n2 > 0) ? (double)kScale2Weight / n2 : 0.0;
-    la.kE[1] = (float)((double)gscale * ew * l2); la.kS[1] = (float)((double)gscale * sw * l2);
-    la.kD[1] = (float)((double)gscale * dw * l2);
+    const float kE[2] = {(float)((double)gscale * ew / N), (float)((double)gscale * ew * l2)};
+    const float kS[2] = {(float)((double)gscale * sw / N), (float)((double)gscale * sw * l2)};
+    const float kD[2] = {(float)((double)gscale * dw / N), (float)((double)gscale * dw * l2)};
 
-    bool vec = (W % 4 == 0) && t3d_aligned16(pred1) && t3d_aligned16(pred2) && (gt_h != 0 || (t3d_aligned16(gt1) &&
-               t3d_aligned16(gt2))) && (conf_h != 0 || (t3d_aligned16(conf1) && t3d_aligned16(conf2))) &&
-               t3d_aligned16(thermal1) && t3d_aligned16(thermal2) && t3d_aligned16(dpred1) &&
-               t3d_aligned16(dpred2) && t3d_aligned16(dconf1) && t3d_aligned16(dconf2);
-    const bool ms = multi && thermal_on;
-    int n_partials = L.tiles_x * L.tiles_y;
-    int rc;
+    // ---- fill the chosen kernel's arguments and launch it
+    int rc = T3D_OK;
     const float* partials2 = nullptr;
     int tiles2 = 0;
-    // gt at another size, downsampled: the marching kernel resamples it as it stages the rows (loss_march_rs_kernel)
-    // when a strip's source segment is one it is faster at (gt_w ~ W); wider segments, upsampled gt, a gt-sized
-    // confidence, multi-scale: tile kernel
-    int rs_span = 0;
-    const bool march_rs = vec && thermal_on && !conf_min_only && !ms && gt_h != 0 && conf_h == 0 &&
-                          gt_h >= H && gt_w >= W && gt_w % 4 == 0 && t3d_aligned16(gt1) && t3d_aligned16(gt2) &&
-                          t3d_loss_march_rs_fits(rs_span = t3d_loss_march_rs_span(W, gt_w));
-    // no thermal images: the basic term alone, a per-pixel stream (loss_basic_kernel) -- with the GT at the prediction's
-    // size, or downsampled with a strip's source segment of at most 144 px (gt_w ~ W: bilinear taps in its loads), and
-    // the confidence absent or at the prediction's size.  Measured on a B200 at 1000 W (tools/plain_loss_time.py):
-    // 384x512 <- 512x512, batch 64: 321.5 us against 341.1 us on the tile kernel; 224x224 <- 512x512, batch 8: 88.1 us
-    // against 41.0 us, so wider segments keep the tile kernel's fused taps, as do an upsampled GT and a GT-sized
-    // confidence
-    const bool basic_rs = gt_h != 0 && gt_h >= H && gt_w >= W && t3d_loss_march_rs_fits(t3d_loss_march_rs_span(W, gt_w));
-    const bool basic = vec && !thermal_on && conf_h == 0 && (gt_h == 0 || basic_rs);
-    if (basic) {
+    switch (path) {
+    case LossPath::kBasic:
+    case LossPath::kBasicTaps: {
         BasicArgs ba;
-        for (int v = 0; v < 2; ++v) {
-            ba.pred[v] = la.pred[v]; ba.gt[v] = la.gt[v]; ba.conf[v] = la.conf[v];
-            ba.dpred[v] = la.dpred[v]; ba.dconf[v] = la.dconf[v];
-        }
-        ba.partials = loss_partials; ba.queue = counter + 1;
-        ba.B = B; ba.H = H; ba.W = W;
-        const Bands bd = plan_bands(H, kBasicRows, kBasicTailRows, kBasicTailDiv);
-        ba.rows_l = bd.rows_l; ba.nbands_l = bd.nbands_l; ba.rows_s = bd.rows_s; ba.nbands_s = bd.nbands_s;
-        ba.nstrips = (W + 127) / 128;
-        ba.alpha = alpha; ba.kb = la.kb; ba.kc = la.kc; ba.conf_max = la.conf_max;
-        ba.gt_h = gt_h; ba.gt_w = gt_w;
-        n_partials = (ba.nbands_l + ba.nbands_s) * ba.nstrips;
-        if (basic_rs) rc = bwd ? launch_basic<true, true>(ba, st) : launch_basic<false, true>(ba, st);
+        ba.op = op; ba.partials = loss_partials; ba.bq = bq;
+        ba.B = B; ba.H = H; ba.W = W; ba.gt_h = gt_h; ba.gt_w = gt_w;
+        if (path == LossPath::kBasicTaps) rc = bwd ? launch_basic<true, true>(ba, st) : launch_basic<false, true>(ba, st);
         else rc = bwd ? launch_basic<true, false>(ba, st) : launch_basic<false, false>(ba, st);
-    } else if (vec && thermal_on && !conf_min_only && (!resampled || march_rs) && (!ms || (H >= 4 && W >= 4))) {
-        // fast path: TMA-fed warp-marching kernel (t3d_loss_march.cu); multi-scale: the half-resolution terms run
-        // first as their own pass (t3d_loss_scale2.cu) and hand their gradient to the marching kernel
+        break;
+    }
+    case LossPath::kMarch:
+    case LossPath::kMarchTaps:
+    case LossPath::kMarchMs:
+    case LossPath::kScale2March: {
+        // TMA-fed warp-marching kernels (t3d_loss_march.cu)
         MarchArgs ma;
-        for (int v = 0; v < 2; ++v) {
-            ma.pred[v] = la.pred[v]; ma.gt[v] = la.gt[v]; ma.conf[v] = la.conf[v]; ma.thermal[v] = la.thermal[v];
-            ma.dpred[v] = la.dpred[v]; ma.dconf[v] = la.dconf[v]; ma.dzp[v] = nullptr;
-        }
-        // multi-scale with one staged thermal plane: both scales in one pass over the rows (loss_march_ms_kernel)
-        const bool fused_ms = ms && (tch == 1 || replicated);
-        if (ms && !fused_ms) {
+        ma.op = op;
+        for (int v = 0; v < 2; ++v) { ma.thermal[v] = v ? thermal2 : thermal1; ma.stats[v] = stats_v[v]; ma.dzp[v] = nullptr; }
+        ma.partials = loss_partials; ma.bq = bq;
+        ma.B = B; ma.H = H; ma.W = W; ma.tch = tch; ma.stiles = stiles; ma.replicated = replicated;
+        ma.kE = kE[0]; ma.kS = kS[0]; ma.kD = kD[0]; ma.kE2 = kE[1]; ma.kS2 = kS[1]; ma.kD2 = kD[1];
+        ma.gt_h = gt_h; ma.gt_w = gt_w;
+        if (path == LossPath::kScale2March) {   // the half-resolution pass hands its gradient to the marching kernel
             Scale2Args sa;
             float* dzp = reinterpret_cast<float*>(ws + L.s2_dzp);
             for (int v = 0; v < 2; ++v) {
-                sa.pred[v] = la.pred[v]; sa.gt[v] = la.gt[v]; sa.thermal[v] = la.thermal[v]; sa.stats[v] = stats_v[v];
+                sa.pred[v] = op.pred[v]; sa.gt[v] = op.gt[v]; sa.thermal[v] = ma.thermal[v]; sa.stats[v] = stats_v[v];
                 sa.dzp[v] = dzp + (size_t)v * B * (H >> 1) * (W >> 1);
                 if (bwd) ma.dzp[v] = sa.dzp[v];
             }
             sa.partials = reinterpret_cast<float*>(ws + L.s2_partials);
             sa.B = B; sa.H = H; sa.W = W; sa.tch = tch; sa.replicated = replicated; sa.stiles = stiles;
             sa.tiles_x = L.s2_tiles_x; sa.tiles_y = L.s2_tiles_y;
-            sa.kE = la.kE[1]; sa.kS = la.kS[1]; sa.kD = la.kD[1];
+            sa.kE = kE[1]; sa.kS = kS[1]; sa.kD = kD[1];
             if (int rc2 = t3d_launch_loss_scale2(sa, bwd, st)) return rc2;
             partials2 = sa.partials; tiles2 = sa.tiles_x * sa.tiles_y;
         }
-        ma.stats[0] = stats_v[0]; ma.stats[1] = stats_v[1]; ma.partials = loss_partials; ma.queue = counter + 1;
-        ma.B = B; ma.H = H; ma.W = W; ma.tch = tch; ma.stiles = la.stiles; ma.replicated = replicated;
-        // bands of 32 rows (a band re-reads the row above and the row below it: taller = less overfetch), the last ~1/8
-        // of the image in 8-row bands queued behind all the large ones (shorter tail of the persistent grid); other band
-        // heights and tails: DESIGN §4 experiment 12 and §5
-        constexpr int kMarchRows = 32, kMarchTailDiv = 8;
-        // (one-pass multi-scale: a band brings 4 halo rows instead of 2 and must start on an even row: 16-row tail bands)
-        const Bands bd = plan_bands(H, kMarchRows, fused_ms ? 16 : 8, kMarchTailDiv);
-        ma.rows_l = bd.rows_l; ma.nbands_l = bd.nbands_l; ma.rows_s = bd.rows_s; ma.nbands_s = bd.nbands_s;
-        ma.nstrips = (W + 127) / 128;
-        ma.alpha = alpha; ma.kb = la.kb; ma.kc = la.kc; ma.kE = la.kE[0]; ma.kS = la.kS[0]; ma.kD = la.kD[0];
-        ma.kE2 = la.kE[1]; ma.kS2 = la.kS[1]; ma.kD2 = la.kD[1];
-        ma.gt_h = gt_h; ma.gt_w = gt_w;
-        n_partials = (ma.nbands_l + ma.nbands_s) * ma.nstrips;
-        rc = march_rs ? t3d_launch_loss_march_rs(ma, rs_span, bwd, st)
-           : fused_ms ? t3d_launch_loss_march_ms(ma, bwd, st) : t3d_launch_loss_march(ma, bwd, st);
-    } else if (bwd) {
-        if (ms) rc = vec ? launch_loss<true, true, true>(la, st) : launch_loss<true, false, true>(la, st);
-        else    rc = vec ? launch_loss<false, true, true>(la, st) : launch_loss<false, false, true>(la, st);
-    } else {
-        if (ms) rc = vec ? launch_loss<true, true, false>(la, st) : launch_loss<true, false, false>(la, st);
-        else    rc = vec ? launch_loss<false, true, false>(la, st) : launch_loss<false, false, false>(la, st);
+        rc = path == LossPath::kMarchTaps ? t3d_launch_loss_march_rs(ma, choice.span, bwd, st)
+           : path == LossPath::kMarchMs ? t3d_launch_loss_march_ms(ma, bwd, st) : t3d_launch_loss_march(ma, bwd, st);
+        break;
+    }
+    case LossPath::kTile: {
+        LossArgs la;
+        la.op = op;
+        la.thermal[0] = thermal_on ? thermal1 : nullptr; la.thermal[1] = thermal_on ? thermal2 : nullptr;
+        la.stats[0] = stats_v[0]; la.stats[1] = stats_v[1]; la.partials = loss_partials;
+        la.B = B; la.H = H; la.W = W; la.tch = thermal_on ? tch : 0;
+        la.tiles_x = L.tiles_x; la.tiles_y = L.tiles_y; la.stiles = stiles;
+        for (int s = 0; s < 2; ++s) { la.kE[s] = kE[s]; la.kS[s] = kS[s]; la.kD[s] = kD[s]; }
+        la.gt_h = gt_h; la.gt_w = gt_w; la.conf_h = conf_h; la.conf_w = conf_w;
+        if (bwd) {
+            if (ms) rc = vec ? launch_loss<true, true, true>(la, st) : launch_loss<true, false, true>(la, st);
+            else    rc = vec ? launch_loss<false, true, true>(la, st) : launch_loss<false, false, true>(la, st);
+        } else {
+            if (ms) rc = vec ? launch_loss<true, true, false>(la, st) : launch_loss<true, false, false>(la, st);
+            else    rc = vec ? launch_loss<false, true, false>(la, st) : launch_loss<false, false, false>(la, st);
+        }
+        break;
+    }
     }
     if (rc) return rc;
     if (main_done) T3D_CUDA(cudaEventRecord(main_done, st));   // lets a caller overlap the second stage with other work
 
+    // ---- second stage
     FinalizeArgs fa;
     fa.partials = loss_partials; fa.out_sample = out_sample; fa.out_batch = out_batch; fa.out_f64 = out_f64;
     fa.partials2 = partials2; fa.tiles2 = tiles2;

@@ -23,10 +23,6 @@
 
 namespace {
 
-constexpr float kEps = 1e-5f;
-constexpr float kHuber = 0.1f;
-constexpr float kConfMin = 1e-5f, kConfMax = 10.0f;
-
 constexpr int kStripPx = 128;            // 32 lanes x 4 pixels
 constexpr int kSegPx = kStripPx + 8;     // + 4-pixel halo each side (keeps 16-byte alignment of AoS rows)
 
@@ -71,16 +67,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t by
 // ------------------------------------------------------------------ math
 struct Sums { float E, S, D; };
 
-// NaN-propagating min / max (SASS FMNMX.NAN): torch.clamp lets NaN through, fminf/fmaxf would not
-__device__ __forceinline__ float min_nan(float a, float b) { float d; asm("min.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b)); return d; }
-__device__ __forceinline__ float max_nan(float a, float b) { float d; asm("max.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b)); return d; }
-
-// sgn(x) * |t-signed value|: (x > 0) ? t : (x < 0 ? -t : 0) with one compare (sgn(0) = 0 like ATen)
-__device__ __forceinline__ float times_sgn(float t, float x) {
-    const float r = __uint_as_float(__float_as_uint(t) ^ (__float_as_uint(x) & 0x80000000u));
-    return (x != 0.f) ? r : 0.f;
-}
-
 // one forward-difference term (SURVEY.md Appendix A).  The zero-padded last column / row is expressed
 // by the caller handing in zb == za, gb == ga (all contributions vanish, sgn(0) = 0).
 __device__ __forceinline__ float q_term(float za, float zb, float ga, float gb, float w, float omw,
@@ -103,7 +89,7 @@ __device__ __forceinline__ float edge_w(float tx, float ty, float inv_mx, float 
     // exp(-8 clamp(tx/mean,0,m)) * exp(-8 clamp(ty/mean,0,m))  (utils/loss.py:240-256); tx, ty >= 0
     const float cx = min_nan(tx * inv_mx, m);
     const float cy = min_nan(ty * inv_my, m);
-    return __expf(-8.0f * (cx + cy));
+    return __expf(-kThermalFactor * (cx + cy));
 }
 
 // REP: the image's 3 planes are bit-identical replicas (what enhance_thermal_contrast always returns,
@@ -197,31 +183,15 @@ __device__ __forceinline__ void march_body(const MarchArgs& a) {
 
     const int H = a.H, W = a.W;
     const size_t plane = (size_t)H * W;
-    const int nbands = a.nbands_l + a.nbands_s;
-    const int n_large = a.B * 2 * a.nbands_l * a.nstrips;
-    const int ntasks = a.B * 2 * nbands * a.nstrips;
-    const float kE = a.kE, kS2 = 2.0f * a.kS, kD = a.kD, kb = a.kb, kc = a.kc, alpha = a.alpha;
+    const float kE = a.kE, kS2 = 2.0f * a.kS, kD = a.kD, kb = a.op.kb, kc = a.op.kc, alpha = a.op.alpha;
     const float alpha_ln2 = alpha * 0.69314718055994531f;
     uint32_t pos = 0;                                  // rows streamed so far by this warp (ring position)
     const int gh = SEG ? a.gt_h : H, gw = SEG ? a.gt_w : W;
     const float sy = SEG ? bscale(gh, H) : 1.f, sx = SEG ? bscale(gw, W) : 1.f;
 
-    for (;;) {
-        int task = 0;
-        if (lane == 0) task = (int)atomicAdd(a.queue, 1u);
-        task = __shfl_sync(0xffffffffu, task, 0);
-        if (task >= ntasks) break;
-        const bool large = task < n_large;
-        const int t1 = large ? task : task - n_large;
-        const int nb = large ? a.nbands_l : a.nbands_s;
-        const int s = t1 % a.nstrips;
-        const int t2 = t1 / a.nstrips;
-        const int k = t2 % nb;
-        const int img = t2 / nb;
-        const int b = img >> 1, view = img & 1;
-        const int ra = large ? k * a.rows_l : a.nbands_l * a.rows_l + k * a.rows_s;
-        const int rb = large ? ra + a.rows_l : min(ra + a.rows_s, H);          // the large bands end at nbands_l * rows_l <= H
-        const int pidx = (img * nbands + (large ? k : a.nbands_l + k)) * a.nstrips + s;     // partials: per image-view, band-major
+    BandItem it;
+    while (next_band_item(a.bq, a.B, H, lane, it)) {
+        const int b = it.b, view = it.view, s = it.strip, ra = it.ra, rb = it.rb;
         const int i_lo = max(ra - 1, 0), i_hi = min(rb, H - 1);
         const int n_rows = i_hi - i_lo + 1;
         const int col0 = s * kStripPx;
@@ -234,9 +204,9 @@ __device__ __forceinline__ void march_body(const MarchArgs& a) {
         const bool right_in_image = (j + 4 < W);
         const int idx = 4 * lane + off;                // smem pixel index of this lane's quad
 
-        const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
-        const float* __restrict__ gt = a.gt[view] + (size_t)b * (size_t)gh * gw * 3;
-        const float* __restrict__ conf = a.conf[view] ? a.conf[view] + (size_t)b * plane : nullptr;
+        const float* __restrict__ pred = a.op.pred[view] + (size_t)b * plane * 3;
+        const float* __restrict__ gt = a.op.gt[view] + (size_t)b * (size_t)gh * gw * 3;
+        const float* __restrict__ conf = a.op.conf[view] ? a.op.conf[view] + (size_t)b * plane : nullptr;
         const float* __restrict__ th = a.thermal[view] + (size_t)b * (REP ? 3 : TCH) * plane;
         // resampled gt: the strip's source segment [s0, s0 + seg_px) covers the x-taps of columns c0 .. c1-1
         RsCtx rs = {0, gw, sx};
@@ -246,8 +216,8 @@ __device__ __forceinline__ void march_body(const MarchArgs& a) {
             seg_bytes = (uint32_t)(((btap(c1 - 1, gw, sx).i1 + 4) & ~3) - rs.s0) * 12u;
         }
         // running output pointers of this lane's quad (row i_lo; advanced by one row per iteration)
-        float* dp_ptr = BWD ? a.dpred[view] + ((size_t)b * plane + (size_t)i_lo * W + j) * 3 : nullptr;
-        float* dc_ptr = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane + (size_t)i_lo * W + j : nullptr;
+        float* dp_ptr = BWD ? a.op.dpred[view] + ((size_t)b * plane + (size_t)i_lo * W + j) * 3 : nullptr;
+        float* dc_ptr = (BWD && a.op.dconf[view]) ? a.op.dconf[view] + (size_t)b * plane + (size_t)i_lo * W + j : nullptr;
         // multi-scale: this lane's two pooled cells per row pair (W % 4 == 0: columns j .. j+3 are always inside 2 * (W / 2))
         const int w2 = W >> 1, rows2 = 2 * (H >> 1);
         const float* dz2_ptr = (S2 && BWD) ? a.dzp[view] + (size_t)b * (H >> 1) * w2 + (j >> 1) : nullptr;
@@ -439,7 +409,7 @@ __device__ __forceinline__ void march_body(const MarchArgs& a) {
         tot.E = warp_sum(tot.E); tot.S = warp_sum(tot.S); tot.D = warp_sum(tot.D);
         if (lane == 0) {
             if (thermal_bad) tot.E = __int_as_float(0x7fc00000);
-            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)pidx * 8);
+            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)it.pidx * kNTerms);
             o[0] = make_float4(sum_b, tot.E, tot.S, tot.D);
             o[1] = make_float4(0.f, 0.f, 0.f, 0.f);
         }
@@ -513,30 +483,14 @@ __global__ void __maxnreg__((WARPS >= 12) ? 168 : 255) loss_march_ms_kernel(cons
 
     const int H = a.H, W = a.W, h2 = H >> 1, w2 = W >> 1;
     const size_t plane = (size_t)H * W;
-    const int nbands = a.nbands_l + a.nbands_s;
-    const int n_large = a.B * 2 * a.nbands_l * a.nstrips;
-    const int ntasks = a.B * 2 * nbands * a.nstrips;
-    const float kE = a.kE, kS2 = 2.0f * a.kS, kD = a.kD, kb = a.kb, kc = a.kc, alpha = a.alpha;
+    const float kE = a.kE, kS2 = 2.0f * a.kS, kD = a.kD, kb = a.op.kb, kc = a.op.kc, alpha = a.op.alpha;
     const float kE_2 = a.kE2, kS2_2 = 2.0f * a.kS2, kD_2 = a.kD2;
     const float alpha_ln2 = alpha * 0.69314718055994531f;
     uint32_t pos = 0;
 
-    for (;;) {
-        int task = 0;
-        if (lane == 0) task = (int)atomicAdd(a.queue, 1u);
-        task = __shfl_sync(0xffffffffu, task, 0);
-        if (task >= ntasks) break;
-        const bool large = task < n_large;
-        const int t1 = large ? task : task - n_large;
-        const int nb = large ? a.nbands_l : a.nbands_s;
-        const int s = t1 % a.nstrips;
-        const int t2 = t1 / a.nstrips;
-        const int k = t2 % nb;
-        const int img = t2 / nb;
-        const int b = img >> 1, view = img & 1;
-        const int ra = large ? k * a.rows_l : a.nbands_l * a.rows_l + k * a.rows_s;            // even (rows_l, rows_s are)
-        const int rb = large ? ra + a.rows_l : min(ra + a.rows_s, H);
-        const int pidx = (img * nbands + (large ? k : a.nbands_l + k)) * a.nstrips + s;
+    BandItem it;
+    while (next_band_item(a.bq, a.B, H, lane, it)) {
+        const int b = it.b, view = it.view, s = it.strip, ra = it.ra, rb = it.rb;   // ra even (rows_l, rows_s are)
         const int i_lo = max(ra - 2, 0), i_hi = min(rb + 1, H - 1);                            // i_lo even
         const int n_rows = i_hi - i_lo + 1;
         const int ri_first = (ra > 0) ? 1 : 0;             // ring index of the first row that is "current" for the full-resolution march
@@ -551,13 +505,13 @@ __global__ void __maxnreg__((WARPS >= 12) ? 168 : 255) loss_march_ms_kernel(cons
         const bool right_in_image = (j + 4 < W);
         const int idx = 4 * lane + off;
 
-        const float* __restrict__ pred = a.pred[view] + (size_t)b * plane * 3;
-        const float* __restrict__ gt = a.gt[view] + (size_t)b * plane * 3;
+        const float* __restrict__ pred = a.op.pred[view] + (size_t)b * plane * 3;
+        const float* __restrict__ gt = a.op.gt[view] + (size_t)b * plane * 3;
         const float* __restrict__ th = a.thermal[view] + (size_t)b * (REP ? 3 : 1) * plane;
         const int r_first = i_lo + ri_first;
-        const float* c_ptr = a.conf[view] ? a.conf[view] + (size_t)b * plane + (size_t)r_first * W + j : nullptr;
-        float* dp_ptr = BWD ? a.dpred[view] + ((size_t)b * plane + (size_t)r_first * W + j) * 3 : nullptr;
-        float* dc_ptr = (BWD && a.dconf[view]) ? a.dconf[view] + (size_t)b * plane + (size_t)r_first * W + j : nullptr;
+        const float* c_ptr = a.op.conf[view] ? a.op.conf[view] + (size_t)b * plane + (size_t)r_first * W + j : nullptr;
+        float* dp_ptr = BWD ? a.op.dpred[view] + ((size_t)b * plane + (size_t)r_first * W + j) * 3 : nullptr;
+        float* dc_ptr = (BWD && a.op.dconf[view]) ? a.op.dconf[view] + (size_t)b * plane + (size_t)r_first * W + j : nullptr;
 
         // 1 / (mean + eps) of the thermal gradients at both scales: fixed-order sums of the stats partials
         float inv_mx, inv_my, inv_mx2, inv_my2;
@@ -817,7 +771,7 @@ __global__ void __maxnreg__((WARPS >= 12) ? 168 : 255) loss_march_ms_kernel(cons
         if (lane == 0) {
             if (thermal_bad) tot.E = __int_as_float(0x7fc00000);
             if (thermal_bad2) tot2.E = __int_as_float(0x7fc00000);
-            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)pidx * 8);
+            float4* o = reinterpret_cast<float4*>(a.partials + (size_t)it.pidx * kNTerms);
             o[0] = make_float4(sum_b, tot.E, tot.S, tot.D);
             o[1] = make_float4(tot2.E, tot2.S, tot2.D, 0.f);
         }
@@ -831,13 +785,7 @@ int launch_ms(const MarchArgs& a, cudaStream_t st) {
     constexpr int NS = 5, WARPS = 12;
     constexpr size_t smem = (size_t)WARPS * NS * StageF::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
     static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
-    static bool attr_done[kT3dMaxDevices] = {};
-    bool& attr_set = attr_done[t3d_device_slot()];
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(loss_march_ms_kernel<REP, BWD, NS, WARPS>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<loss_march_ms_kernel<REP, BWD, NS, WARPS>>((int)smem)) return rc;
     T3D_LAUNCH("loss_march_ms_kernel", st,
                loss_march_ms_kernel<REP, BWD, NS, WARPS><<<t3d_sm_count(), WARPS * 32, smem, st>>>(a));
     return T3D_OK;
@@ -850,13 +798,7 @@ int launch(const MarchArgs& a, cudaStream_t st) {
     constexpr int NS = 4, WARPS = (TCH == 3) ? 10 : 12;
     constexpr size_t smem = (size_t)WARPS * NS * Stage<TCH, S2>::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
     static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
-    static bool attr_done[kT3dMaxDevices] = {};
-    bool& attr_set = attr_done[t3d_device_slot()];
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(loss_march_kernel<TCH, REP, BWD, S2, NS, WARPS>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<loss_march_kernel<TCH, REP, BWD, S2, NS, WARPS>>((int)smem)) return rc;
     T3D_LAUNCH("loss_march_kernel", st,
                loss_march_kernel<TCH, REP, BWD, S2, NS, WARPS><<<t3d_sm_count(), WARPS * 32, smem, st>>>(a));
     return T3D_OK;
@@ -873,13 +815,7 @@ int launch_rs(const MarchArgs& a, cudaStream_t st) {
     constexpr int NS = 4, WARPS = 8;
     constexpr size_t smem = (size_t)WARPS * NS * Stage<TCH, false, kSegMax>::kFloats * sizeof(float) + (size_t)WARPS * NS * 8;
     static_assert(smem <= 227 * 1024, "ring does not fit in shared memory");
-    static bool attr_done[kT3dMaxDevices] = {};
-    bool& attr_set = attr_done[t3d_device_slot()];
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(loss_march_rs_kernel<TCH, REP, BWD, kSegMax, NS, WARPS>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<loss_march_rs_kernel<TCH, REP, BWD, kSegMax, NS, WARPS>>((int)smem)) return rc;
     T3D_LAUNCH("loss_march_rs_kernel", st,
                loss_march_rs_kernel<TCH, REP, BWD, kSegMax, NS, WARPS><<<t3d_sm_count(), WARPS * 32, smem, st>>>(a));
     return T3D_OK;

@@ -12,16 +12,9 @@
 
 namespace {
 
-constexpr float kHuber = 0.1f;
 constexpr int kT2H = 16, kT2W = 64, kS2Threads = 256;      // pooled cells per CTA
 constexpr int kR2H = kT2H + 2, kR2W = kT2W + 4;            // rows: one halo cell each side; columns: two on the left (so that a
                                                            // region row starts on a 4-pixel boundary), one used + one spare right
-
-__device__ __forceinline__ float min_nan(float a, float b) { float d; asm("min.NaN.f32 %0, %1, %2;" : "=f"(d) : "f"(a), "f"(b)); return d; }
-__device__ __forceinline__ float times_sgn(float t, float x) {
-    const float r = __uint_as_float(__float_as_uint(t) ^ (__float_as_uint(x) & 0x80000000u));
-    return (x != 0.f) ? r : 0.f;
-}
 
 struct Sums3 { float E, S, D; };
 
@@ -66,7 +59,7 @@ __global__ void __launch_bounds__(kS2Threads) loss_scale2_kernel(const Scale2Arg
         for (int t = lane; t < a.stiles; t += 32) s += (double)sp[(size_t)t * 4];
         s = warp_sum(s);
         const double n2 = (double)h2 * w2;
-        if (lane == 0) s_inv[wrp] = 1.0f / ((float)(s / n2) + 1e-5f);
+        if (lane == 0) s_inv[wrp] = 1.0f / ((float)(s / n2) + kEps);
     }
     // ---- pooled planes of cells I0-1 .. I0+kT2H, J0-2 .. J0+kT2W+1 (cells outside the pooled image: 0).
     // One work item = two horizontally adjacent cells = 4 pixels x 2 rows: 128-bit loads (W % 4 == 0, aligned).
@@ -117,7 +110,7 @@ __global__ void __launch_bounds__(kS2Threads) loss_scale2_kernel(const Scale2Arg
             const bool vx = J < w2 - 1, vy = I < h2 - 1;
             const float g0 = pg[R][C];
             const float tx = vx ? fabsf(pg[R][C + 1] - g0) : 0.f, ty = vy ? fabsf(pg[R + 1][C] - g0) : 0.f;
-            const float w = __expf(-8.0f * (min_nan(tx * inv_mx, m) + min_nan(ty * inv_my, m)));
+            const float w = __expf(-kThermalFactor * (min_nan(tx * inv_mx, m) + min_nan(ty * inv_my, m)));
             const bool own = (r >= 1) && (c >= 1);
             qx = q_term2(vx, pz[R][C], pz[R][C + 1], pgz[R][C], pgz[R][C + 1], w, a.kE, 2.0f * a.kS, a.kD, own, acc);
             qy = q_term2(vy, pz[R][C], pz[R + 1][C], pgz[R][C], pgz[R + 1][C], w, a.kE, 2.0f * a.kS, a.kD, own, acc);

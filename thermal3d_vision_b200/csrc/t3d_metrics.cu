@@ -829,13 +829,7 @@ int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
     src.gt_h = gt_h; src.gt_w = gt_w; src.H = H; src.W = W; src.resample = (gt_h != H) || (gt_w != W);
     src.fx = (double)gt_w / (double)W; src.fy = (double)gt_h / (double)H;
     dim3 g((unsigned)chunks, (unsigned)B);
-    static bool attr_done[kT3dMaxDevices] = {};
-    bool& attr_set = attr_done[t3d_device_slot()];
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(median_scale_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      kCandCap * (int)sizeof(unsigned int)));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<median_scale_kernel>(kCandCap * (int)sizeof(unsigned int))) return rc;
     if (phase != T3D_PHASE_REST) {
         if (median_scaling && phase == T3D_PHASE_SAMPLE)      // ahead of time, beside other kernels: the thin form
             T3D_LAUNCH("metrics_sample_kernel", st, metrics_sample_kernel<256><<<dim3(2, B), 256, 0, st>>>(src, pred_offset, w.bracket, w.counters));

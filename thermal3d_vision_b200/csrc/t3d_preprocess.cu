@@ -917,14 +917,8 @@ int t3d_preprocess_train_u16(const uint16_t* raw, int B, int src_h, int src_w, i
         const size_t stage_bytes = same ? 0 : (size_t)(kHistThreads / 32) * 2 * ((src_w + 7) & ~7) * sizeof(uint16_t);
         const size_t hsmem = (size_t)kWinWords * 4 + (same ? 0 : (size_t)((dst_w + 1) & ~1) * sizeof(uint2)) + stage_bytes;
         T3D_REQUIRE(hsmem <= 200 * 1024, "source rows too wide for the shared-memory staging (src_w <= ~9000)");
-        static bool attr_done[kT3dMaxDevices] = {};
-        bool& attr_set = attr_done[t3d_device_slot()];
-        if (!attr_set) {
-            const int max_smem = 200 * 1024;
-            T3D_CUDA(cudaFuncSetAttribute(resize_hist_u16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-            T3D_CUDA(cudaFuncSetAttribute(resize_hist_u16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem));
-            attr_set = true;
-        }
+        if (int rc = t3d_set_max_dynamic_smem<resize_hist_u16_kernel<true>>(200 * 1024)) return rc;
+        if (int rc = t3d_set_max_dynamic_smem<resize_hist_u16_kernel<false>>(200 * 1024)) return rc;
         if (same)
             T3D_LAUNCH("resize_hist_u16_kernel", st, resize_hist_u16_kernel<false><<<B * chunks, kHistThreads, hsmem, st>>>(
                 raw, resized, hist, meta, w.gxt, w.gyt, B, src_h, src_w, dst_h, dst_w, chunks));
@@ -937,19 +931,14 @@ int t3d_preprocess_train_u16(const uint16_t* raw, int B, int src_h, int src_w, i
     const uint16_t* nsrc = same ? raw : resized;
     const int vec = (dst_w % 4 == 0) && t3d_aligned16(out) && ((reinterpret_cast<uintptr_t>(nsrc) & 7u) == 0);
     if (vec) {
-        constexpr int kStageMax = kNormStageMax;
-        static bool nattr_done[kT3dMaxDevices] = {};
-        bool& nattr = nattr_done[t3d_device_slot()];
-        if (!nattr) {
+        constexpr int kLutBytes = kLutMax * 8, kStagedBytes = kLutMax * 8 + kNormStageMax;
 #define T3D_NORM_ATTR(REP_, ST_) \
-            T3D_CUDA(cudaFuncSetAttribute(normalize_stats_u16_kernel<REP_, ST_, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutMax * 8)); \
-            T3D_CUDA(cudaFuncSetAttribute(normalize_stats_u16_kernel<REP_, ST_, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutMax * 8 + kStageMax))
-            T3D_NORM_ATTR(1, true); T3D_NORM_ATTR(3, true); T3D_NORM_ATTR(1, false); T3D_NORM_ATTR(3, false);
+        if (int rc = t3d_set_max_dynamic_smem<normalize_stats_u16_kernel<REP_, ST_, false>>(kLutBytes)) return rc; \
+        if (int rc = t3d_set_max_dynamic_smem<normalize_stats_u16_kernel<REP_, ST_, true>>(kStagedBytes)) return rc
+        T3D_NORM_ATTR(1, true); T3D_NORM_ATTR(3, true); T3D_NORM_ATTR(1, false); T3D_NORM_ATTR(3, false);
 #undef T3D_NORM_ATTR
-            T3D_CUDA(cudaFuncSetAttribute(normalize_stats_u16_kernel<1, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutMax * 8 + kStageMax));
-            T3D_CUDA(cudaFuncSetAttribute(normalize_stats_u16_kernel<3, true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kLutMax * 8 + kStageMax));
-            nattr = true;
-        }
+        if (int rc = t3d_set_max_dynamic_smem<normalize_stats_u16_kernel<1, true, true, true>>(kStagedBytes)) return rc;
+        if (int rc = t3d_set_max_dynamic_smem<normalize_stats_u16_kernel<3, true, true, true>>(kStagedBytes)) return rc;
         constexpr int kNormCtasPerSm = 32;
         const int nitems = B * kNormBands;
         const int grid = min(nitems, t3d_sm_count() * kNormCtasPerSm);
@@ -958,7 +947,7 @@ int t3d_preprocess_train_u16(const uint16_t* raw, int B, int src_h, int src_w, i
         if (s2) T3D_REQUIRE(t3d_aligned16(nsrc), "half-resolution statistics need 16-byte aligned frames");
         const int band_rows = (dst_h + kNormBands - 1) / kNormBands + (s2 ? 2 : 1);  // + the row(s) below (gradient statistics)
         const size_t stage_bytes = (size_t)band_rows * dst_w * sizeof(uint16_t);
-        const bool staged = (dst_w % 8 == 0) && stage_bytes <= (size_t)kStageMax && t3d_aligned16(nsrc);
+        const bool staged = (dst_w % 8 == 0) && stage_bytes <= (size_t)kNormStageMax && t3d_aligned16(nsrc);
 #define T3D_NORM_LAUNCH(REP_, ST_) do { \
             if (staged) T3D_LAUNCH("normalize_stats_u16_kernel", st, (normalize_stats_u16_kernel<REP_, ST_, true><<<grid, kNormThreads, kLutMax * 8 + stage_bytes, st>>>( \
                 nsrc, percentiles, out, dst_h, dst_w, grad_stats, w.lut, w.lutmeta, nitems))); \
@@ -1005,12 +994,7 @@ static int run_float_percentiles(const float* x, int B, int channels, int n, con
                                  double* percentiles, const FpctWs& w, cudaStream_t st) {
     const int count = (channels == 3) ? n : n * channels;
     T3D_CUDA(cudaMemsetAsync(w.counters, 0, (size_t)B * 8 * sizeof(int), st));
-    static bool attr_done[kT3dMaxDevices] = {};
-    bool& attr_set = attr_done[t3d_device_slot()];
-    if (!attr_set) {
-        T3D_CUDA(cudaFuncSetAttribute(fpct_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFCandCap * (int)sizeof(unsigned int)));
-        attr_set = true;
-    }
+    if (int rc = t3d_set_max_dynamic_smem<fpct_select_kernel>(kFCandCap * (int)sizeof(unsigned int))) return rc;
     T3D_LAUNCH("fpct_sample_kernel", st, fpct_sample_kernel<<<B, t3d_select::kThreads, 0, st>>>(
         x, n, channels, close_flags, w.bracket, (float)(pct_lo / 100.0), (float)(pct_hi / 100.0)));
     dim3 gc((unsigned)max(1, min(kFChunks, (count + 4095) / 4096)), (unsigned)B);

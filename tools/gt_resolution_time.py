@@ -42,10 +42,11 @@ def loss_bytes(B, H, W, gt_hw):
 
 def parent_handle(path):
     h = C.CDLL(os.path.abspath(path))
-    f, p, i = h.t3d_loss_fwd_bwd_resampled, C.c_void_p, C.c_int      # the parent's C ABI (version 2)
-    f.restype, f.argtypes = i, ([p] * 4 + [i] * 2 + [p] * 2 + [i] * 2 + [p] * 2 + [i] + [p] * 4 + [i] * 4
-                                + [C.c_float] * 5 + [p] * 3 + [p, C.c_size_t, p])
+    res, args = _lib._SIGNATURES["t3d_loss_fwd_bwd"]     # the parent's C ABI is the same (version 3)
+    h.t3d_loss_fwd_bwd.restype, h.t3d_loss_fwd_bwd.argtypes = res, args
     h.t3d_last_error.restype = C.c_char_p
+    h.t3d_version.restype = C.c_int
+    assert h.t3d_version() == _lib.ABI_VERSION
     return h
 
 
@@ -72,11 +73,12 @@ def loss_case(B, H, W, dev, parent, iters):
     P = _lib.ptr
 
     def call_parent():
-        rc = parent.t3d_loss_fwd_bwd_resampled(
+        rc = parent.t3d_loss_fwd_bwd(
             P(d["pred1"]), P(d["pred2"]), P(gt[0]), P(gt[1]), GT_HW[0], GT_HW[1], P(d["conf1"]), P(d["conf2"]), H, W,
-            P(th[0]), P(th[1]), 3 | tl.THERMAL_REPLICATED, P(out["dpred1"]), P(out["dpred2"]), P(out["dconf1"]),
-            P(out["dconf2"]), B, H, W, 0, KW["alpha"], KW["edge_weight"], KW["smoothness_weight"], KW["detail_weight"],
-            1.0 / B, P(out["per_sample"]), P(out["batch"]), None, P(ws), ws.numel(), _lib.current_stream_ptr())
+            P(th[0]), P(th[1]), 3 | tl.THERMAL_REPLICATED, None, None, 0, P(out["dpred1"]), P(out["dpred2"]),
+            P(out["dconf1"]), P(out["dconf2"]), B, H, W, 0, KW["alpha"], KW["edge_weight"], KW["smoothness_weight"],
+            KW["detail_weight"], 1.0 / B, P(out["per_sample"]), P(out["batch"]), None, None, P(ws), ws.numel(),
+            _lib.current_stream_ptr())
         assert rc == 0, parent.t3d_last_error()
 
     variants = {"rs": lambda: call(gt[0], gt[1]), "parent": call_parent, "same": lambda: call(gs[0], gs[1])}
