@@ -178,6 +178,12 @@ def _pool_np(a, s):
     return a[:h * s, :w * s].reshape(h, s, w, s).mean(axis=(1, 3))
 
 
+def _pool_f32(a, s):
+    """The reference's F.avg_pool2d of an fp32 image, promoted to float64."""
+    t = torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+    return F.avg_pool2d(t[None, None], s, s)[0, 0].numpy().astype(np.float64)
+
+
 def _sdiff_np(a):
     """signed zero-padded forward differences."""
     dx = np.zeros_like(a)
@@ -193,7 +199,8 @@ def loss_fwd_bwd_f64(p1, p2, g1, g2, c1=None, c2=None, t1=None, t2=None, alpha=0
     """float64 forward + closed-form backward (SURVEY.md Appendix A).
 
     Returns dict(total, basic, edge, smooth, detail, dp1, dp2, dc1, dc2).
-    The gray image is rounded to fp32 first (see _gray_np); everything else fp64.
+    The gray image is rounded to fp32 first (see _gray_np), and the backward of |dz| at scale 2 takes the sign of the
+    reference's fp32 pooled differences (see _pool_f32); everything else fp64.
     """
     out = {"basic": 0.0, "edge": 0.0, "smooth": 0.0, "detail": 0.0}
     grads = []
@@ -221,6 +228,9 @@ def loss_fwd_bwd_f64(p1, p2, g1, g2, c1=None, c2=None, t1=None, t2=None, alpha=0
                 n = h * w_
                 tx, ty = (np.abs(a) for a in _sdiff_np(gr))
                 sx, sy = _sdiff_np(z)
+                # d|dz|/dz = sign(dz) of the reference's fp32 pooled image: two cells that pool to the same fp32 value
+                # have sign 0 there, whatever their float64 means say (at s == 1 the fp32 signs are already exact)
+                gsx, gsy = (sx, sy) if s == 1 else _sdiff_np(_pool_f32(z0, s))
                 bx, by = (np.abs(a) for a in _sdiff_np(gz))
                 ax, ay = np.abs(sx), np.abs(sy)
                 m = CLAMP_VIEW[view]
@@ -237,7 +247,7 @@ def loss_fwd_bwd_f64(p1, p2, g1, g2, c1=None, c2=None, t1=None, t2=None, alpha=0
                     return (lam / n) * np.sign(sd) * (edge_weight * (1 - wt)
                                                       + smoothness_weight * 2 * a * wt
                                                       + detail_weight * dh)
-                qx, qy = q(sx, ax, bx), q(sy, ay, by)   # zero on the padded last col / row (sign(0)=0)
+                qx, qy = q(gsx, ax, bx), q(gsy, ay, by)   # zero on the padded last col / row (sign(0)=0)
                 dz = -qx - qy
                 dz[:, 1:] += qx[:, :-1]
                 dz[1:, :] += qy[:-1, :]

@@ -853,10 +853,9 @@ int t3d_launch_loss_march_ms(const MarchArgs& a, bool bwd, cudaStream_t st) {
 
 int t3d_launch_loss_march(const MarchArgs& a, bool bwd, cudaStream_t st) {
     const bool s2 = bwd && a.dzp[0] != nullptr && a.dzp[1] != nullptr;
-    if (s2) {       // multi-scale backward: add the scale-2 gradient
-        if (a.tch == 3 && a.replicated) return launch<1, true, true, true>(a, st);
-        if (a.tch == 3) return launch<3, false, true, true>(a, st);
-        return launch<1, false, true, true>(a, st);
+    if (s2) {       // multi-scale backward: add the scale-2 gradient (one staged plane takes loss_march_ms_kernel instead)
+        T3D_REQUIRE(a.tch == 3 && !a.replicated, "the two-pass multi-scale path takes three distinct thermal planes");
+        return launch<3, false, true, true>(a, st);
     }
     if (a.tch == 3 && a.replicated) return bwd ? launch<1, true, true, false>(a, st) : launch<1, true, false, false>(a, st);
     if (a.tch == 3) return bwd ? launch<3, false, true, false>(a, st) : launch<3, false, false, false>(a, st);
