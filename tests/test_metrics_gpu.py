@@ -99,11 +99,12 @@ def _check_batch(tm, pm_or_depth, gt, cuda_device, **kw):
 
 
 @pytest.mark.parametrize("kind", ["walls", "ties", "constant", "two_values", "ramp", "tiny_spread"])
-def test_one_kernel_path_on_clustered_depth(cuda_device, kind):
-    """The one-kernel fast path (t3d_metrics_fused.cu) on distributions that stress its bucketed median candidates:
-    spatially coherent depth (whole chunks inside one bucket), heavy ties (every candidate the same key), constant
-    images (the bracket holds everything -> candidate overflow -> exact fallback), an even split between two values
-    (the two middle order statistics differ and live in different buckets), a ramp, a spread of a few ulps."""
+def test_median_candidates_on_clustered_depth(cuda_device, kind):
+    """The sampled median brackets and the candidates the extraction kernels collect inside them, on distributions
+    that stress them: spatially coherent depth (whole chunks inside the bracket: the CTA stage spills to the image's
+    list), heavy ties (every candidate the same key), constant images (the bracket holds everything -> candidate
+    overflow -> exact fallback), an even split between two values (the two middle order statistics differ), a ramp,
+    a spread of a few ulps.  AoS and planar predictions, with and without median scaling."""
     from thermal3d_vision_b200 import metrics as tm
     rng = np.random.default_rng(11)
     B, H, W = 11, 96, 128                      # B not a multiple of the wave size
@@ -133,8 +134,9 @@ def test_one_kernel_path_on_clustered_depth(cuda_device, kind):
     _check_batch(tm, pm, gt, cuda_device, median_scaling=False)
 
 
-def test_one_kernel_path_resampled_gt_many_images(cuda_device):
-    """GT at another size (nearest resample inside the kernel) and enough images for several waves of the queue."""
+def test_resampled_gt_many_images(cuda_device):
+    """GT at another size (nearest resample through the fast kernels' index tables), 19 images, one of them with an
+    empty mask; two runs give the same bits."""
     from oracle import ref_preprocess
     from thermal3d_vision_b200 import metrics as tm
     rng = np.random.default_rng(5)
@@ -155,6 +157,50 @@ def test_one_kernel_path_resampled_gt_many_images(cuda_device):
     # two runs: bit-identical (fixed-order sums, exact selection)
     r2 = tm.compute_depth_metrics_batch(torch.from_numpy(pm).to(cuda_device), torch.from_numpy(big).to(cuda_device))
     assert torch.equal(torch.nan_to_num(r["metrics_f64"]), torch.nan_to_num(r2["metrics_f64"]))
+
+
+def _misaligned(t):
+    """A contiguous copy at element offset 1 of its storage: not 16-byte aligned."""
+    buf = torch.empty(t.numel() + 1, dtype=t.dtype, device=t.device)
+    v = buf[1:].view(t.shape)
+    v.copy_(t)
+    return v
+
+
+@pytest.mark.parametrize("case", ["aos", "planar", "aos_gt_other_size", "masked", "w_not_mult_4",
+                                  "misaligned", "z_view", "w_not_mult_4_gt_other_size"])
+def test_extraction_and_sum_kernels_per_input_class(cuda_device, case):
+    """choose_metrics_path: which extraction and sum kernels each input class runs (the library's launch names), and
+    that the metrics equal the oracle's on each of them."""
+    from oracle import ref_preprocess
+    from thermal3d_vision_b200 import _lib
+    from thermal3d_vision_b200 import metrics as tm
+    rng = np.random.default_rng(21)
+    B, H, W = 2, 48, 53 if case.startswith("w_not_mult_4") else 64
+    gh, gw = (80, 72) if case.endswith("gt_other_size") else (H, W)
+    gt = (1.5 + 3 * np.abs(rng.standard_normal((B, gh, gw)))).astype(np.float32)
+    gt[0, :5] = 0.0
+    gt_small = np.stack([ref_preprocess.resize_nearest(g, (H, W)) for g in gt]) if (gh, gw) != (H, W) else gt
+    pm = rng.standard_normal((B, H, W, 3)).astype(np.float32)
+    pm[..., 2] = np.abs(gt_small * (1 + 0.2 * rng.standard_normal(gt_small.shape)).astype(np.float32)) + 0.02
+    z = np.ascontiguousarray(pm[..., 2])
+    mask = ((rng.random((B, H, W)) < 0.7) & (gt_small > 0)) if case == "masked" else None
+    d = torch.from_numpy(pm).to(cuda_device)
+    pred = {"planar": torch.from_numpy(z).to(cuda_device), "misaligned": _misaligned(torch.from_numpy(z).to(cuda_device)),
+            "z_view": d[..., 2]}.get(case, d)
+    fast = case in ("aos", "planar", "aos_gt_other_size")
+    torch.cuda.synchronize()
+    _lib.profile_begin("depth_extract|metrics_sum", 64)
+    r = tm.compute_depth_metrics_batch(pred, torch.from_numpy(gt).to(cuda_device),
+                                       None if mask is None else torch.from_numpy(mask).to(cuda_device))
+    torch.cuda.synchronize()
+    names = [n for n, _, _ in _lib.profile_timeline(64)]
+    _lib.profile_end()
+    assert names == (["depth_extract_fast_kernel", "metrics_sum_fast_kernel"] if fast else
+                     ["depth_extract_kernel", "metrics_sum_kernel"]), names
+    got = r["metrics_f64"].cpu().numpy()
+    for b in range(B):
+        _close(got[b, :7], _vec(ref_metrics.compute_depth_metrics(z[b], gt_small[b], mask=None if mask is None else mask[b])))
 
 
 def test_nan_and_degenerate_predictions(cuda_device):

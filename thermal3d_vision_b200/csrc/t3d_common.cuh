@@ -147,6 +147,13 @@ __device__ __forceinline__ float warp_min(float v) {
 
 __device__ __forceinline__ float sgnf(float x) { return (x > 0.f) ? 1.f : ((x < 0.f) ? -1.f : 0.f); }
 
+// cv2 INTER_NEAREST source index of destination index d: min(floor(d * scale), src - 1), scale = src / dst in fp64
+// (utils/evaluate_depth_metrics.py:321-323).  Every nearest resample of the library goes through this one rule: the
+// results are bit-exact against cv2 only while it matches cv2's.
+__device__ __forceinline__ int nearest_src(int d, double scale, int src) {
+    return min((int)floor(__dmul_rn((double)d, scale)), src - 1);
+}
+
 // gray = 0.299 c0 + 0.587 c1 + 0.114 c2, fp32, left to right, no FMA contraction
 // (utils/loss.py:120; the rounding is an input to every thermal term).
 __device__ __forceinline__ float gray3(float c0, float c1, float c2) {

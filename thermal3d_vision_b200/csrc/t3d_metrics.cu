@@ -72,10 +72,9 @@ struct PixelSrc {            // how to read (gt, pred, valid) of pixel i of imag
 
 __device__ __forceinline__ void read_pixel(const PixelSrc& s, const float* __restrict__ g, const float* __restrict__ p,
                                            const unsigned char* __restrict__ m, int i, float& gv, float& pv, bool& ok) {
-    if (s.resample) {   // cv2 INTER_NEAREST (utils/evaluate_depth_metrics.py:321-323)
+    if (s.resample) {   // cv2 INTER_NEAREST
         const int y = i / s.W, x = i - y * s.W;
-        const int sx = min((int)floor(__dmul_rn((double)x, s.fx)), s.gt_w - 1);
-        const int sy = min((int)floor(__dmul_rn((double)y, s.fy)), s.gt_h - 1);
+        const int sx = nearest_src(x, s.fx, s.gt_w), sy = nearest_src(y, s.fy, s.gt_h);
         gv = __ldg(g + (size_t)sy * s.gt_w + sx);
     } else {
         gv = __ldg(g + i);
@@ -116,10 +115,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 1024 ? 1 : 4) metrics_samp
             const int i0 = (n >= kSample) ? 4 * (int)(((long long)(k >> 2) * (n >> 2)) / (kSample >> 2)) + (k & 3) : k;
             const int i = min(i0, n - 1);
             size_t gi = (size_t)i;
-            if (s.resample) {   // cv2 INTER_NEAREST (utils/evaluate_depth_metrics.py:321-323), as read_pixel
+            if (s.resample) {   // as read_pixel
                 const int y = i / s.W, x = i - y * s.W;
-                const int sx = min((int)floor(__dmul_rn((double)x, s.fx)), s.gt_w - 1);
-                const int sy = min((int)floor(__dmul_rn((double)y, s.fy)), s.gt_h - 1);
+                const int sx = nearest_src(x, s.fx, s.gt_w), sy = nearest_src(y, s.fy, s.gt_h);
                 gi = (size_t)sy * s.gt_w + sx;
             }
             gvs[q] = __ldg(g + gi);
@@ -193,6 +191,60 @@ __device__ __noinline__ void spill_candidates(unsigned int* __restrict__ stage, 
         }
 }
 
+// The candidates of stream a (0 = gt, 1 = pred) that a thread flagged in one iteration (bit u: keys[u]) go to the CTA
+// stage from the slot the thread reserved for them on; past the stage's end they go to image b's list.
+template <int U>
+__device__ __forceinline__ void stage_candidates(unsigned int (&scand)[2][kCtaCand], int a, int slot, unsigned int flags,
+                                                 const unsigned int (&keys)[U], int* __restrict__ counters,
+                                                 unsigned int* __restrict__ cand, int b) {
+    if (slot + U <= kCtaCand) {
+#pragma unroll
+        for (int u = 0; u < U; ++u) if (flags & (1u << u)) scand[a][slot++] = keys[u];
+    } else spill_candidates<U>(scand[a], slot, flags, keys, &counters[8 * b + 6 + a], &counters[8 * b + 3], cand + ((size_t)b * 2 + a) * kCandCap);
+}
+
+// The end of an extraction CTA: the counts {n_valid, pred_nan, gt_nan (if GT_NAN), lt_g, lt_p} go to image b's counters
+// with one global atomic per counter and CTA, then the staged candidates of each stream (scount[a] slots reserved)
+// reserve their place in the image's list and are copied there.  The helpers here take the kernel's tid: a threadIdx.x
+// read of their own would lose the range the kernel's launch bounds give it, and with it some of the kernel's code.
+template <bool GT_NAN>
+__device__ __forceinline__ void finish_extract_cta(int tid, int (&cnt)[5], int (&sred)[5], const int (&scount)[2], int (&sbase)[2],
+                                                   const unsigned int (&scand)[2][kCtaCand], int* __restrict__ counters,
+                                                   unsigned int* __restrict__ cand, int b) {
+#pragma unroll
+    for (int k = 0; k < 5; ++k) if (GT_NAN || k != 2) cnt[k] = __reduce_add_sync(0xffffffffu, cnt[k]);
+    int* c = counters + 8 * b;
+    if ((tid & 31) == 0) {                             // CTA-level first: one global atomic per counter per CTA
+#pragma unroll
+        for (int k = 0; k < 5; ++k) if ((GT_NAN || k != 2) && cnt[k]) atomicAdd(&sred[k], cnt[k]);
+    }
+    __syncthreads();
+    if (tid < 5 && sred[tid]) atomicAdd(&c[tid < 3 ? tid : tid + 1], sred[tid]);
+    if (tid < 2) {
+        const int k = min(scount[tid], kCtaCand);        // what did not fit the stage went to the list directly (spill)
+        const int base = k ? atomicAdd(&c[6 + tid], k) : 0;
+        if (base + k > kCandCap) { atomicExch(&c[3], 1); sbase[tid] = -1; }      // list overflow (heavy ties) -> exact fallback
+        else sbase[tid] = base;
+    }
+    __syncthreads();
+#pragma unroll
+    for (int a = 0; a < 2; ++a) {
+        const int base = sbase[a], k = min(scount[a], kCtaCand);
+        if (base >= 0)
+            for (int q = tid; q < k; q += kChunkThreads) cand[((size_t)b * 2 + a) * kCandCap + base + q] = scand[a][q];
+    }
+}
+
+// The nearest-resample index tables of a fast-path CTA (H + W <= kResampleMaxDim): stab[x] = source column of column x,
+// stab[W + y] = offset of the source row of row y.  Readable after the next __syncthreads.
+__device__ __forceinline__ void fill_nearest_tables(int* stab, int tid, int H, int W, int gt_h, int gt_w) {
+    const double fx = (double)gt_w / (double)W, fy = (double)gt_h / (double)H;
+    for (int i = tid; i < W + H; i += kChunkThreads) {
+        if (i < W) stab[i] = nearest_src(i, fx, gt_w);
+        else stab[i] = nearest_src(i - W, fy, gt_h) * gt_w;
+    }
+}
+
 // ------------------------------------------------------------------ X: extract (K5) + count + collect
 // pred element (b, i) lives at pred[(b*n + i) * pred_stride + pred_offset]: stride 3 / offset 2 reads
 // the Z channel of an AoS pointmap in place (depth is never materialised by the caller).
@@ -204,7 +256,7 @@ depth_extract_kernel(const PixelSrc s, int pred_offset, float* __restrict__ vz, 
                      unsigned int* __restrict__ cand) {
     __shared__ unsigned int scand[2][kCtaCand];
     __shared__ int scount[2], sbase[2], sred[5];
-    const int b = blockIdx.y, n = s.H * s.W, tid = threadIdx.x, lane = tid & 31;
+    const int b = blockIdx.y, n = s.H * s.W, tid = threadIdx.x;
     const float* __restrict__ g = s.gt + (size_t)b * s.gt_h * s.gt_w;
     const float* __restrict__ p = s.pred + (size_t)b * n * s.pred_stride + pred_offset;
     const unsigned char* __restrict__ m = s.mask ? s.mask + (size_t)b * n : nullptr;
@@ -248,47 +300,12 @@ depth_extract_kernel(const PixelSrc s, int pred_offset, float* __restrict__ vz, 
             fg |= (unsigned)(okg && kgs[u] >= lo_g && kgs[u] <= hi_g) << u;
             fp |= (unsigned)(okp && kps[u] >= lo_p && kps[u] <= hi_p) << u;
         }
-        if (fg) {                       // one shared-memory atomic per thread with candidates (~1 in 4)
-            int slot = atomicAdd(&scount[0], __popc(fg));
-            if (slot + U <= kCtaCand) {
-#pragma unroll
-                for (int u = 0; u < U; ++u) if (fg & (1u << u)) scand[0][slot++] = kgs[u];
-            } else spill_candidates<U>(scand[0], slot, fg, kgs, &counters[8 * b + 6], &counters[8 * b + 3], cand + ((size_t)b * 2) * kCandCap);
-        }
-        if (fp) {
-            int slot = atomicAdd(&scount[1], __popc(fp));
-            if (slot + U <= kCtaCand) {
-#pragma unroll
-                for (int u = 0; u < U; ++u) if (fp & (1u << u)) scand[1][slot++] = kps[u];
-            } else spill_candidates<U>(scand[1], slot, fp, kps, &counters[8 * b + 7], &counters[8 * b + 3], cand + ((size_t)b * 2 + 1) * kCandCap);
-        }
+        // one shared-memory atomic per thread with candidates (~1 in 4)
+        if (fg) stage_candidates<U>(scand, 0, atomicAdd(&scount[0], __popc(fg)), fg, kgs, counters, cand, b);
+        if (fp) stage_candidates<U>(scand, 1, atomicAdd(&scount[1], __popc(fp)), fp, kps, counters, cand, b);
     }
-    nv = __reduce_add_sync(0xffffffffu, nv); pnan = __reduce_add_sync(0xffffffffu, pnan);
-    gnan = __reduce_add_sync(0xffffffffu, gnan);
-    lt_g = __reduce_add_sync(0xffffffffu, lt_g); lt_p = __reduce_add_sync(0xffffffffu, lt_p);
-    int* c = counters + 8 * b;
-    if (lane == 0) {                                   // CTA-level first: one global atomic per counter per CTA
-        if (nv) atomicAdd(&sred[0], nv);
-        if (pnan) atomicAdd(&sred[1], pnan);
-        if (gnan) atomicAdd(&sred[2], gnan);
-        if (lt_g) atomicAdd(&sred[3], lt_g);
-        if (lt_p) atomicAdd(&sred[4], lt_p);
-    }
-    __syncthreads();
-    if (tid < 5 && sred[tid]) atomicAdd(&c[tid < 3 ? tid : tid + 1], sred[tid]);
-    if (tid < 2) {
-        const int k = min(scount[tid], kCtaCand);        // what did not fit the stage went to the list directly (spill)
-        const int base = k ? atomicAdd(&c[6 + tid], k) : 0;
-        if (base + k > kCandCap) { atomicExch(&c[3], 1); sbase[tid] = -1; }      // list overflow (heavy ties) -> exact fallback
-        else sbase[tid] = base;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int a = 0; a < 2; ++a) {
-        const int base = sbase[a], k = min(scount[a], kCtaCand);
-        if (base >= 0)
-            for (int q = tid; q < k; q += kChunkThreads) cand[((size_t)b * 2 + a) * kCandCap + base + q] = scand[a][q];
-    }
+    int cnt[5] = {nv, pnan, gnan, lt_g, lt_p};
+    finish_extract_cta<true>(tid, cnt, sred, scount, sbase, scand, counters, cand, b);
 }
 
 // Fast form of X for the common case: no caller mask, 16-byte aligned, n % 4 == 0, prediction either planar
@@ -309,14 +326,8 @@ depth_extract_fast_kernel(const float* __restrict__ pred, const float* __restric
     __shared__ int scount[2], sbase[2], sred[5];
     __shared__ unsigned int scount2;                              // slot counters of both streams: gt low half, pred high half
     __shared__ int stab[RESAMPLE ? kResampleMaxDim : 1];          // cv2 INTER_NEAREST source column (W) / row offset (H)
-    const int b = blockIdx.y, tid = threadIdx.x, lane = tid & 31;
-    if (RESAMPLE) {     // utils/evaluate_depth_metrics.py:321-323: sx = min(floor(x * gw / W), gw - 1), same for rows
-        const double fx = (double)gt_w / (double)W, fy = (double)gt_h / (double)H;
-        for (int i = tid; i < W + H; i += kChunkThreads) {
-            if (i < W) stab[i] = min((int)floor(__dmul_rn((double)i, fx)), gt_w - 1);
-            else stab[i] = min((int)floor(__dmul_rn((double)(i - W), fy)), gt_h - 1) * gt_w;
-        }
-    }
+    const int b = blockIdx.y, tid = threadIdx.x;
+    if (RESAMPLE) fill_nearest_tables(stab, tid, H, W, gt_h, gt_w);
     const float* __restrict__ gimg = gt + (size_t)b * gt_h * gt_w;
     const float4* __restrict__ g4 = reinterpret_cast<const float4*>(gimg);
     const float4* __restrict__ p4 = reinterpret_cast<const float4*>(pred + (size_t)b * n * PSTRIDE);
@@ -378,48 +389,14 @@ depth_extract_fast_kernel(const float* __restrict__ pred, const float* __restric
                 const unsigned int op = fp ? (unsigned)atomicAdd(&scount[1], __popc(fp)) : 0u;
                 old = min(og, 0xffffu) | (min(op, 0xffffu) << 16);        // >= kCtaCand either way: spills
             }
-            if (fg) {
-                int slot = (int)(old & 0xffffu);
-                if (slot + 4 <= kCtaCand) {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u) if (fg & (1u << u)) scand[0][slot++] = kgs[u];
-                } else spill_candidates<4>(scand[0], slot, fg, kgs, &counters[8 * b + 6], &counters[8 * b + 3], cand + ((size_t)b * 2) * kCandCap);
-            }
-            if (fp) {
-                int slot = (int)(old >> 16);
-                if (slot + 4 <= kCtaCand) {
-#pragma unroll
-                    for (int u = 0; u < 4; ++u) if (fp & (1u << u)) scand[1][slot++] = kps[u];
-                } else spill_candidates<4>(scand[1], slot, fp, kps, &counters[8 * b + 7], &counters[8 * b + 3], cand + ((size_t)b * 2 + 1) * kCandCap);
-            }
+            if (fg) stage_candidates<4>(scand, 0, (int)(old & 0xffffu), fg, kgs, counters, cand, b);
+            if (fp) stage_candidates<4>(scand, 1, (int)(old >> 16), fp, kps, counters, cand, b);
         }
     }
     __syncthreads();
     if (packed && tid < 2) scount[tid] = (int)((scount2 >> (16 * tid)) & 0xffffu);
-    nv = __reduce_add_sync(0xffffffffu, nv); pnan = __reduce_add_sync(0xffffffffu, pnan);
-    lt_g = __reduce_add_sync(0xffffffffu, lt_g); lt_p = __reduce_add_sync(0xffffffffu, lt_p);
-    int* c = counters + 8 * b;
-    if (lane == 0) {                                   // CTA-level first: one global atomic per counter per CTA
-        if (nv) atomicAdd(&sred[0], nv);
-        if (pnan) atomicAdd(&sred[1], pnan);
-        if (lt_g) atomicAdd(&sred[3], lt_g);
-        if (lt_p) atomicAdd(&sred[4], lt_p);
-    }
-    __syncthreads();
-    if (tid < 5 && sred[tid]) atomicAdd(&c[tid < 3 ? tid : tid + 1], sred[tid]);
-    if (tid < 2) {
-        const int k = min(scount[tid], kCtaCand);        // what did not fit the stage went to the list directly (spill)
-        const int base = k ? atomicAdd(&c[6 + tid], k) : 0;
-        if (base + k > kCandCap) { atomicExch(&c[3], 1); sbase[tid] = -1; }      // list overflow (heavy ties) -> exact fallback
-        else sbase[tid] = base;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int a = 0; a < 2; ++a) {
-        const int base = sbase[a], k = min(scount[a], kCtaCand);
-        if (base >= 0)
-            for (int q = tid; q < k; q += kChunkThreads) cand[((size_t)b * 2 + a) * kCandCap + base + q] = scand[a][q];
-    }
+    int cnt[5] = {nv, pnan, 0, lt_g, lt_p};           // no NaN GT passes the validity test: gt_nan is not counted
+    finish_extract_cta<false>(tid, cnt, sred, scount, sbase, scand, counters, cand, b);
 }
 
 // ------------------------------------------------------------------ M: exact medians -> scale
@@ -496,6 +473,26 @@ median_scale_kernel(const float* __restrict__ vz, const float* __restrict__ vg, 
 }
 
 // ------------------------------------------------------------------ M3: per-pixel terms (t3d_metrics_internal.cuh)
+// The partial vector of chunk `chunk` of image b: the threads' v (four sums, three delta-counts, a pad), summed by
+// warp butterflies and then over the warps in a fixed order (deterministic).
+__device__ __forceinline__ void write_chunk_partials(int tid, double (&v)[kNPart], double (&red)[kChunkThreads / 32][kNPart],
+                                                     double* __restrict__ partials, int b, int chunks, int chunk) {
+#pragma unroll
+    for (int k = 0; k < kNPart - 1; ++k) v[k] = warp_sum(v[k]);
+    const int lane = tid & 31, wrp = tid >> 5;
+    if (lane == 0) {
+#pragma unroll
+        for (int k = 0; k < kNPart; ++k) red[wrp][k] = v[k];
+    }
+    __syncthreads();
+    if (tid < kNPart) {
+        double t = 0;
+#pragma unroll
+        for (int w = 0; w < kChunkThreads / 32; ++w) t += red[w][tid];
+        partials[((size_t)b * chunks + chunk) * kNPart + tid] = t;
+    }
+}
+
 template <bool GENERAL>
 __global__ void __launch_bounds__(kChunkThreads, 4)
 metrics_sum_kernel(const float* __restrict__ vz, const float* __restrict__ vg,
@@ -552,20 +549,7 @@ metrics_sum_kernel(const float* __restrict__ vz, const float* __restrict__ vg,
         }
     }
     double v[kNPart] = {acc[0], acc[1], acc[2], acc[3], (double)cnt[0], (double)cnt[1], (double)cnt[2], 0.0};
-#pragma unroll
-    for (int k = 0; k < kNPart - 1; ++k) v[k] = warp_sum(v[k]);
-    const int lane = threadIdx.x & 31, wrp = threadIdx.x >> 5;
-    if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < kNPart; ++k) red[wrp][k] = v[k];
-    }
-    __syncthreads();
-    if (threadIdx.x < kNPart) {
-        double t = 0;
-#pragma unroll
-        for (int w = 0; w < kChunkThreads / 32; ++w) t += red[w][threadIdx.x];
-        partials[((size_t)b * chunks + chunk) * kNPart + threadIdx.x] = t;
-    }
+    write_chunk_partials(threadIdx.x, v, red, partials, b, chunks, chunk);
 }
 
 // Fast form of the sum pass (pairs with depth_extract_fast_kernel): GT straight from the caller's array (nearest-
@@ -580,11 +564,7 @@ metrics_sum_fast_kernel(const float* __restrict__ zplane, const float* __restric
     __shared__ int stab[RESAMPLE ? kResampleMaxDim : 1];
     const int b = blockIdx.y, chunk = blockIdx.x, tid = threadIdx.x;
     if (RESAMPLE) {
-        const double fx = (double)gt_w / (double)W, fy = (double)gt_h / (double)H;
-        for (int i = tid; i < W + H; i += kChunkThreads) {
-            if (i < W) stab[i] = min((int)floor(__dmul_rn((double)i, fx)), gt_w - 1);
-            else stab[i] = min((int)floor(__dmul_rn((double)(i - W), fy)), gt_h - 1) * gt_w;
-        }
+        fill_nearest_tables(stab, tid, H, W, gt_h, gt_w);
         __syncthreads();
     }
     // scale = median(gt) / median(pred)  (utils/metrics.py:47)
@@ -645,20 +625,7 @@ metrics_sum_fast_kernel(const float* __restrict__ zplane, const float* __restric
         for (int k = 0; k < 4; ++k) acc[k] += (double)accf[k];
     }
     double v[kNPart] = {acc[0], acc[1], acc[2], acc[3], (double)cnt[0], (double)cnt[1], (double)cnt[2], 0.0};
-#pragma unroll
-    for (int k = 0; k < kNPart - 1; ++k) v[k] = warp_sum(v[k]);
-    const int lane = tid & 31, wrp = tid >> 5;
-    if (lane == 0) {
-#pragma unroll
-        for (int k = 0; k < kNPart; ++k) red[wrp][k] = v[k];
-    }
-    __syncthreads();
-    if (tid < kNPart) {
-        double t = 0;
-#pragma unroll
-        for (int w = 0; w < kChunkThreads / 32; ++w) t += red[w][tid];
-        partials[((size_t)b * chunks + chunk) * kNPart + tid] = t;
-    }
+    write_chunk_partials(tid, v, red, partials, b, chunks, chunk);
 }
 
 // ------------------------------------------------------------------ M4: finalize
@@ -791,6 +758,32 @@ __global__ void __launch_bounds__(256) project_points_kernel(const float* __rest
     }
 }
 
+// The extraction / sum kernel pair of a call; choose_metrics_path picks one.
+enum class MetricsPath {
+    kFastAos,       // depth_extract_fast_kernel<3> + metrics_sum_fast_kernel: the Z channel of an AoS pointmap
+    kFastPlanar,    // depth_extract_fast_kernel<1> + metrics_sum_fast_kernel: a planar prediction
+    kMasked,        // depth_extract_kernel<true> + metrics_sum_kernel<true>: a caller mask
+    kResampled,     // depth_extract_kernel<true> + metrics_sum_kernel<false>: a GT at another size, read per pixel
+    kPlain,         // depth_extract_kernel<false> + metrics_sum_kernel<false>: every other call
+};
+struct MetricsPathChoice { MetricsPath path; bool resample; };   // resample: the GT is nearest-resampled
+
+// aligned: the prediction and the GT are 16-byte aligned.
+MetricsPathChoice choose_metrics_path(int H, int W, int gt_h, int gt_w, bool mask, bool aligned, int pred_stride,
+                                      int pred_offset) {
+    const bool resample = gt_h != H || gt_w != W;
+    // The fast kernels derive the validity from the GT (no caller mask), take 4 pixels per thread with 128-bit loads
+    // (W % 4 == 0, so a quad lies in one row, also of the resampled GT; aligned arrays) and resample through index
+    // tables in shared memory (H + W <= kResampleMaxDim).  They read an AoS pointmap's Z channel or a planar prediction.
+    if (!mask && W % 4 == 0 && aligned && (!resample || H + W <= kResampleMaxDim)) {
+        if (pred_stride == 3 && pred_offset == 2) return {MetricsPath::kFastAos, resample};
+        if (pred_stride == 1 && pred_offset == 0) return {MetricsPath::kFastPlanar, resample};
+    }
+    // A caller mask may select non-positive or non-finite GT: the masked sum evaluates the literal formulas.
+    if (mask) return {MetricsPath::kMasked, resample};
+    return {resample ? MetricsPath::kResampled : MetricsPath::kPlain, resample};
+}
+
 }  // namespace
 
 extern "C" {
@@ -823,10 +816,12 @@ int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
         w.counters = reinterpret_cast<int*>(state);
         w.bracket = reinterpret_cast<unsigned int*>(state) + (size_t)B * 8;
     }
+    const MetricsPathChoice choice = choose_metrics_path(H, W, gt_h, gt_w, mask != nullptr,
+                                                         t3d_aligned16(pred) && t3d_aligned16(gt), pred_stride, pred_offset);
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     PixelSrc src;
     src.pred = pred; src.gt = gt; src.mask = mask; src.pred_stride = pred_stride;
-    src.gt_h = gt_h; src.gt_w = gt_w; src.H = H; src.W = W; src.resample = (gt_h != H) || (gt_w != W);
+    src.gt_h = gt_h; src.gt_w = gt_w; src.H = H; src.W = W; src.resample = choice.resample;
     src.fx = (double)gt_w / (double)W; src.fy = (double)gt_h / (double)H;
     dim3 g((unsigned)chunks, (unsigned)B);
     if (int rc = t3d_set_max_dynamic_smem<median_scale_kernel>(kCandCap * (int)sizeof(unsigned int))) return rc;
@@ -841,38 +836,41 @@ int t3d_depth_metrics(const float* pred, int pred_stride, int pred_offset,
         }
         if (phase == T3D_PHASE_SAMPLE) return T3D_OK;
     }
-    const bool fast_x = !mask && (W % 4 == 0) && t3d_aligned16(pred) && t3d_aligned16(gt) &&
-                        (!src.resample || H + W <= kResampleMaxDim) && (src.resample || (gt_h * gt_w) % 4 == 0) &&
-                        ((pred_stride == 3 && pred_offset == 2) || (pred_stride == 1 && pred_offset == 0));
-    float* medians_out = out_medians ? out_medians : w.scale;       // [B][2]: median(gt), median(pred)
-#define T3D_XFAST(PS_, RS_) T3D_LAUNCH("depth_extract_kernel", st, (depth_extract_fast_kernel<PS_, RS_><<<g, kChunkThreads, 0, st>>>( \
-            pred, gt, n, w.vz, w.counters, w.bracket, w.cand, H, W, gt_h, gt_w)))
-    if (fast_x && pred_stride == 3) { if (src.resample) T3D_XFAST(3, true); else T3D_XFAST(3, false); }
-    else if (fast_x) { if (src.resample) T3D_XFAST(1, true); else T3D_XFAST(1, false); }
-#undef T3D_XFAST
-    else if (mask || src.resample)
-        T3D_LAUNCH("depth_extract_kernel", st, depth_extract_kernel<true><<<g, kChunkThreads, 0, st>>>(
+    float* medians = out_medians ? out_medians : w.scale;           // [B][2]: median(gt), median(pred)
+    // vg = nullptr: the fast paths keep no planar GT copy, an image whose bracket missed re-reads the caller's arrays
+    auto fast = [&](auto extract, const float* zplane) {
+        const auto sum = choice.resample ? metrics_sum_fast_kernel<true> : metrics_sum_fast_kernel<false>;
+        T3D_LAUNCH("depth_extract_fast_kernel", st, extract<<<g, kChunkThreads, 0, st>>>(
+            pred, gt, n, w.vz, w.counters, w.bracket, w.cand, H, W, gt_h, gt_w));
+        T3D_LAUNCH("median_scale_kernel", st, median_scale_kernel<<<dim3(2, B), kMedThreads, kCandCap * sizeof(unsigned int), st>>>(
+            w.vz, nullptr, w.counters, w.cand, w.bracket, n, median_scaling, medians, src, pred_offset));
+        T3D_LAUNCH("metrics_sum_fast_kernel", st, sum<<<g, kChunkThreads, 0, st>>>(
+            zplane, gt, medians, w.counters, median_scaling, n, chunks, w.partials, H, W, gt_h, gt_w));
+        return T3D_OK;
+    };
+    auto general = [&](auto extract, auto sum) {
+        T3D_LAUNCH("depth_extract_kernel", st, extract<<<g, kChunkThreads, 0, st>>>(
             src, pred_offset, w.vz, w.vg, w.counters, w.bracket, w.cand));
-    else
-        T3D_LAUNCH("depth_extract_kernel", st, depth_extract_kernel<false><<<g, kChunkThreads, 0, st>>>(
-            src, pred_offset, w.vz, w.vg, w.counters, w.bracket, w.cand));
-    float* medians = medians_out;
-    T3D_LAUNCH("median_scale_kernel", st, median_scale_kernel<<<dim3(2, B), kMedThreads, kCandCap * sizeof(unsigned int), st>>>(
-        w.vz, fast_x ? nullptr : w.vg, w.counters, w.cand, w.bracket, n, median_scaling, medians, src, pred_offset));
-    if (fast_x) {
-        const float* zplane = (pred_stride == 3) ? w.vz : pred;       // a planar prediction is its own Z plane
-        if (src.resample)
-            T3D_LAUNCH("metrics_sum_kernel", st, metrics_sum_fast_kernel<true><<<g, kChunkThreads, 0, st>>>(
-                zplane, gt, medians, w.counters, median_scaling, n, chunks, w.partials, H, W, gt_h, gt_w));
-        else
-            T3D_LAUNCH("metrics_sum_kernel", st, metrics_sum_fast_kernel<false><<<g, kChunkThreads, 0, st>>>(
-                zplane, gt, medians, w.counters, median_scaling, n, chunks, w.partials, H, W, gt_h, gt_w));
-    } else if (mask)       // a caller-supplied mask may select non-positive / non-finite GT: literal formulas
-        T3D_LAUNCH("metrics_sum_kernel", st, metrics_sum_kernel<true><<<g, kChunkThreads, 0, st>>>(
+        T3D_LAUNCH("median_scale_kernel", st, median_scale_kernel<<<dim3(2, B), kMedThreads, kCandCap * sizeof(unsigned int), st>>>(
+            w.vz, w.vg, w.counters, w.cand, w.bracket, n, median_scaling, medians, src, pred_offset));
+        T3D_LAUNCH("metrics_sum_kernel", st, sum<<<g, kChunkThreads, 0, st>>>(
             w.vz, w.vg, medians, w.counters, median_scaling, n, chunks, w.partials));
-    else
-        T3D_LAUNCH("metrics_sum_kernel", st, metrics_sum_kernel<false><<<g, kChunkThreads, 0, st>>>(
-            w.vz, w.vg, medians, w.counters, median_scaling, n, chunks, w.partials));
+        return T3D_OK;
+    };
+    const bool rs = choice.resample;
+    int rc = T3D_OK;
+    switch (choice.path) {
+    case MetricsPath::kFastAos:
+        rc = fast(rs ? depth_extract_fast_kernel<3, true> : depth_extract_fast_kernel<3, false>, w.vz);
+        break;
+    case MetricsPath::kFastPlanar:                                    // a planar prediction is its own Z plane
+        rc = fast(rs ? depth_extract_fast_kernel<1, true> : depth_extract_fast_kernel<1, false>, pred);
+        break;
+    case MetricsPath::kMasked: rc = general(depth_extract_kernel<true>, metrics_sum_kernel<true>); break;
+    case MetricsPath::kResampled: rc = general(depth_extract_kernel<true>, metrics_sum_kernel<false>); break;
+    case MetricsPath::kPlain: rc = general(depth_extract_kernel<false>, metrics_sum_kernel<false>); break;
+    }
+    if (rc) return rc;
     T3D_LAUNCH("metrics_finalize_kernel", st, metrics_finalize_kernel<<<B, 32 * kNPart, 0, st>>>(w.partials, w.counters, chunks, out, out_f64));
     return T3D_OK;
 }

@@ -61,7 +61,7 @@ __global__ void __launch_bounds__(256) resize_bilinear_kernel(const void* __rest
     }
 }
 
-// cv2 INTER_NEAREST: sx = min(floor(dx * src_w / dst_w), src_w - 1) (utils/evaluate_depth_metrics.py:321-323)
+// cv2 INTER_NEAREST (nearest_src)
 __global__ void __launch_bounds__(256) resize_nearest_kernel(const float* __restrict__ src, float* __restrict__ dst,
                                                              int B, int sh, int sw, int dh, int dw) {
     const double fx = (double)sw / (double)dw, fy = (double)sh / (double)dh;
@@ -72,8 +72,7 @@ __global__ void __launch_bounds__(256) resize_nearest_kernel(const float* __rest
         const size_t t = idx / dw;
         const int y = (int)(t % dh);
         const int b = (int)(t / dh);
-        const int sx = min((int)floor(__dmul_rn((double)x, fx)), sw - 1);
-        const int sy = min((int)floor(__dmul_rn((double)y, fy)), sh - 1);
+        const int sx = nearest_src(x, fx, sw), sy = nearest_src(y, fy, sh);
         dst[idx] = __ldg(src + ((size_t)b * sh + sy) * sw + sx);
     }
 }
