@@ -265,6 +265,21 @@ int t3d_channels_close(const float* x, int B, int n, int* close_flags, void* str
 int t3d_fixed_range_normalize(const float* x, float* y, size_t n, size_t plane, const int* close_flag,
                               int normalized, void* stream);
 
+/* Batched enhance_thermal_fixed_range of raw uint16 frames [B,src_h,src_w], resize included, in one pass:
+ * out [B,out_channels,dst_h,dst_w] float32, out_channels (1 or 3) identical planes.
+ *   T3D_PATH_TRAIN:     cv2.resize to uint16 (data/dataset_loader.py:242), raw counts, then the window with
+ *                       normalized=False: clip [21800, 25000] -> (x - 21800) / 3200, float32.
+ *   T3D_PATH_INFERENCE: /65535.0f, float cv2.resize (thermal_dustr_inference.py:42-52), then the window with
+ *                       normalized=True (x * 65535.0f first), float32.
+ * Each path uses the `normalized` flag that matches the values it holds; both are bit-exact against the reference.
+ * grad_stats / stats_scales: as t3d_preprocess_train_u16 writes them (same layout, same shapes), gray(v, v, v) of the
+ * output for 3 planes; grad_stats must be NULL where t3d_preprocess_stats_tiles(dst_h, dst_w) == 0 or `out` is not
+ * 16-byte aligned.  No workspace. */
+#define T3D_PATH_TRAIN 0
+#define T3D_PATH_INFERENCE 1
+int t3d_preprocess_fixed_range_u16(const uint16_t* raw, int B, int src_h, int src_w, int dst_h, int dst_w, int path,
+                                   float* out, int out_channels, float* grad_stats, int stats_scales, void* stream);
+
 /* ------------------------------------------------- pointmap -> depth, metrics */
 size_t t3d_depth_metrics_workspace_bytes(int B, int H, int W);
 

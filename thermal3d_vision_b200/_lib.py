@@ -56,6 +56,7 @@ _SIGNATURES = {
                                              c_ptr, c_ptr, c_ptr, C.c_size_t, c_ptr]),
     "t3d_channels_close": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, c_ptr]),
     "t3d_fixed_range_normalize": (C.c_int, [c_ptr, c_ptr, C.c_size_t, C.c_size_t, c_ptr, C.c_int, c_ptr]),
+    "t3d_preprocess_fixed_range_u16": (C.c_int, [c_ptr] + [C.c_int] * 6 + [c_ptr, C.c_int, c_ptr, C.c_int, c_ptr]),
     "t3d_depth_metrics_workspace_bytes": (C.c_size_t, [C.c_int] * 3),
     "t3d_depth_metrics": (C.c_int, [c_ptr, C.c_int, C.c_int, c_ptr, C.c_int, C.c_int, c_ptr]
                           + [C.c_int] * 4 + [c_ptr] * 3 + [c_ptr, C.c_size_t, c_ptr, C.c_int, c_ptr]),

@@ -14,24 +14,6 @@
 
 namespace {
 
-template <typename SrcT, bool DIV65535>
-__device__ __forceinline__ float src_value(const SrcT* __restrict__ p) {
-    const float v = (float)__ldg(p);
-    return DIV65535 ? __fdiv_rn(v, 65535.0f) : v;
-}
-
-template <typename SrcT, bool DIV65535>
-__device__ __forceinline__ float bilinear_at(const SrcT* __restrict__ src, int sw, const Tap& ty, const Tap& tx) {
-    const SrcT* r0 = src + (size_t)ty.s0 * sw;
-    const SrcT* r1 = src + (size_t)ty.s1 * sw;
-    // horizontal pass then vertical pass, every product rounded separately (no FMA)
-    const float h0 = __fadd_rn(__fmul_rn(src_value<SrcT, DIV65535>(r0 + tx.s0), tx.c0),
-                               __fmul_rn(src_value<SrcT, DIV65535>(r0 + tx.s1), tx.c1));
-    const float h1 = __fadd_rn(__fmul_rn(src_value<SrcT, DIV65535>(r1 + tx.s0), tx.c0),
-                               __fmul_rn(src_value<SrcT, DIV65535>(r1 + tx.s1), tx.c1));
-    return __fadd_rn(__fmul_rn(h0, ty.c0), __fmul_rn(h1, ty.c1));
-}
-
 // ------------------------------------------------------------------ K1: resize kernels
 // MODE 0: u16 -> u16 (train path, data/dataset_loader.py:242)
 // MODE 1: u16 -> f32 with /65535 first (inference path, thermal_dustr_inference.py:42-52)
@@ -519,7 +501,6 @@ __global__ void __launch_bounds__(256) normalize_u16_kernel(const uint16_t* __re
 // bits, no per-pixel fp64 divide) is copied to shared memory, and the sums of |Dx gray|, |Dy gray| of the
 // OUTPUT image are reduced per CTA into stats[b][band][0..1] (gray = 0.299 v + 0.587 v + 0.114 v in fp32
 // when the output is replicated to 3 planes).
-constexpr int kNormBands = 24;       // CTAs per frame == statistic partials per frame (T3D_STATS_TILES)
 constexpr int kNormThreads = 256;
 constexpr int kNormStageMax = 24 * 1024;  // staged band bytes: LUT 32 KB + band <= 56 KB per CTA, 4 CTAs per SM
 // shapes whose bands the half-resolution pass handles: even bands of <= 16 rows, W / 2 columns <= one per thread,
@@ -581,37 +562,6 @@ __device__ __noinline__ void normalize_band_direct(const uint16_t* __restrict__ 
 // STAGED (W % 8 == 0, the band fits): the band's raw rows (+ the row below) and the LUT arrive in shared memory as
 // ONE batch of cp.async copies -- a single exposed memory latency per CTA instead of one per marched row (the
 // marches are short: 8 rows per warp at 384 rows), and the march itself then reads shared memory only.
-// Half-resolution sums of a band (utils/loss.py:133-174: |Dx|, |Dy| of the 2x2 average-pooled gray image, zero-padded
-// last column / row), for the multi-scale loss.  Thread = pooled column (W / 2 <= kNormThreads), the band's pooled rows
-// (+ the one below) in registers; the right neighbour comes from a shuffle, across warps from shared memory.
-constexpr int kS2MaxPool = 9;            // pooled rows of a band + 1 (bands of <= 16 rows)
-template <typename Pooled>
-__device__ __forceinline__ void half_res_band_sums(int y0, int y1, int H, int W, float (*edge)[kS2MaxPool],
-                                                   Pooled pooled, float& tx2, float& ty2) {
-    const int tid = threadIdx.x, lane = tid & 31, wrp = tid >> 5;
-    const int h2 = H >> 1, w2 = W >> 1;
-    const int I0 = y0 >> 1, I1 = min(y1, 2 * h2) >> 1;               // y0 is even: the band's own pooled rows [I0, I1)
-    const int nown = I1 - I0, npool = nown + ((I1 < h2) ? 1 : 0);
-    const int J = tid;
-    float pv[kS2MaxPool];
-#pragma unroll
-    for (int r = 0; r < kS2MaxPool; ++r) pv[r] = (r < npool && J < w2) ? pooled(I0 + r, J) : 0.f;
-    if (lane == 0) {
-#pragma unroll
-        for (int r = 0; r < kS2MaxPool; ++r) edge[wrp][r] = pv[r];
-    }
-    __syncthreads();
-#pragma unroll
-    for (int r = 0; r < kS2MaxPool - 1; ++r) {
-        float right = __shfl_down_sync(0xffffffffu, pv[r], 1);
-        if (lane == 31) right = edge[wrp + 1][r];
-        if (r < nown && J < w2) {
-            if (J + 1 < w2) tx2 += fabsf(right - pv[r]);
-            if (I0 + r + 1 < h2) ty2 += fabsf(pv[r + 1] - pv[r]);
-        }
-    }
-}
-
 template <int REP, bool STATS, bool STAGED, bool S2 = false>
 __global__ void __launch_bounds__(kNormThreads, 4) normalize_stats_u16_kernel(const uint16_t* __restrict__ src,
                                                                            const double* __restrict__ p,

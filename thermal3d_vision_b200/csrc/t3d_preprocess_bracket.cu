@@ -23,18 +23,6 @@ namespace {
 constexpr int kSamp = 4096;
 constexpr int kBrStride = kBrSlots;          // uints per windowed histogram (window bins + the below / above slot)
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void cp_async16(uint32_t dst_saddr, const void* src) {
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" :: "r"(dst_saddr), "l"(src) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" :: "n"(N) : "memory"); }
-__device__ __forceinline__ unsigned int lds_u16(uint32_t saddr) {
-    unsigned short v;
-    asm volatile("ld.shared.u16 %0, [%1];" : "=h"(v) : "r"(saddr));
-    return v;
-}
-
 // exact u16 -> fp32 without the conversion pipe: 0x4B000000 | v is the float 2^23 + v
 __device__ __forceinline__ float u16_to_float(unsigned int v) { return __fsub_rn(__uint_as_float(0x4B000000u | v), 8388608.0f); }
 // round-half-even of 0 <= x < 2^22 to an integer (what cvt.rni / cv2's saturate_cast<ushort> do): x + 2^23
@@ -286,32 +274,6 @@ constexpr int kRzWarps = kRzThreads / 32;
 constexpr int kRzU = 8;                 // consecutive output pixels per lane
 constexpr int kRzStrip = 32 * kRzU;
 constexpr int kRing = 4;
-
-// H54 -- the dataset's horizontal geometry.  640 -> 512 columns (data/dataset_loader.py:242 with the training size of
-// train_thermal_dustr.py) is a 5:4 reduction: scale = 1.25 exactly, so cv2's x taps are periodic -- 4 outputs from 5
-// inputs, weights {1/8, 3/8, 5/8, 7/8}, no border clamping -- and become compile-time constants: a lane's 8 output
-// pixels read 10 consecutive source pixels (five 32-bit shared loads instead of sixteen 16-bit ones, no tap
-// registers).  Same arithmetic, same order, same bits.  (The vertical 512 -> 384 is 4:3: its taps are not exactly
-// periodic in floating point and stay in the table.)
-template <int K> struct W54 { static constexpr float f = (2 * (K & 3) + 1) * 0.125f; static constexpr float c = 1.0f - f; };
-
-__device__ __forceinline__ void hpass54(uint32_t saddr, float h[8]) {
-    unsigned int w[5];
-#pragma unroll
-    for (int i = 0; i < 5; ++i) asm volatile("ld.shared.u32 %0, [%1];" : "=r"(w[i]) : "r"(saddr + 4u * i));
-    float p[10];
-#pragma unroll
-    for (int i = 0; i < 5; ++i) { p[2 * i] = (float)(w[i] & 0xffffu); p[2 * i + 1] = (float)(w[i] >> 16); }
-    // output u reads source pixels u + u / 4 and the next one
-    h[0] = __fadd_rn(__fmul_rn(p[0], W54<0>::c), __fmul_rn(p[1], W54<0>::f));
-    h[1] = __fadd_rn(__fmul_rn(p[1], W54<1>::c), __fmul_rn(p[2], W54<1>::f));
-    h[2] = __fadd_rn(__fmul_rn(p[2], W54<2>::c), __fmul_rn(p[3], W54<2>::f));
-    h[3] = __fadd_rn(__fmul_rn(p[3], W54<3>::c), __fmul_rn(p[4], W54<3>::f));
-    h[4] = __fadd_rn(__fmul_rn(p[5], W54<0>::c), __fmul_rn(p[6], W54<0>::f));
-    h[5] = __fadd_rn(__fmul_rn(p[6], W54<1>::c), __fmul_rn(p[7], W54<1>::f));
-    h[6] = __fadd_rn(__fmul_rn(p[7], W54<2>::c), __fmul_rn(p[8], W54<2>::f));
-    h[7] = __fadd_rn(__fmul_rn(p[8], W54<3>::c), __fmul_rn(p[9], W54<3>::f));
-}
 
 // one warp: resize + classify output rows [ya, yb) of strip `strip` of frame `f`
 template <bool DENSE, bool H54>

@@ -152,7 +152,9 @@ def npy_header(path: str):
 
 def load_thermal_batch(paths: Sequence[str], img_size=(224, 224), device=None, threads: int = 8, **kw):
     """paths -> ThermalBatch on the GPU: native PNG decode into pinned memory, one H2D copy, then
-    ``preprocess_thermal_batch`` (= FreiburgDataset._load_thermal_image + enhance_thermal_contrast per frame)."""
+    ``preprocess_thermal_batch`` (= FreiburgDataset._load_thermal_image + enhance_thermal_contrast per frame; with
+    ``normalization="fixed_range"`` + enhance_thermal_fixed_range, the loader's alternative at
+    data/dataset_loader.py:111,119).  Keyword arguments go to ``preprocess_thermal_batch``."""
     from . import preprocessing as _pre
     raw = read_thermal_png_batch(paths, threads=threads, pin=True)
     dev = torch.device(device if device is not None else "cuda")

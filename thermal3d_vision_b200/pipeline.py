@@ -47,12 +47,18 @@ class HotPathStep:
     produced (they are the model's input) but the loss does not read them, and the preprocessing computes no
     thermal-gradient statistics; edge_weight / smoothness_weight / detail_weight do not apply and the packed vector's
     slots 2-4 are 0.  It has no multi-scale form.
+
+    Normalisation.  ``normalization="percentile"`` (default) normalises the thermal frames as the dataset loader does
+    (enhance_thermal_contrast, per-frame 2nd / 98th percentiles); ``"fixed_range"`` uses the loader's alternative,
+    the Freiburg radiometric window (enhance_thermal_fixed_range on the train path's raw counts): one kernel per step,
+    no sampling ahead and no workspace for the preprocessing (the metric chain still samples ahead), no histogram.
     """
 
     def __init__(self, B: int, H: int, W: int, raw_hw=(512, 640), device=None, multi_scale: bool = False,
                  alpha=0.2, edge_weight=0.5, smoothness_weight=0.3, detail_weight=0.4, distributed: bool = False,
                  exchange: str = "peer", pipelined: bool = False, sobel: bool = False, gt_hw=None,
-                 use_thermal_aware_loss: bool = True):
+                 use_thermal_aware_loss: bool = True, normalization: str = "percentile"):
+        self.normalization = _pre.check_normalization(normalization)
         if not use_thermal_aware_loss and multi_scale:
             raise ValueError("multi_scale is a form of the thermal-aware loss: use_thermal_aware_loss=False has none")
         self.use_thermal_aware_loss = bool(use_thermal_aware_loss)
@@ -94,11 +100,11 @@ class HotPathStep:
         self.loss_views = list(self.loss_sets)
         # both views are preprocessed by ONE call when the caller hands them over as the two halves of a single
         # [2B,...] tensor (what run_host's staging does): outputs are halves of one buffer as well
-        self.pre_sets = [{
-            "thermal": torch.empty(2 * B, 3, H, W, **f32),
-            "percentiles": torch.empty(2 * B, 2, dtype=torch.float64, device=dev),
-            "workspace": torch.empty(lib.t3d_preprocess_workspace_bytes(2 * B, H, W), dtype=torch.uint8, device=dev),
-        } for _ in range(2)]
+        self.pre_sets = [{"thermal": torch.empty(2 * B, 3, H, W, **f32)} for _ in range(2)]
+        if self.normalization == "percentile":
+            for p in self.pre_sets:
+                p["percentiles"] = torch.empty(2 * B, 2, dtype=torch.float64, device=dev)
+                p["workspace"] = torch.empty(lib.t3d_preprocess_workspace_bytes(2 * B, H, W), dtype=torch.uint8, device=dev)
         if self.use_thermal_aware_loss:      # the thermal-gradient sums the loss reads (the plain loss reads none)
             for p in self.pre_sets:
                 p["grad_stats"] = torch.empty(2 * B, max(lib.t3d_preprocess_stats_tiles(H, W), 1), 4, **f32)
@@ -125,7 +131,7 @@ class HotPathStep:
         if self.pipelined:
             for m in self.met_sets:
                 m["state"] = torch.empty(lib.t3d_depth_metrics_state_bytes(B), dtype=torch.uint8, device=dev)
-        else:
+        elif self.normalization == "percentile":
             self.pre_sets[1]["workspace"] = self.pre_sets[0]["workspace"]
         self.loss_out, self.pre_both, self.met_out = self.loss_sets[0], self.pre_sets[0], self.met_sets[0]
         if self.sobel:
@@ -267,6 +273,8 @@ class HotPathStep:
         stacked = (raw1.is_contiguous() and raw2.is_contiguous() and raw1.shape == raw2.shape and
                    raw1.untyped_storage().data_ptr() == raw2.untyped_storage().data_ptr() and
                    raw2.storage_offset() == raw1.storage_offset() + raw1.numel())      # halves of one tensor
+        if self.histogram and self.normalization == "fixed_range":
+            raise ValueError("histogram=True: the fixed-range normalisation computes no histogram")
         if self.histogram and "histogram" not in pre:
             pre["histogram"] = torch.empty(2 * B, 65536, dtype=torch.int32, device=self.device)
 
@@ -279,6 +287,9 @@ class HotPathStep:
         # form with the 1 024-thread sampling kernels, which are faster when they have the machine to themselves)
         ahead = self.pipelined and stacked and not self.histogram and self._primed
         self._primed = True
+        pre_ahead = ahead and self.normalization == "percentile"     # the fixed window has nothing to sample
+        pre_kw = dict(half_res_stats=self.multi_scale, shared=True, grad_stats=self.use_thermal_aware_loss,
+                      normalization=self.normalization)
         if ahead:
             # ungated, on their own streams: ordered only after the inputs and after the last user of this set's
             # sampling state (step - 2: its preprocessing / metric chain)
@@ -287,12 +298,12 @@ class HotPathStep:
                 self.s_samp_m.wait_event(self.ev_met[i])
                 _metrics.compute_depth_metrics_batch(pred1, gt_depth, out=met, phase=_metrics.PHASE_SAMPLE)
                 self.ev_sm[i].record(self.s_samp_m)
+        if pre_ahead:
             with torch.cuda.stream(self.s_samp_p):
                 self.s_samp_p.wait_event(ready)
                 self.s_samp_p.wait_event(self.ev_pre[i])
                 _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=False,
-                                              half_res_stats=self.multi_scale, phase=_metrics.PHASE_SAMPLE, shared=True,
-                                              grad_stats=self.use_thermal_aware_loss)
+                                              phase=_metrics.PHASE_SAMPLE, **pre_kw)
                 self.ev_sp[i].record(self.s_samp_p)
         phase = _metrics.PHASE_REST if ahead else _metrics.PHASE_ALL
         s_met = self.s_met_alt if (i & 1) else self.s_met
@@ -309,12 +320,11 @@ class HotPathStep:
             self.s_pre.wait_event(ready)
             if gate is not None:
                 self.s_pre.wait_event(gate)
-            if ahead:
+            if pre_ahead:
                 self.s_pre.wait_event(self.ev_sp[i])
             if stacked:
                 tb = _pre.preprocess_thermal_batch(raw_both, size, path="train", out=pre, histogram=self.histogram,
-                                                   half_res_stats=self.multi_scale, phase=phase, shared=True,
-                                                   grad_stats=self.use_thermal_aware_loss)
+                                                   phase=phase if pre_ahead else _metrics.PHASE_ALL, **pre_kw)
                 gs = tb.grad_stats
                 stats_scales = tb.stats_scales
                 (t1, t2), stats = (tb.thermal[:B], tb.thermal[B:]), ((None, None) if gs is None else (gs[:B], gs[B:]))
@@ -324,11 +334,9 @@ class HotPathStep:
                                             torch.empty(lib.t3d_preprocess_workspace_bytes(B, self.H, self.W), dtype=torch.uint8,
                                                         device=self.device) for k, v in pre.items()} for h in range(2)]
                 a = _pre.preprocess_thermal_batch(raw1, size, path="train", out=self._pre_halves[i][0], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale, shared=True,
-                                                  grad_stats=self.use_thermal_aware_loss)
+                                                  **pre_kw)
                 b = _pre.preprocess_thermal_batch(raw2, size, path="train", out=self._pre_halves[i][1], histogram=self.histogram,
-                                                  half_res_stats=self.multi_scale, shared=True,
-                                                  grad_stats=self.use_thermal_aware_loss)
+                                                  **pre_kw)
                 (t1, t2), stats = (a.thermal, b.thermal), (a.grad_stats, b.grad_stats)
                 stats_scales = min(a.stats_scales, b.stats_scales)
             pgrads, n_pgrads = None, 0
@@ -579,9 +587,13 @@ class EvalStep:
     path='train': data/dataset_loader.py:237-249 + enhance_thermal_contrast (u16 resize, raw counts);
     path='inference': utils/evaluate_depth_metrics.py:162-197 (/65535, float resize, float percentiles).
     GT depth of another size is nearest-resampled inside the metric kernels (utils/evaluate_depth_metrics.py:320-323).
+    normalization='fixed_range': the thermal batch on the Freiburg fixed window (enhance_thermal_fixed_range) instead of
+    the per-frame percentiles, on either path -- what a model trained on that normalisation must be evaluated on.
     """
 
-    def __init__(self, B: int, H: int, W: int, raw_hw=(512, 640), gt_hw=None, device=None, path: str = "train"):
+    def __init__(self, B: int, H: int, W: int, raw_hw=(512, 640), gt_hw=None, device=None, path: str = "train",
+                 normalization: str = "percentile"):
+        self.normalization = _pre.check_normalization(normalization)
         self.B, self.H, self.W, self.raw_hw, self.path = B, H, W, tuple(raw_hw), path
         self.gt_hw = tuple(gt_hw) if gt_hw is not None else (H, W)
         self.device = torch.device(device if device is not None else "cuda")
@@ -589,10 +601,11 @@ class EvalStep:
         f32 = dict(dtype=torch.float32, device=dev)
         # every buffer twice: batches alternate, so that `prefetch` can sample batch k+1 while batch k is in flight and
         # the thermal batch a call returns stays valid until the call after the next one
-        self.pre_sets = [{"thermal": torch.empty(B, 3, H, W, **f32),
-                          "percentiles": torch.empty(B, 2, dtype=torch.float64, device=dev),
-                          "workspace": torch.empty(lib.t3d_preprocess_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev)}
-                         for _ in range(2)]
+        self.pre_sets = [{"thermal": torch.empty(B, 3, H, W, **f32)} for _ in range(2)]
+        if self.normalization == "percentile":
+            for p in self.pre_sets:
+                p["percentiles"] = torch.empty(B, 2, dtype=torch.float64, device=dev)
+                p["workspace"] = torch.empty(lib.t3d_preprocess_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev)
         self.met_sets = [{"workspace": torch.empty(lib.t3d_depth_metrics_workspace_bytes(B, H, W), dtype=torch.uint8, device=dev),
                           "state": torch.empty(lib.t3d_depth_metrics_state_bytes(B), dtype=torch.uint8, device=dev),
                           "metrics": torch.empty(B, 8, **f32), "metrics_f64": torch.empty(B, 8, dtype=torch.float64, device=dev),
@@ -622,20 +635,23 @@ class EvalStep:
         of the batch in flight; the `run_batch` call for the same tensors then starts with its heavy kernels.  Call it
         BEFORE the `run_batch` of the batch in front (what is recorded now is that the inputs are ready now).  In a
         real evaluation loop the raw frames of batch k+1 are known while the model still works on batch k -- the
-        pointmap is not: pass `pointmap=None` and only the preprocessing is sampled ahead."""
-        if self.path != "train":
+        pointmap is not: pass `pointmap=None` and only the preprocessing is sampled ahead.  With
+        normalization='fixed_range' (either path) the preprocessing has nothing to sample: only the metric chain is."""
+        fixed = self.normalization == "fixed_range"
+        if self.path != "train" and not fixed:
             return
         with _lib.device_guard(self.device):
             j = self._next
             self._next ^= 1
             main = torch.cuda.current_stream(self.device)
             self.ev_ready[j].record(main)
-            with torch.cuda.stream(self.s_samp_p):
-                self.s_samp_p.wait_event(self.ev_ready[j])
-                self.s_samp_p.wait_event(self.ev_pre_done[j])          # the last batch on this set is done with it
-                _pre.preprocess_thermal_batch(raw, (self.W, self.H), path="train", out=self.pre_sets[j], histogram=False,
-                                              phase=_metrics.PHASE_SAMPLE, shared=True)
-                self.ev_sp[j].record(self.s_samp_p)
+            if not fixed:
+                with torch.cuda.stream(self.s_samp_p):
+                    self.s_samp_p.wait_event(self.ev_ready[j])
+                    self.s_samp_p.wait_event(self.ev_pre_done[j])      # the last batch on this set is done with it
+                    _pre.preprocess_thermal_batch(raw, (self.W, self.H), path="train", out=self.pre_sets[j], histogram=False,
+                                                  phase=_metrics.PHASE_SAMPLE, shared=True)
+                    self.ev_sp[j].record(self.s_samp_p)
             if pointmap is not None:
                 with torch.cuda.stream(self.s_samp_m):
                     self.s_samp_m.wait_event(self.ev_ready[j])
@@ -670,10 +686,11 @@ class EvalStep:
                 me = _metrics.compute_depth_metrics_batch(pointmap, gt_depth, out=met, phase=met_phase)
                 self.join.record(self.side)
                 self.ev_met_done[j].record(self.side)
-            main.wait_event(self.ev_sp[j])                   # likewise for the preprocessing's sampling state
+            if self.normalization == "percentile":
+                main.wait_event(self.ev_sp[j])               # likewise for the preprocessing's sampling state
             # shared=True: the metric pipeline runs beside the preprocessing (side stream)
             tb = _pre.preprocess_thermal_batch(raw, (self.W, self.H), path=self.path, out=pre, histogram=False, phase=pre_phase,
-                                               shared=True)
+                                               shared=True, normalization=self.normalization)
             self.ev_pre_done[j].record(main)
             main.wait_event(self.join)
             self.acc.update(me["metrics_f64"])

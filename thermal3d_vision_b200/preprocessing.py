@@ -71,9 +71,19 @@ def resize_nearest(src: torch.Tensor, size_hw) -> torch.Tensor:
 
 
 # ----------------------------------------------------------------------------- batched train / inference paths
+NORMALIZATIONS = ("percentile", "fixed_range")
+PATH_CODES = {"train": 0, "inference": 1}      # T3D_PATH_TRAIN / T3D_PATH_INFERENCE (include/t3d.h)
+
+
+def check_normalization(normalization: str) -> str:
+    if normalization not in NORMALIZATIONS:
+        raise ValueError(f"normalization must be one of {NORMALIZATIONS}, got {normalization!r}")
+    return normalization
+
+
 class ThermalBatch(NamedTuple):
     thermal: torch.Tensor                      # [B, C, h, w] float32 in [0, 1]
-    percentiles: torch.Tensor                  # [B, 2] float64 (p2, p98)
+    percentiles: Optional[torch.Tensor]        # [B, 2] float64 (p2, p98); None on the fixed window
     histogram: Optional[torch.Tensor] = None   # [B, 65536] int32 view of the uint32 counts (train path)
     grad_stats: Optional[torch.Tensor] = None  # [B, tiles, 4] partial sums of |Dx gray|, |Dy gray| (train path)
     stats_scales: int = 1                      # 2: grad_stats[..., 2:4] hold the half-resolution sums (multi-scale loss)
@@ -83,7 +93,8 @@ class ThermalBatch(NamedTuple):
 def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: str = "train",
                              out_channels: int = 3, out: Optional[dict] = None,
                              histogram: bool = True, half_res_stats: bool = False, phase: int = 0,
-                             shared: bool = False, grad_stats: bool = True) -> ThermalBatch:
+                             shared: bool = False, grad_stats: bool = True,
+                             normalization: str = "percentile") -> ThermalBatch:
     """16-bit radiometric frames [B,Hs,Ws] -> normalised thermal [B,3,h,w].
 
     img_size is (W, H) in cv2 order like the reference's --img_size.  path='train':
@@ -99,7 +110,14 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
     shared=True (train path) is a scheduling hint: other kernels run concurrently on another stream (the metric chain
     of pipeline.HotPathStep / EvalStep), so the resize kernel leaves them room on every SM.  Same results.
     grad_stats=False (train path): no thermal-gradient sums (ThermalBatch.grad_stats is None), for a loss that does not
-    use the thermal images; the thermal planes are the same."""
+    use the thermal images; the thermal planes are the same.
+    normalization='fixed_range': enhance_thermal_fixed_range (utils/preprocessing.py:32-73) instead of the percentile
+    normalisation -- the Freiburg radiometric window [21800, 25000], the same absolute scale for every frame -- in one
+    kernel that resizes and normalises (t3d_preprocess_fixed_range_u16).  Each path applies the window to the values it
+    holds: raw counts on the train path (normalized=False), [0, 1] values on the inference path (normalized=True).
+    It computes no statistic of the frame: percentiles and histogram are None, `histogram` and `shared` do not apply,
+    phase=1 launches nothing and any other phase is the whole call.  grad_stats / half_res_stats as on the train path."""
+    check_normalization(normalization)
     x = _to_cuda(raw_u16).contiguous()
     if x.dtype != torch.uint16:
         raise ValueError(f"raw frames must be uint16, got {x.dtype}")
@@ -114,6 +132,8 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
     thermal = out.get("thermal")
     if thermal is None:
         thermal = torch.empty(B, out_channels, dh, dw, dtype=torch.float32, device=dev)
+    if normalization == "fixed_range":
+        return _fixed_range_batch(x, dh, dw, path, out_channels, thermal, out, half_res_stats, phase, grad_stats, stream)
     pct = out.get("percentiles")
     if pct is None:
         pct = torch.empty(B, 2, dtype=torch.float64, device=dev)
@@ -127,12 +147,7 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
         ws = out.get("workspace")
         if ws is None or ws.numel() < ws_bytes:
             ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
-        tiles = lib.t3d_preprocess_stats_tiles(dh, dw) if grad_stats else 0
-        stats = None
-        if tiles > 0:
-            stats = out.get("grad_stats")
-            if stats is None:
-                stats = torch.empty(B, tiles, 4, dtype=torch.float32, device=dev)
+        stats = _grad_stats_buffer(lib, out, B, dh, dw, dev) if grad_stats else None
         scales = 1
         if half_res_stats and stats is not None and lib.t3d_preprocess_stats_scales(dh, dw) == 2:
             scales = 2
@@ -152,6 +167,28 @@ def preprocess_thermal_batch(raw_u16: torch.Tensor, img_size=(224, 224), path: s
         _lib.check(rc, "t3d_contrast_normalize_f32")
         return ThermalBatch(thermal, pct, None)
     raise ValueError("path must be 'train' or 'inference'")
+
+
+def _grad_stats_buffer(lib, out, B, dh, dw, dev):
+    tiles = lib.t3d_preprocess_stats_tiles(dh, dw)
+    if tiles <= 0:
+        return None
+    stats = out.get("grad_stats")
+    return stats if stats is not None else torch.empty(B, tiles, 4, dtype=torch.float32, device=dev)
+
+
+def _fixed_range_batch(x, dh, dw, path, out_channels, thermal, out, half_res_stats, phase, grad_stats, stream):
+    if path not in PATH_CODES:
+        raise ValueError("path must be 'train' or 'inference'")
+    lib = _lib.lib()
+    B, sh, sw = x.shape
+    stats = _grad_stats_buffer(lib, out, B, dh, dw, x.device) if grad_stats and path == "train" else None
+    scales = 2 if half_res_stats and stats is not None and lib.t3d_preprocess_stats_scales(dh, dw) == 2 else 1
+    if phase != 1:          # T3D_PHASE_SAMPLE: nothing to sample ahead on the fixed window
+        rc = lib.t3d_preprocess_fixed_range_u16(_lib.ptr(x), B, sh, sw, dh, dw, PATH_CODES[path], _lib.ptr(thermal),
+                                                out_channels, _lib.ptr(stats), scales, stream)
+        _lib.check(rc, "t3d_preprocess_fixed_range_u16")
+    return ThermalBatch(thermal, None, None, stats, scales)
 
 
 @_lib.on_tensor_device
