@@ -597,17 +597,18 @@ metrics_sum_fast_kernel(const float* __restrict__ zplane, const float* __restric
         const float za8[8] = {za.x, za.y, za.z, za.w, zb.x, zb.y, zb.z, zb.w};
         float pr[8];
         bool ok[8];
-        bool all_normal = true;        // every selected pixel: gt and scaled prediction positive, normal, finite
+        bool all_in_range = true;      // every selected pixel: gt and scaled prediction in [2^-120, 2^126)
 #pragma unroll
         for (int e = 0; e < 8; ++e) {
             pr[e] = __fmul_rn(za8[e], s);                                            // pred *= scale   (:48)
             const unsigned int gbits = __float_as_uint(gtv[e]), pbits = __float_as_uint(pr[e]);
             ok[e] = (gbits - 1u) < 0x7f7fffffu;                                      // gt > 0 & finite (:27)
-            const bool normal = ((gbits - 0x00800000u) < 0x7f000000u) && ((pbits - 0x00800000u) < 0x7f000000u);
-            all_normal = all_normal && (normal || !ok[e]);
+            // bits in [0x03800000, 0x7e800000): the range metric_terms_nodiv is exact on (t3d_metrics_internal.cuh)
+            const bool in_range = ((gbits - 0x03800000u) < 0x7b000000u) && ((pbits - 0x03800000u) < 0x7b000000u);
+            all_in_range = all_in_range && (in_range || !ok[e]);
         }
         float accf[4] = {0.f, 0.f, 0.f, 0.f};
-        if (all_normal) {
+        if (all_in_range) {
             float accl2 = 0.f;
             int unselected = 0;
 #pragma unroll
@@ -617,7 +618,7 @@ metrics_sum_fast_kernel(const float* __restrict__ zplane, const float* __restric
             }
             cnt[0] -= unselected; cnt[1] -= unselected; cnt[2] -= unselected;        // g = q = 1 counted as "inside"
             accf[3] = accl2 * 0.48045301391820144f;                                  // ln(2)^2
-        } else {                                                                     // zero / negative / NaN / Inf / subnormal: literal formulas
+        } else {                                                                     // zero / negative / NaN / Inf / tiny / huge: literal formulas
 #pragma unroll 1
             for (int e = 0; e < 8; ++e) metric_terms<false>(ok[e] ? gtv[e] : qnan, za8[e], s, accf, cnt);
         }

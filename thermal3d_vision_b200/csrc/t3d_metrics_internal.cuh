@@ -31,9 +31,10 @@ __device__ __forceinline__ void metric_terms(float gt, float z, float s, float a
     cnt[0] += th < 1.25f; cnt[1] += th < 1.5625f; cnt[2] += th < 1.953125f;  // :52-54
     const float d = __fsub_rn(gt, pr);
     const float d2 = __fmul_rn(d, d);
-    const float rg = __fdividef(1.0f, gt);
-    accf[0] += fabsf(d) * rg;                                                // :56  |gt - pred| / gt
-    accf[1] += d2 * rg;                                                      // :57
+    // IEEE divisions, as numpy: 1 / gt is subnormal for gt > 2^126 (an approximate reciprocal flushes it to 0) and
+    // overflows for gt < 2^-128
+    accf[0] += __fdiv_rn(fabsf(d), gt);                                      // :56  |gt - pred| / gt
+    accf[1] += __fdiv_rn(d2, gt);                                            // :57
     accf[2] += d2;                                                           // :58
     accf[3] += dl * dl;                                                      // :59
 }
@@ -51,21 +52,25 @@ __device__ __forceinline__ void metric_terms_fast(float gt, float pr, float accf
     cnt[0] += (valid && th < 1.25f); cnt[1] += (valid && th < 1.5625f); cnt[2] += (valid && th < 1.953125f);   // :52-54
     const float d = g - q;
     const float d2 = d * d;
-    const float rg = __fdividef(1.0f, g);
-    accf[0] = fmaf(fabsf(d), rg, accf[0]);                                   // :56  |gt - pred| / gt
-    accf[1] = fmaf(d2, rg, accf[1]);                                         // :57
+    accf[0] += __fdiv_rn(fabsf(d), g);                                       // :56  |gt - pred| / gt (IEEE, as metric_terms)
+    accf[1] += __fdiv_rn(d2, g);                                             // :57
     accf[2] += d2;                                                           // :58
     accf[3] = fmaf(dl, dl, accf[3]);                                         // :59
 }
 
-// Division-free form of the same terms for g, q positive NORMAL finite numbers (valid pixels; invalid ones are
-// passed as g = q = 1).  numpy: thresh = max(gt/pred, pred/gt) = fl(a / b), a = max, b = min
+// Division-free form of the same terms for g, q in [2^-120, 2^126) (valid pixels; invalid ones are passed as
+// g = q = 1).  numpy: thresh = max(gt/pred, pred/gt) = fl(a / b), a = max, b = min
 // (IEEE division is monotone), counted against T in {1.25, 1.5625, 1.953125} (:51-54).  For such T (in (1, 2), even
 // mantissa) fl(a / b) < T  <=>  a / b < T - 2^-24 (the midpoint below T; a tie rounds to even = T)
 // <=>  a - T b + 2^-24 b < 0, and that sign is computed EXACTLY by two FMAs: r = fma(-T, b, a) is exact whenever
-// |a - T b| < b / 64 (a and T b are multiples of ulp(b) / 64) and otherwise so much larger than 2^-24 b that its
-// rounding cannot change the sign of the sum; fma(2^-24, b, r) rounds once, which never flips a sign.
+// |a - T b| < b / 64 and ulp(b) / 64 >= 2^-149, and otherwise so much larger than 2^-24 b that its rounding cannot
+// change the sign of the sum; fma(2^-24, b, r) rounds once, which never flips a sign (a negative sum that underflows
+// is -0: sign bit set).  Exactness: a and T b are multiples of ulp(b) / 64 (T = k / 64), so r is one too, with at most
+// 24 significant bits when |r| < b / 64 -- an fp32 number if that grid is not finer than the fp32 subnormal
+// spacing 2^-149, i.e. ulp(b) >= 2^-143, b >= 2^-120.  Below that r is rounded and the sign can flip (the kernel
+// sends such pixels to the literal formula; tests/test_metrics_nodiv_cpu.py restates both FMAs).
 // -> the delta-counts are those of the correctly rounded quotient, without dividing.
+// Above: g < 2^126 keeps 1 / g normal (rcp.approx.ftz flushes a subnormal reciprocal to 0).
 // log: u = q / g to ~1 ulp (reciprocal + one Newton step), |log gt - log pred| = ln2 |lg2 u|; the caller folds
 // ln2^2 into the sum of lg2(u)^2 (accl2).
 __device__ __forceinline__ float rcp_fast(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
